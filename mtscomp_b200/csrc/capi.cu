@@ -160,6 +160,8 @@ int set_attrs(mtsb_ctx* c) {
   CK(cudaFuncSetAttribute(fwd_transform_kernel<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
   CK(cudaFuncSetAttribute(fwd_transform_kernel<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
   CK(cudaFuncSetAttribute(fwd_transform_kernel<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
+  CK(cudaFuncSetAttribute(fwd_transform_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
+  CK(cudaFuncSetAttribute(fwd_transform_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
   CK(cudaFuncSetAttribute((par_lz_kernel<1024, 16384>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PAR_LZ_MIRROR));
   CK(cudaFuncSetAttribute((par_lz_kernel<256, 4096>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PAR_LZ_MIRROR));
 #define MTS_INV_ATTR(T) \

@@ -1,6 +1,9 @@
 // cuda_emu.cpp — fiber scheduler for cuda_emu.h (development tool, see the header's banner).
 #include "cuda_emu.h"
 
+#include <mutex>
+#include <unordered_map>
+
 thread_local uint3 threadIdx, blockIdx;
 thread_local dim3 blockDim, gridDim;
 
@@ -8,6 +11,23 @@ namespace emu {
 
 thread_local Block* g_blk = nullptr;
 thread_local unsigned char* g_dyn_smem = nullptr;
+thread_local int g_last_error = 0;
+
+static std::mutex g_attr_mu;
+static std::unordered_map<const void*, size_t> g_max_dyn_smem;   // kernel -> its MaxDynamicSharedMemorySize
+
+int set_max_dyn_smem(const void* fn, int bytes) {
+  if (bytes < 0 || (size_t)bytes > kDynSmemOptin) return cudaErrorInvalidValue;
+  std::lock_guard<std::mutex> g(g_attr_mu);
+  g_max_dyn_smem[fn] = (size_t)bytes;
+  return 0;
+}
+
+static size_t max_dyn_smem(const void* fn) {
+  std::lock_guard<std::mutex> g(g_attr_mu);
+  auto it = g_max_dyn_smem.find(fn);
+  return it == g_max_dyn_smem.end() ? kDynSmemDefault : it->second;
+}
 
 asm(R"(
 .text
@@ -90,7 +110,8 @@ static void run_block(Block& b, dim3 bd, const std::function<void()>& body) {
   g_blk = nullptr;
 }
 
-void launch(dim3 grid, dim3 block, size_t smem, const std::function<void()>& body) {
+void launch(const void* fn, dim3 grid, dim3 block, size_t smem, const std::function<void()>& body) {
+  if (smem > kDynSmemOptin || smem > max_dyn_smem(fn)) { g_last_error = cudaErrorInvalidValue; return; }
   size_t nblocks = (size_t)grid.x * grid.y * grid.z;
   if (nblocks == 0) return;
   unsigned nthr = std::thread::hardware_concurrency();

@@ -78,7 +78,14 @@ static inline void yield() {
   emu_switch(&b->sp[b->cur], b->sched_sp);
 }
 
-void launch(dim3 grid, dim3 block, size_t smem, const std::function<void()>& body);
+// Dynamic shared memory a launch may ask for: 48 KB unless the kernel's cudaFuncAttributeMaxDynamicSharedMemorySize
+// says otherwise, and never more than the opt-in limit of an sm_100 block (sharedMemPerBlockOptin below).  A launch
+// past its limit runs nothing and leaves cudaErrorInvalidValue for the next cudaGetLastError, as on the device.
+static const size_t kDynSmemDefault = 48 * 1024, kDynSmemOptin = 232448;
+extern thread_local int g_last_error;           // cudaGetLastError's slot (per host thread, as in the runtime)
+int set_max_dyn_smem(const void* fn, int bytes);
+template <class F> static inline const void* fn_addr(F f) { return reinterpret_cast<const void*>(f); }
+void launch(const void* fn, dim3 grid, dim3 block, size_t smem, const std::function<void()>& body);
 
 }  // namespace emu
 
@@ -277,9 +284,12 @@ enum cudaMemcpyKind { cudaMemcpyHostToHost, cudaMemcpyHostToDevice, cudaMemcpyDe
 enum { cudaStreamNonBlocking = 1, cudaEventDisableTiming = 2, cudaHostAllocDefault = 0 };
 enum cudaFuncAttribute { cudaFuncAttributeMaxDynamicSharedMemorySize = 8, cudaFuncAttributePreferredSharedMemoryCarveout = 9 };
 enum { cudaSharedmemCarveoutMaxShared = 100 };
-static inline const char* cudaGetErrorString(cudaError_t e) { return e ? "emu error" : "no error"; }
-static inline cudaError_t cudaGetLastError() { return 0; }
-static inline cudaError_t cudaPeekAtLastError() { return 0; }
+static inline const char* cudaGetErrorString(cudaError_t e) {
+  return e == cudaSuccess ? "no error" : e == cudaErrorInvalidValue ? "invalid argument"
+       : e == cudaErrorMemoryAllocation ? "out of memory" : "emu error";
+}
+static inline cudaError_t cudaGetLastError() { cudaError_t e = emu::g_last_error; emu::g_last_error = 0; return e; }
+static inline cudaError_t cudaPeekAtLastError() { return emu::g_last_error; }
 static inline cudaError_t cudaSetDevice(int) { return 0; }
 static inline cudaError_t cudaGetDevice(int* d) { *d = 0; return 0; }
 static inline cudaError_t cudaGetDeviceCount(int* n) { *n = 1; return 0; }
@@ -307,7 +317,9 @@ static inline cudaError_t cudaEventElapsedTime(float* ms, cudaEvent_t a, cudaEve
   *ms = std::chrono::duration<float, std::milli>(b->t - a->t).count();
   return 0;
 }
-template <class F> static inline cudaError_t cudaFuncSetAttribute(F, cudaFuncAttribute, int) { return 0; }
+template <class F> static inline cudaError_t cudaFuncSetAttribute(F f, cudaFuncAttribute a, int v) {
+  return a == cudaFuncAttributeMaxDynamicSharedMemorySize ? emu::set_max_dyn_smem(emu::fn_addr(f), v) : 0;
+}
 struct cudaDeviceProp { int multiProcessorCount; int major, minor; size_t sharedMemPerBlockOptin; char name[64]; size_t totalGlobalMem; };
 static inline cudaError_t cudaGetDeviceProperties(cudaDeviceProp* p, int) {
   p->multiProcessorCount = 8; p->major = 10; p->minor = 0; p->sharedMemPerBlockOptin = 232448;
@@ -320,5 +332,5 @@ enum { cudaMemoryTypeUnregistered = 0, cudaMemoryTypeHost = 1, cudaMemoryTypeDev
 static inline cudaError_t cudaPointerGetAttributes(cudaPointerAttributes* a, const void*) { a->type = 2; return 0; }
 
 #define MTS_LAUNCH(kernel, grid, block, smem, stream, ...) \
-  emu::launch((grid), (block), (smem), [&]() { kernel(__VA_ARGS__); })
+  emu::launch(emu::fn_addr(kernel), (grid), (block), (smem), [&]() { kernel(__VA_ARGS__); })
 #define MTS_DYN_SMEM(name) unsigned char* name = emu::g_dyn_smem

@@ -11,6 +11,8 @@
 // ('F': nc runs of ns elements) or row-major ('C'), at the same element offset as the raw chunk.
 // Every CTA works on a full-width tile of TT consecutive rows, which is one contiguous span of the row-major side.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace mts {
@@ -20,6 +22,33 @@ template <class T> __host__ __device__ inline int tile_pitch(int nc) {
   if (sizeof(T) == 1) { int p = (nc + 3) & ~3; if ((p & 4) == 0) p += 4; return p; }
   if (sizeof(T) == 2) { int p = (nc + 1) & ~1; if ((p & 2) == 0) p += 2; return p; }
   return nc | 1;
+}
+
+// ------------------------------------------------------------------------------------------------ element arithmetic
+// Differences and sums of float32 / float64 elements give the NaN that NumPy gives on x86-64, the hosts that write and
+// read these files: a NaN operand comes back quieted (the first one if both are NaN), and a NaN made from numbers
+// (inf - inf) is the default NaN with the sign bit set.  The device's own rule (always 0x7fffffff) would change the
+// transform bytes, and the decoded bits, of any recording with a NaN in it.  Integers: plain modular arithmetic.
+template <class T> __device__ __forceinline__ T nan_as_x86(T, T, T r) { return r; }
+template <class F, class U> __device__ __forceinline__ F nan_as_x86_fp(F a, F b, F r, U quiet, U dflt) {
+  U u;
+  if (a != a) { memcpy(&u, &a, sizeof u); u |= quiet; }
+  else if (b != b) { memcpy(&u, &b, sizeof u); u |= quiet; }
+  else if (r != r) u = dflt;
+  else return r;
+  memcpy(&r, &u, sizeof r);
+  return r;
+}
+__device__ __forceinline__ float nan_as_x86(float a, float b, float r) { return nan_as_x86_fp(a, b, r, 0x00400000u, 0xffc00000u); }
+__device__ __forceinline__ double nan_as_x86(double a, double b, double r) {
+  return nan_as_x86_fp(a, b, r, 0x0008000000000000ull, 0xfff8000000000000ull);
+}
+template <class T> __device__ __forceinline__ T sub_el(T a, T b) { return nan_as_x86(a, b, (T)(a - b)); }
+template <class T> __device__ __forceinline__ T add_el(T a, T b) { return nan_as_x86(a, b, (T)(a + b)); }
+// Time difference x[t] - x[t-1].  The chunk's first row is copied, as np.diff's caller does (mtscomp.py:143-159), not
+// reduced by a zero: that would quiet a signalling NaN.  (For integers the two are the same.)
+template <class T> __device__ __forceinline__ T time_diff(T cur, T prev, bool first_row) {
+  return std::is_floating_point<T>::value && first_row ? cur : sub_el(cur, prev);
 }
 
 // ------------------------------------------------------------------------------------------------ K1 forward
@@ -40,7 +69,7 @@ __global__ void __launch_bounds__(512) fwd_transform_kernel(const T* __restrict_
   T* y = dst + cd.elem_off;
   const bool td = (flags & FLAG_TIME_DIFF) != 0, sd = (flags & FLAG_SPATIAL_DIFF) != 0;
 
-  // smem row r holds sample t0-1+r; row 0 is zero for the chunk's first tile, so "x[t]-x[t-1]" keeps row 0 as is.
+  // smem row r holds sample t0-1+r; row 0 is zero for the chunk's first tile (never used: time_diff copies that row).
   const long long base = (long long)(t0 - 1) * nc;
   const int n_el = (rows + 1) * nc;
   for (int e = threadIdx.x; e < n_el; e += blockDim.x) {
@@ -56,8 +85,8 @@ __global__ void __launch_bounds__(512) fwd_transform_kernel(const T* __restrict_
       int r = e / nc, c = e - r * nc;
       const T* p = s + (r + 1) * P + c;
       T v = p[0];
-      if (td) v = (T)(v - p[-P]);
-      if (sd && c > 0) { T w = p[-1]; if (td) w = (T)(w - p[-P - 1]); v = (T)(v - w); }
+      if (td) v = time_diff(v, p[-P], t0 + r == 0);
+      if (sd && c > 0) { T w = p[-1]; if (td) w = time_diff(w, p[-P - 1], t0 + r == 0); v = sub_el(v, w); }
       y[(long long)t0 * nc + e] = v;
     }
   } else {
@@ -66,8 +95,8 @@ __global__ void __launch_bounds__(512) fwd_transform_kernel(const T* __restrict_
       for (int r = lane_id(); r < rows; r += 32) {
         const T* p = s + (r + 1) * P + c;
         T v = p[0];
-        if (td) v = (T)(v - p[-P]);
-        if (sd && c > 0) { T w = p[-1]; if (td) w = (T)(w - p[-P - 1]); v = (T)(v - w); }
+        if (td) v = time_diff(v, p[-P], t0 + r == 0);
+        if (sd && c > 0) { T w = p[-1]; if (td) w = time_diff(w, p[-P - 1], t0 + r == 0); v = sub_el(v, w); }
         y[(long long)c * ns + t0 + r] = v;
       }
     }
@@ -291,7 +320,7 @@ __global__ void __launch_bounds__(INV_TILE_MAXT, 2) fwd_tile_kernel(const T* __r
 #pragma unroll
         for (int r = 0; r < R; r++) {
           const T cur = p[(long long)(g * R + r) * nc];
-          v[r] = td ? (T)(cur - prev) : cur;
+          v[r] = td ? time_diff(cur, prev, !halo && g == 0 && r == 0) : cur;
           prev = cur;
         }
       } else {
@@ -299,8 +328,9 @@ __global__ void __launch_bounds__(INV_TILE_MAXT, 2) fwd_tile_kernel(const T* __r
         for (int r = 0; r < R; r++) {
           T cur = 0, curl = 0;
           if (r < nr) { cur = p[(long long)(g * R + r) * nc]; if (left) curl = p[(long long)(g * R + r) * nc - 1]; }
-          T a = td ? (T)(cur - prev) : cur;
-          if (left) a = (T)(a - (td ? (T)(curl - prevl) : curl));
+          const bool first = !halo && g == 0 && r == 0;
+          T a = td ? time_diff(cur, prev, first) : cur;
+          if (left) a = sub_el(a, td ? time_diff(curl, prevl, first) : curl);
           v[r] = a;
           prev = cur; prevl = curl;
         }
@@ -554,10 +584,11 @@ __global__ void __launch_bounds__(128) inv_cols_kernel(const T* __restrict__ in,
 
 
 // ------------------------------------------------------------------------------------------------ floating point inverse
-// float32 / float64 (FLAG_FLOAT): the forward differences are single IEEE subtractions, so the integer kernels above
-// are simply instantiated for float / double.  The inverse is different: np.cumsum accumulates sequentially in the
-// array's own precision (mtscomp.py:162-169), and reproducing the reference Reader bit for bit means adding in the
-// same order — one thread per row (spatial pass, into a scratch copy) and one thread per channel (time pass).
+// float32 / float64 (FLAG_FLOAT): the forward differences are single IEEE subtractions (sub_el, with NumPy's NaNs), so
+// the integer kernels above are simply instantiated for float / double.  The inverse is different: np.cumsum
+// accumulates sequentially in the array's own precision (mtscomp.py:162-169), and reproducing the reference Reader bit
+// for bit means adding in the same order (add_el) — one thread per row (spatial pass, into a scratch copy) and one
+// thread per channel (time pass).
 template <class T>
 __global__ void __launch_bounds__(128) inv_float_space_kernel(const T* __restrict__ in, T* __restrict__ tmp,
                                                               const ChunkDesc* __restrict__ chunks, int nc, int flags) {
@@ -572,7 +603,7 @@ __global__ void __launch_bounds__(128) inv_float_space_kernel(const T* __restric
   for (int c = 0; c < nc; c++) {
     const long long i = oc ? (long long)t * nc + c : (long long)c * ns + t;
     const T v = x[i];
-    acc = c == 0 ? v : acc + v;
+    acc = c == 0 ? v : add_el(acc, v);
     y[i] = acc;
   }
 }
@@ -590,7 +621,7 @@ __global__ void __launch_bounds__(128) inv_float_time_kernel(const T* __restrict
   T acc = 0;
   for (int t = 0; t < ns; t++) {
     const T v = x[oc ? (long long)t * nc + c : (long long)c * ns + t];
-    acc = (t == 0 || !td) ? v : acc + v;
+    acc = (t == 0 || !td) ? v : add_el(acc, v);
     y[(long long)t * nc + c] = acc;
   }
 }

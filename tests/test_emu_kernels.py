@@ -157,24 +157,49 @@ def test_emulated_float_golden(emu, name):
 
 
 @pytest.mark.parametrize('nc,dtype', [(1, 'int16'), (31, 'uint8'), (447, 'int16'), (449, 'int16'), (449, 'int64'),
-                                      (900, 'int32'), (1800, 'int16'), (2100, 'int16'), (450, 'uint8')])
+                                      (900, 'int32'), (1800, 'int16'), (2100, 'int16'), (450, 'uint8'),
+                                      (190, 'float32'), (94, 'float64'), (1793, 'float32'), (1793, 'float64')])
 def test_emulated_tile_kernels_channel_counts(emu, nc, dtype):
     """The channel-major tile kernels give a thread 1, 2 or 4 channels depending on n_channels and fall back to the
-    generic kernels beyond that: every regime, ragged chunk lengths, all four difference settings."""
+    generic kernels beyond that: every regime, ragged chunk lengths, all four difference settings.  Float arrays go
+    through both orders: the generic forward kernel stages a tile of 65 rows in shared memory, more than the default
+    48 KB from 190 float32 / 94 float64 channels on ('C'), and above 1792 channels in either order."""
     from mtscomp_b200 import _native
     rng = np.random.default_rng(nc)
-    ns = [70, 33, 5, 129]
+    is_float = np.dtype(dtype).kind == 'f'
+    ns = [70, 33, 5, 129] if not (is_float and nc > 1792) else [9, 1, 4]
     x = np.cumsum(rng.integers(-3, 4, (sum(ns), nc)), axis=0).astype(dtype)
     rows = np.concatenate(([0], np.cumsum(ns)))
-    for td, sd in ((True, False), (True, True), (False, True), (False, False)):
-        fl = _native.flags_of(td, sd, 'F')
-        kw = dict(do_time_diff=td, do_spatial_diff=sd, chunk_order='F')
-        for i in range(len(ns)):
-            assert emu.delta_transform(x[rows[i]:rows[i + 1]], fl).tobytes() == ora.transform_chunk(x[rows[i]:rows[i + 1]], **kw)
-        comp = [ora.encode_chunk(x[rows[i]:rows[i + 1]], **kw) for i in range(len(ns))]
-        offs = np.concatenate(([0], np.cumsum([len(c) for c in comp])))
-        out, st = emu.decompress(b''.join(comp), offs, rows, nc, dtype, fl)
-        assert not st.any() and np.array_equal(out, x), (td, sd)
+    for order in ('F', 'C') if is_float else ('F',):
+        for td, sd in ((True, False), (True, True), (False, True), (False, False)):
+            fl = _native.flags_of(td, sd, order)
+            kw = dict(do_time_diff=td, do_spatial_diff=sd, chunk_order=order)
+            for i in range(len(ns)):
+                assert emu.delta_transform(x[rows[i]:rows[i + 1]], fl).tobytes() == ora.transform_chunk(x[rows[i]:rows[i + 1]], **kw)
+            comp = [ora.encode_chunk(x[rows[i]:rows[i + 1]], **kw) for i in range(len(ns))]
+            offs = np.concatenate(([0], np.cumsum([len(c) for c in comp])))
+            out, st = emu.decompress(b''.join(comp), offs, rows, nc, dtype, fl)
+            assert not st.any() and out.tobytes() == x.tobytes(), (order, td, sd)
+
+
+@pytest.mark.parametrize('dtype', ['float32', 'float64'])
+@pytest.mark.parametrize('nc', [7, 449, 1793])
+def test_emulated_float_special_values(emu, dtype, nc):
+    """Signed zeros, subnormals, differences that overflow, inf - inf, quiet NaNs with payloads and signalling NaNs at
+    the first and last row of every chunk and at the first and last column, through the forward and inverse kernels,
+    compress and decompress, in both orders and all four difference settings.  The chunk's first row must be copied,
+    not reduced by zero: that would quiet a signalling NaN there.  (The host emulation computes with the host's NaN
+    rules, so it cannot show the device's; tests/test_gpu_transform_regimes.py checks those on a GPU.)"""
+    from transform_cases import FLAG_SETS, NAN_PAYLOAD_SKIP, check_four_paths, float_data, nan_payloads_checked, \
+        ragged_rows
+    rows = ragged_rows(dtype, nc, tail=0 if nc > 1000 else 40)
+    for kind in ('smooth', 'wild'):
+        x = float_data(kind, dtype, rows, nc, seed=nc)
+        for order in 'FC':
+            for td, sd in FLAG_SETS:
+                check_four_paths(emu, x, rows, td, sd, order)
+    if not nan_payloads_checked():
+        pytest.skip(NAN_PAYLOAD_SKIP)
 
 
 def test_emulated_inverse_ragged_batches(emu):
