@@ -21,11 +21,32 @@ using namespace mts;
 namespace {
 
 thread_local std::string g_err;
+int fail(mtsb_ctx* c, int code, const char* fmt, ...);
+
+#define CK(call)                                                                                     \
+  do {                                                                                               \
+    cudaError_t e__ = (call);                                                                        \
+    if (e__ != cudaSuccess) return fail(c, MTSB_E_CUDA, "%s: %s", #call, cudaGetErrorString(e__)); \
+  } while (0)
+#define CKL()                                                                                                  \
+  do {                                                                                                         \
+    cudaError_t e__ = cudaGetLastError();                                                                      \
+    if (e__ != cudaSuccess) return fail(c, MTSB_E_CUDA, "kernel launch (%s:%d): %s", __FILE__, __LINE__, cudaGetErrorString(e__)); \
+  } while (0)
+#define NEED(buf, n)                                                                       \
+  do {                                                                                     \
+    if ((buf).ensure(n)) return fail(c, MTSB_E_NOMEM, "cannot allocate %zu bytes for " #buf, (size_t)(n)); \
+  } while (0)
+
 
 struct Buf {
   void* p = nullptr;
   size_t cap = 0;
   bool host = false;
+  Buf() = default;
+  Buf(const Buf&) = delete;
+  Buf& operator=(const Buf&) = delete;
+  ~Buf() { release(); }
   int ensure(size_t n) {
     if (n <= cap) return 0;
     release();
@@ -44,13 +65,78 @@ struct Buf {
 static const int INDEX_TAIL = 16;                  // {segment bytes, k, magic, sum}: the end of both index formats (deflate.cuh)
 static const int INDEX_TAIL_V2 = 24;               // the second format has {sub-block bytes, step bytes} before it
 
+// The double-buffered copy pipeline of the host-buffer paths.  Sub-batch k's input goes up on copy_in into in[k & 1]
+// while the kernels work on the sub-batch before it, and its output comes down on copy_out from out[k & 1] while they
+// work on the next one.  A side whose pair is null is device memory that the kernels use in place.
+struct CopyPipe {
+  cudaStream_t stream = nullptr, copy_in = nullptr, copy_out = nullptr;   // the kernels' stream, H2D, D2H
+  cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr}, ev_done = nullptr;
+  Buf* in[2] = {nullptr, nullptr};     // the buffer pairs of the call in progress
+  Buf* out[2] = {nullptr, nullptr};
+  CopyPipe() = default;
+  CopyPipe(const CopyPipe&) = delete;
+  bool create(cudaStream_t compute) {
+    stream = compute;
+    if (cudaStreamCreateWithFlags(&copy_in, cudaStreamNonBlocking) != cudaSuccess ||
+        cudaStreamCreateWithFlags(&copy_out, cudaStreamNonBlocking) != cudaSuccess) return false;
+    for (int i = 0; i < 2; i++) { cudaEventCreateWithFlags(&ev_in[i], cudaEventDisableTiming); cudaEventCreateWithFlags(&ev_out[i], cudaEventDisableTiming); }
+    cudaEventCreateWithFlags(&ev_done, cudaEventDisableTiming);
+    return true;
+  }
+  ~CopyPipe() {
+    for (int i = 0; i < 2; i++) { if (ev_in[i]) cudaEventDestroy(ev_in[i]); if (ev_out[i]) cudaEventDestroy(ev_out[i]); }
+    if (ev_done) cudaEventDestroy(ev_done);
+    if (copy_in) cudaStreamDestroy(copy_in);
+    if (copy_out) cudaStreamDestroy(copy_out);
+  }
+  // takes the call's pairs (NEEDed by the caller) and queues the upload of sub-batch 0
+  int start(mtsb_ctx* c, Buf* in0, Buf* in1, Buf* out0, Buf* out1, const void* src0, size_t bytes0) {
+    in[0] = in0; in[1] = in1; out[0] = out0; out[1] = out1;
+    if (!in[0]) return 0;
+    // the copy-in stream must not start before work already queued on the caller's stream (e.g. producing `src`)
+    CK(cudaEventRecord(ev_done, stream));
+    CK(cudaStreamWaitEvent(copy_in, ev_done, 0));
+    return upload(c, 0, src0, bytes0);
+  }
+  int upload(mtsb_ctx* c, int k, const void* src, size_t bytes) {   // queues the upload of sub-batch k
+    if (!in[0]) return 0;
+    CK(cudaMemcpyAsync(in[k & 1]->p, src, bytes, cudaMemcpyHostToDevice, copy_in));
+    CK(cudaEventRecord(ev_in[k & 1], copy_in));
+    return 0;
+  }
+  int input(mtsb_ctx* c, int k, const void*& p) {   // p: sub-batch k's input, once its upload is done
+    if (in[0]) { CK(cudaStreamWaitEvent(stream, ev_in[k & 1], 0)); p = in[k & 1]->p; }
+    return 0;
+  }
+  int output(mtsb_ctx* c, int k, void*& p) {        // p: where sub-batch k's output goes, once it is free
+    if (!out[0]) return 0;
+    if (k >= 2) CK(cudaStreamWaitEvent(stream, ev_out[k & 1], 0));   // D2H of sub-batch k-2 has drained it
+    p = out[k & 1]->p;
+    return 0;
+  }
+  int download(mtsb_ctx* c, int k, void* dst, size_t bytes) {   // queues the download of sub-batch k, whose kernels are done
+    if (!out[0]) return 0;
+    CK(cudaMemcpyAsync(dst, out[k & 1]->p, bytes, cudaMemcpyDeviceToHost, copy_out));
+    CK(cudaEventRecord(ev_out[k & 1], copy_out));
+    return 0;
+  }
+  int finish(mtsb_ctx* c) { if (out[0]) CK(cudaStreamSynchronize(copy_out)); return 0; }   // waits for the last download
+};
+
+// The sub-batches of a call: chunks [first[k], first[k + 1]); max_in / max_out: the largest input / output of one
+struct Batches {
+  std::vector<int> first;
+  long long max_in = 0, max_out = 0;
+  int count() const { return (int)first.size() - 1; }
+};
+
 }  // namespace
 
 struct mtsb_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
-  int sm_count = 148;
+  long long sm_count = 148;
   std::string err;
   // params
   long long par_inflate = 1;   // decode index-less zlib streams block-parallel (inflate_par.cuh)
@@ -58,11 +144,11 @@ struct mtsb_ctx {
   long long par_cells = -1;     // index-less streams: -1 by stream count, 1 = blocks resolved in parallel into cells, 0 = chain of tiles
   long long par_lz_wide = -1;   // LZ resolve kernel shape: -1 by stream count, 1 = 1024-thread CTAs, 0 = 256-thread CTAs
   long long par_batch_bytes = 2ll << 30;   // host-buffer sub-batch of index-less chunks (output bytes): large enough to amortise the block search
-  long long par_stats[4] = {0, 0, 0, 0};   // last call: survivors, candidates, chained blocks, streams resumed
+  // last call: survivors of the block search, candidate blocks, chained blocks, streams resumed
+  long long par_survivors = 0, par_candidates = 0, par_chained = 0, par_resumed = 0;
   long long seg_bytes = 262144, batch_bytes = 2ll << 30, host_batch_bytes = 512ll << 20, write_index = 1;
-  cudaStream_t copy_in = nullptr, copy_out = nullptr;   // H2D / D2H streams of the host-buffer paths
-  cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr}, ev_done = nullptr;
-  int lz_ctas_per_sm = 2;
+  CopyPipe io;
+  long long lz_ctas_per_sm = 2;
   // device scratch
   Buf d_pstreams, d_surv, d_cand, d_pcount, d_tokens, d_cells, d_ptab, d_plist, d_pbad;   // block-parallel inflate scratch
   std::vector<uint32_t> lz_adler;   // per segment of the current sub-batch: adler32 left by par_lz_kernel ...
@@ -75,7 +161,7 @@ struct mtsb_ctx {
   Buf d_raw, d_raw2, d_out2, d_comp2, d_T, d_tok, d_hist, d_codes, d_hdrs, d_tab, d_so, d_seg_adler, d_chunk_adler, d_chunk_off, d_out,
       d_partial, d_comp, d_status, d_tadler, d_gather, d_subabs, d_subtok, d_invstate, d_invcells;
   int inv_cells_isz = 0;           // element size of the launch that last wrote the look-back cells
-  unsigned inv_epoch = 0;          // epoch of the last inv_tile_kernel launch (tags its look-back cells)
+  long long inv_epoch = 0;         // epoch of the last inv_tile_kernel launch (tags its look-back cells)
   long long inv_order_block = 2;   // inv_tile_kernel: consecutive tiles of a chunk that get consecutive tickets
   long long inv_single_pass = 1;   // channel-major inverse transform in one pass (inv_tile_kernel); 0: tile sums + apply
   Buf h_tab, h_small;
@@ -89,6 +175,10 @@ struct mtsb_ctx {
   bool attr_set = false;
 
   mtsb_ctx() { h_tab.host = true; h_small.host = true; }
+  ~mtsb_ctx() {
+    for (cudaEvent_t e : ev_pool) cudaEventDestroy(e);
+    if (own_stream) cudaStreamDestroy(stream);
+  }
   cudaEvent_t ev() {
     if (ev_used == ev_pool.size()) { cudaEvent_t e; cudaEventCreate(&e); ev_pool.push_back(e); }
     return ev_pool[ev_used++];
@@ -119,21 +209,6 @@ int fail(mtsb_ctx* c, int code, const char* fmt, ...) {
   g_err = buf;
   return code;
 }
-
-#define CK(call)                                                                                     \
-  do {                                                                                               \
-    cudaError_t e__ = (call);                                                                        \
-    if (e__ != cudaSuccess) return fail(c, MTSB_E_CUDA, "%s: %s", #call, cudaGetErrorString(e__)); \
-  } while (0)
-#define CKL()                                                                                                  \
-  do {                                                                                                         \
-    cudaError_t e__ = cudaGetLastError();                                                                      \
-    if (e__ != cudaSuccess) return fail(c, MTSB_E_CUDA, "kernel launch (%s:%d): %s", __FILE__, __LINE__, cudaGetErrorString(e__)); \
-  } while (0)
-#define NEED(buf, n)                                                                       \
-  do {                                                                                     \
-    if ((buf).ensure(n)) return fail(c, MTSB_E_NOMEM, "cannot allocate %zu bytes for " #buf, (size_t)(n)); \
-  } while (0)
 
 int tile_rows(int nc, int isz, int extra_rows) {
   long long P = isz == 1 ? tile_pitch<uint8_t>(nc) : isz == 2 ? tile_pitch<uint16_t>(nc) : (nc | 1);
@@ -206,6 +281,49 @@ int small_copy(mtsb_ctx* c, void* dst, const void* src, size_t bytes) {
   CKL();
   return 0;
 }
+
+// A sub-batch's tables in one blob: each array starts at a 256-byte aligned offset.  stage() fills h_tab, upload()
+// copies it to d_tab with one small_copy.
+struct TableBlob {
+  struct Part { const void* src; size_t off, bytes; };
+  std::vector<Part> parts;
+  size_t bytes = 0;
+  template <class T> size_t add(const std::vector<T>& v) {
+    const size_t off = (bytes + 255) & ~(size_t)255;
+    parts.push_back(Part{v.data(), off, v.size() * sizeof(T)});
+    bytes = off + v.size() * sizeof(T);
+    return off;
+  }
+  int stage(mtsb_ctx* c) const {
+    NEED(c->h_tab, bytes);
+    NEED(c->d_tab, bytes);
+    for (const Part& p : parts) if (p.bytes) memcpy((char*)c->h_tab.p + p.off, p.src, p.bytes);
+    return 0;
+  }
+  int upload(mtsb_ctx* c) const { return small_copy(c, c->d_tab.p, c->h_tab.p, bytes); }
+  template <class T> static const T* dev(const mtsb_ctx* c, size_t off) { return (const T*)((const char*)c->d_tab.p + off); }
+};
+
+// Device words read back at the end of a step: add() queues a small_copy of each area to the next 16-byte aligned
+// offset of h_small (which the caller NEEDs large enough); after sync(), get(i) is the i-th area on the host.
+struct ReadBack {
+  mtsb_ctx* c;
+  std::vector<size_t> off;
+  size_t used = 0;
+  int rc = 0;
+  explicit ReadBack(mtsb_ctx* c_) : c(c_) {}
+  void add(const void* dev, size_t bytes) {
+    off.push_back(used);
+    if (!rc) rc = small_copy(c, (char*)c->h_small.p + used, dev, bytes);
+    used += (bytes + 15) & ~(size_t)15;
+  }
+  int sync() {
+    if (rc) return rc;
+    CK(cudaStreamSynchronize(c->stream));
+    return 0;
+  }
+  template <class T> const T* get(int i) const { return (const T*)((const char*)c->h_small.p + off[i]); }
+};
 
 // ---------------------------------------------------------------- launches shared by several entry points
 template <class T>
@@ -377,6 +495,39 @@ bool valid_common(mtsb_ctx* c, int n_chunks, const long long* rows, int nc, int 
   return true;
 }
 
+// mtsb_set_param / mtsb_get_param: the named fields and how a value is checked before it is stored
+// (P_RANGE: lo..hi else an error, P_MIN: at least lo else an error, P_CLAMP: clamped to lo..hi, P_BOOL: 0 / 1,
+// P_TRI: -1 automatic / 0 / 1, P_WORD: an unsigned 32-bit word, P_READ_ONLY: statistics and properties)
+enum ParamRule { P_RANGE, P_MIN, P_CLAMP, P_BOOL, P_TRI, P_WORD, P_READ_ONLY };
+struct Param { const char* name; long long mtsb_ctx::*field; ParamRule rule; long long lo, hi; };
+const Param PARAMS[] = {
+    {"seg_bytes", &mtsb_ctx::seg_bytes, P_RANGE, 4096, 1ll << 30},
+    {"batch_bytes", &mtsb_ctx::batch_bytes, P_MIN, 1 << 20, 0},
+    {"host_batch_bytes", &mtsb_ctx::host_batch_bytes, P_MIN, 1 << 20, 0},
+    {"par_batch_bytes", &mtsb_ctx::par_batch_bytes, P_MIN, 1 << 20, 0},
+    {"write_index", &mtsb_ctx::write_index, P_BOOL, 0, 0},
+    {"par_inflate", &mtsb_ctx::par_inflate, P_BOOL, 0, 0},
+    {"par_indexed", &mtsb_ctx::par_indexed, P_BOOL, 0, 0},
+    {"par_single_pass", &mtsb_ctx::par_single_pass, P_BOOL, 0, 0},
+    {"seg_v2", &mtsb_ctx::seg_v2, P_BOOL, 0, 0},
+    {"inv_single_pass", &mtsb_ctx::inv_single_pass, P_BOOL, 0, 0},
+    {"par_cells", &mtsb_ctx::par_cells, P_TRI, 0, 0},
+    {"par_lz_wide", &mtsb_ctx::par_lz_wide, P_TRI, 0, 0},
+    {"inv_order_block", &mtsb_ctx::inv_order_block, P_CLAMP, 1, 64},
+    {"lz_ctas_per_sm", &mtsb_ctx::lz_ctas_per_sm, P_CLAMP, 1, 8},
+    {"inv_epoch", &mtsb_ctx::inv_epoch, P_WORD, 0, 0},     // (tests: the wrap of the look-back epochs)
+    {"par_survivors", &mtsb_ctx::par_survivors, P_READ_ONLY, 0, 0},
+    {"par_candidates", &mtsb_ctx::par_candidates, P_READ_ONLY, 0, 0},
+    {"par_chained", &mtsb_ctx::par_chained, P_READ_ONLY, 0, 0},
+    {"par_resumed", &mtsb_ctx::par_resumed, P_READ_ONLY, 0, 0},
+    {"sm_count", &mtsb_ctx::sm_count, P_READ_ONLY, 0, 0},
+};
+const Param* find_param(const char* name) {
+  for (const Param& p : PARAMS)
+    if (!strcmp(p.name, name)) return &p;
+  return nullptr;
+}
+
 }  // namespace
 
 // =============================================================================================== basic API
@@ -405,15 +556,7 @@ mtsb_ctx* mtsb_create(int device_id, void* stream) {
     }
     c->own_stream = true;
   }
-  if (cudaStreamCreateWithFlags(&c->copy_in, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaStreamCreateWithFlags(&c->copy_out, cudaStreamNonBlocking) != cudaSuccess) {
-    fail(nullptr, MTSB_E_CUDA, "cudaStreamCreate failed"); mtsb_destroy(c); return nullptr;
-  }
-  for (int i = 0; i < 2; i++) {
-    cudaEventCreateWithFlags(&c->ev_in[i], cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&c->ev_out[i], cudaEventDisableTiming);
-  }
-  cudaEventCreateWithFlags(&c->ev_done, cudaEventDisableTiming);
+  if (!c->io.create(c->stream)) { fail(nullptr, MTSB_E_CUDA, "cudaStreamCreate failed"); mtsb_destroy(c); return nullptr; }
   if (set_attrs(c)) { g_err = c->err; mtsb_destroy(c); return nullptr; }
   return c;
 }
@@ -422,18 +565,6 @@ void mtsb_destroy(mtsb_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
-  Buf* bufs[] = {&c->d_pstreams, &c->d_surv, &c->d_cand, &c->d_pcount, &c->d_tokens, &c->d_cells, &c->d_ptab, &c->d_plist, &c->d_pbad,
-                 &c->d_segv2, &c->d_btab, &c->d_subout, &c->d_pieces,
-                 &c->d_raw, &c->d_raw2, &c->d_out2, &c->d_comp2, &c->d_T, &c->d_tok, &c->d_hist, &c->d_codes, &c->d_hdrs, &c->d_tab, &c->d_so,
-                 &c->d_seg_adler, &c->d_chunk_adler, &c->d_chunk_off, &c->d_out, &c->d_partial, &c->d_comp,
-                 &c->d_status, &c->d_tadler, &c->d_gather, &c->d_subabs, &c->d_subtok, &c->d_invstate, &c->d_invcells, &c->h_tab, &c->h_small};
-  for (Buf* b : bufs) b->release();
-  for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
-  for (int i = 0; i < 2; i++) { if (c->ev_in[i]) cudaEventDestroy(c->ev_in[i]); if (c->ev_out[i]) cudaEventDestroy(c->ev_out[i]); }
-  if (c->ev_done) cudaEventDestroy(c->ev_done);
-  if (c->copy_in) cudaStreamDestroy(c->copy_in);
-  if (c->copy_out) cudaStreamDestroy(c->copy_out);
-  if (c->own_stream) cudaStreamDestroy(c->stream);
   delete c;
 }
 
@@ -447,50 +578,26 @@ int mtsb_sync(mtsb_ctx* c) {
 
 int mtsb_set_param(mtsb_ctx* c, const char* name, long long v) {
   if (!c || !name) return MTSB_E_ARG;
-  std::string s(name);
-  if (s == "seg_bytes") { if (v < 4096 || v > (1ll << 30)) return fail(c, MTSB_E_ARG, "seg_bytes out of range"); c->seg_bytes = v; }
-  else if (s == "batch_bytes") { if (v < (1 << 20)) return fail(c, MTSB_E_ARG, "batch_bytes too small"); c->batch_bytes = v; }
-  else if (s == "host_batch_bytes") { if (v < (1 << 20)) return fail(c, MTSB_E_ARG, "host_batch_bytes too small"); c->host_batch_bytes = v; }
-  else if (s == "write_index") c->write_index = v ? 1 : 0;
-  else if (s == "par_inflate") c->par_inflate = v ? 1 : 0;
-  else if (s == "par_indexed") c->par_indexed = v ? 1 : 0;
-  else if (s == "par_single_pass") c->par_single_pass = v ? 1 : 0;
-  else if (s == "seg_v2") c->seg_v2 = v ? 1 : 0;
-  else if (s == "inv_single_pass") c->inv_single_pass = v ? 1 : 0;
-  else if (s == "inv_epoch") c->inv_epoch = (unsigned)v;          // (tests: the wrap of the look-back epochs)
-  else if (s == "inv_order_block") c->inv_order_block = std::min<long long>(std::max<long long>(v, 1), 64);
-  else if (s == "par_cells") c->par_cells = v < 0 ? -1 : (v ? 1 : 0);
-  else if (s == "par_lz_wide") c->par_lz_wide = v < 0 ? -1 : (v ? 1 : 0);
-  else if (s == "par_batch_bytes") { if (v < (1 << 20)) return fail(c, MTSB_E_ARG, "par_batch_bytes too small"); c->par_batch_bytes = v; }
-  else if (s == "lz_ctas_per_sm") c->lz_ctas_per_sm = (int)std::min<long long>(8, std::max<long long>(1, v));
-  else return fail(c, MTSB_E_ARG, "unknown parameter %s", name);
+  const Param* p = find_param(name);
+  if (!p || p->rule == P_READ_ONLY) return fail(c, MTSB_E_ARG, "unknown parameter %s", name);
+  switch (p->rule) {
+    case P_RANGE: if (v < p->lo || v > p->hi) return fail(c, MTSB_E_ARG, "%s out of range", name); break;
+    case P_MIN: if (v < p->lo) return fail(c, MTSB_E_ARG, "%s too small", name); break;
+    case P_CLAMP: v = std::min(std::max(v, p->lo), p->hi); break;
+    case P_BOOL: v = v ? 1 : 0; break;
+    case P_TRI: v = v < 0 ? -1 : (v ? 1 : 0); break;
+    case P_WORD: v = (unsigned)v; break;
+    default: break;
+  }
+  c->*(p->field) = v;
   return 0;
 }
 
 long long mtsb_get_param(mtsb_ctx* c, const char* name) {
   if (!c || !name) return MTSB_E_ARG;
-  std::string s(name);
-  if (s == "seg_bytes") return c->seg_bytes;
-  if (s == "batch_bytes") return c->batch_bytes;
-  if (s == "host_batch_bytes") return c->host_batch_bytes;
-  if (s == "write_index") return c->write_index;
-  if (s == "par_inflate") return c->par_inflate;
-  if (s == "par_lz_wide") return c->par_lz_wide;
-  if (s == "par_cells") return c->par_cells;
-  if (s == "par_indexed") return c->par_indexed;
-  if (s == "par_single_pass") return c->par_single_pass;
-  if (s == "seg_v2") return c->seg_v2;
-  if (s == "inv_single_pass") return c->inv_single_pass;
-  if (s == "inv_order_block") return c->inv_order_block;
-  if (s == "inv_epoch") return c->inv_epoch;
-  if (s == "par_batch_bytes") return c->par_batch_bytes;
-  if (s == "par_survivors") return c->par_stats[0];
-  if (s == "par_candidates") return c->par_stats[1];
-  if (s == "par_chained") return c->par_stats[2];
-  if (s == "par_resumed") return c->par_stats[3];
-  if (s == "lz_ctas_per_sm") return c->lz_ctas_per_sm;
-  if (s == "sm_count") return c->sm_count;
-  return MTSB_E_ARG;
+  const Param* p = find_param(name);
+  if (!p) return MTSB_E_ARG;
+  return c->*(p->field);
 }
 
 long long mtsb_compress_bound(mtsb_ctx* c, long long raw_bytes, long long ns, int nc, int itemsize, int flags) {
@@ -613,6 +720,136 @@ int mtsb_inverse_transform(mtsb_ctx* c, const void* src, int src_is_device, long
 }
 
 // =============================================================================================== compress
+// Compress sub-batches: bounded by batch_bytes; smaller when a host buffer is involved so that copies pipeline with
+// kernels.  Device-resident calls have nothing to overlap with: one large sub-batch keeps the persistent match-finder
+// CTAs busy to the end (measured on 600 chunks: 2 GiB 99.9, 4 GiB 100.6, one 13.9 GB batch 101.7 GB/s).
+static Batches plan_encode_batches(const mtsb_ctx* c, int n_chunks, const long long* chunk_rows, long long row_bytes,
+                                   int itemsize, int flags, bool host_io) {
+  const long long sb_limit = host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : std::max<long long>(c->batch_bytes, 16ll << 30);
+  Batches sb;
+  for (int a = 0; a < n_chunks;) {
+    sb.first.push_back(a);
+    int b = a;
+    long long bb = 0, bd = 0;
+    while (b < n_chunks && b - a < 60000) {
+      long long ns = chunk_rows[b + 1] - chunk_rows[b], cb = ns * row_bytes;
+      if (b > a && bb + cb > sb_limit) break;
+      bb += cb; bd += chunk_bound(c, cb, seg_size_for(c, ns, itemsize, flags)); b++;
+    }
+    sb.max_in = std::max(sb.max_in, bb);
+    sb.max_out = std::max(sb.max_out, bd);
+    a = b;
+  }
+  sb.first.push_back(n_chunks);
+  return sb;
+}
+
+// One compress sub-batch: its chunks, their segments (the work units of the match finder and the encoder) and the
+// table blob [ChunkDesc nb][DeflateSeg n_segs][AdlerSeg n_segs][first nb+1]
+struct EncodeBatch {
+  int nb = 0, max_ns = 0, n_subs = 0;
+  long long bound = 0;            // worst-case output
+  std::vector<ChunkDesc> cds;
+  std::vector<DeflateSeg> segs;
+  std::vector<AdlerSeg> as;       // the segments' bytes, for the per-chunk adler32 fold
+  std::vector<int> first;         // chunk i's segments: [first[i], first[i + 1])
+  TableBlob tab;
+  size_t o_cd = 0, o_seg = 0, o_as = 0, o_first = 0;
+};
+
+static void plan_encode_tables(const mtsb_ctx* c, const long long* chunk_rows, int nc, int itemsize, int flags, int c0,
+                               int c1, EncodeBatch& b) {
+  const long long row_bytes = (long long)nc * itemsize, row0 = chunk_rows[c0];
+  b.nb = c1 - c0;
+  b.cds.resize(b.nb);
+  b.first.resize(b.nb + 1);
+  for (int i = 0; i < b.nb; i++) {
+    long long ns = chunk_rows[c0 + i + 1] - chunk_rows[c0 + i];
+    long long raw = ns * row_bytes;
+    long long seg = seg_size_for(c, ns, itemsize, flags);
+    int k = (int)((raw + seg - 1) / seg);
+    ChunkDesc& cd = b.cds[i];
+    cd.elem_off = (chunk_rows[c0 + i] - row0) * nc;
+    cd.ns = (int)ns;
+    cd.first_seg = (int)b.segs.size();
+    cd.n_seg = k;
+    cd.pad_ = (int)seg;
+    b.first[i] = (int)b.segs.size();
+    b.max_ns = std::max(b.max_ns, (int)ns);
+    long long base = cd.elem_off * itemsize;
+    for (int j = 0; j < k; j++) {
+      DeflateSeg s;
+      s.in_off = base + (long long)j * seg;
+      s.tok_off = s.in_off;
+      s.in_len = (int)std::min<long long>(seg, raw - (long long)j * seg);
+      s.chunk = i;
+      s.flags = (j == 0 ? SEG_FIRST : 0) | (j == k - 1 ? SEG_LAST : 0);
+      s.sub_first = b.n_subs;
+      b.n_subs += idx_n_sub(s.in_len);
+      b.segs.push_back(s);
+    }
+    b.bound += chunk_bound(c, raw, seg);
+  }
+  b.first[b.nb] = (int)b.segs.size();
+  b.as.resize(b.segs.size());
+  for (size_t i = 0; i < b.segs.size(); i++) b.as[i] = AdlerSeg{b.segs[i].in_off, b.segs[i].in_len, 0};
+  b.o_cd = b.tab.add(b.cds);
+  b.o_seg = b.tab.add(b.segs);
+  b.o_as = b.tab.add(b.as);
+  b.o_first = b.tab.add(b.first);
+}
+
+// The kernels that encode one sub-batch (its tables uploaded): forward transform of `raw` into d_T, match finder,
+// per-chunk adler32, Huffman tables, output offsets (d_chunk_off), encoder and, with write_index, the index trailers
+static int launch_encode(mtsb_ctx* c, const EncodeBatch& b, const void* raw, int nc, int itemsize, int flags,
+                         unsigned char* outp) {
+  const int nb = b.nb, n_segs = (int)b.segs.size();
+  const ChunkDesc* d_cd = TableBlob::dev<ChunkDesc>(c, b.o_cd);
+  const DeflateSeg* d_seg = TableBlob::dev<DeflateSeg>(c, b.o_seg);
+  const AdlerSeg* d_as = TableBlob::dev<AdlerSeg>(c, b.o_as);
+  const int* d_first = TableBlob::dev<int>(c, b.o_first);
+  c->begin(1);
+  if (int r = launch_fwd(c, itemsize, raw, c->d_T.p, d_cd, nb, b.max_ns, nc, flags)) return r;
+  c->end();
+  c->begin(3);
+  {
+    NEED(c->d_invstate, 256);
+    CK(cudaMemsetAsync(c->d_invstate.p, 0, 64, c->stream));    // the match finder's segment counter
+    const int grid = (int)std::min<long long>(n_segs, c->sm_count * c->lz_ctas_per_sm);
+    auto k = itemsize == 2 ? lz77_kernel<2, LZ_NT> : lz77_kernel<1, LZ_NT>;
+    const size_t smem = itemsize == 2 ? LzSmem<2, LZ_NT>::total : LzSmem<1, LZ_NT>::total;
+    MTS_LAUNCH(k, dim3(grid), dim3(LZ_NT + 32), smem, c->stream, (const unsigned char*)c->d_T.p, d_seg, n_segs, (unsigned short*)c->d_tok.p, (unsigned*)c->d_hist.p, (DeflateSegOut*)c->d_so.p, (unsigned*)c->d_seg_adler.p, c->write_index ? (unsigned long long*)c->d_subtok.p : (unsigned long long*)nullptr, (unsigned*)c->d_invstate.p);
+    CKL();
+    c->launches++;
+  }
+  c->end();
+  c->begin(4);
+  // the match finder left each segment's adler32 (it streams every byte of T anyway): fold them per chunk
+  MTS_LAUNCH(adler_combine_kernel, dim3((nb + 127) / 128), dim3(128), 0, c->stream, d_as, (const uint32_t*)c->d_seg_adler.p, d_first, nb, (uint32_t*)c->d_chunk_adler.p);
+  CKL();
+  c->launches++;
+  MTS_LAUNCH(huff_kernel, dim3(n_segs), dim3(32), 0, c->stream, d_seg, n_segs, (unsigned*)c->d_hist.p, (unsigned*)c->d_codes.p, (unsigned*)c->d_hdrs.p, (DeflateSegOut*)c->d_so.p);
+  CKL();
+  MTS_LAUNCH(scan_kernel, dim3(1), dim3(1024), 0, c->stream, d_seg, n_segs, (DeflateSegOut*)c->d_so.p, (long long*)c->d_chunk_off.p, nb, d_cd, (int)c->write_index);
+  CKL();
+  c->launches += 2;
+  c->end();
+  c->begin(5);
+  auto ek = itemsize == 2 ? encode_kernel<true> : encode_kernel<false>;
+  MTS_LAUNCH(ek, dim3(n_segs), dim3(ENC_THREADS), 0, c->stream, (const unsigned char*)c->d_T.p, d_seg, n_segs, (const unsigned short*)c->d_tok.p, (const unsigned*)c->d_codes.p, (const unsigned*)c->d_hdrs.p, (const DeflateSegOut*)c->d_so.p, (const unsigned*)c->d_chunk_adler.p, outp, (const unsigned long long*)c->d_subtok.p, c->write_index ? (unsigned long long*)c->d_subabs.p : (unsigned long long*)nullptr);
+  CKL();
+  c->launches++;
+  if (c->write_index) {
+    MTS_LAUNCH(trailer_kernel, dim3(nb), dim3(128), 0, c->stream, d_seg, (const DeflateSegOut*)c->d_so.p, d_cd,
+               (const long long*)c->d_chunk_off.p, (const unsigned long long*)c->d_subabs.p, outp,
+               (unsigned)(LZ_NT * (itemsize == 2 ? 2 : 1)));
+    CKL();
+    c->launches++;
+  }
+  c->end();
+  return 0;
+}
+
 int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_chunks, const long long* chunk_rows,
                          int nc, int itemsize, int flags, void* dst, int dst_is_device, long long dst_capacity,
                          long long* out_offsets) {
@@ -631,95 +868,24 @@ int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_
 
   out_offsets[0] = 0;
   long long total_out = 0;
-  // sub-batches: bounded by batch_bytes; smaller when a host buffer is involved so that copies pipeline with kernels
-  const bool host_io = !src_is_device || !dst_is_device;
-  // device-resident calls have nothing to overlap with: one large sub-batch keeps the persistent match-finder CTAs
-  // busy to the end (measured on 600 chunks: 2 GiB 99.9, 4 GiB 100.6, one 13.9 GB batch 101.7 GB/s)
-  const long long sb_limit = host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : std::max<long long>(c->batch_bytes, 16ll << 30);
-  std::vector<int> sb_first;
-  long long max_sb_bytes = 0, max_sb_bound = 0;
-  for (int a = 0; a < n_chunks;) {
-    sb_first.push_back(a);
-    int b = a;
-    long long bb = 0, bd = 0;
-    while (b < n_chunks && b - a < 60000) {
-      long long ns = chunk_rows[b + 1] - chunk_rows[b], cb = ns * row_bytes;
-      if (b > a && bb + cb > sb_limit) break;
-      bb += cb; bd += chunk_bound(c, cb, seg_size_for(c, ns, itemsize, flags)); b++;
-    }
-    max_sb_bytes = std::max(max_sb_bytes, bb);
-    max_sb_bound = std::max(max_sb_bound, bd);
-    a = b;
-  }
-  sb_first.push_back(n_chunks);
-  const int n_sb = (int)sb_first.size() - 1;
-  Buf* raw_buf[2] = {&c->d_raw, &c->d_raw2};
-  Buf* out_buf[2] = {&c->d_out, &c->d_out2};
-  if (!src_is_device) { NEED(c->d_raw, (size_t)max_sb_bytes + 256); if (n_sb > 1) NEED(c->d_raw2, (size_t)max_sb_bytes + 256); }
-  if (!dst_is_device) { NEED(c->d_out, (size_t)max_sb_bound + 256); if (n_sb > 1) NEED(c->d_out2, (size_t)max_sb_bound + 256); }
-  auto sb_bytes = [&](int k) { return (chunk_rows[sb_first[k + 1]] - chunk_rows[sb_first[k]]) * row_bytes; };
-  if (!src_is_device) {
-    // the copy-in stream must not start before work already queued on the caller's stream (e.g. producing `src`)
-    CK(cudaEventRecord(c->ev_done, c->stream));
-    CK(cudaStreamWaitEvent(c->copy_in, c->ev_done, 0));
-    CK(cudaMemcpyAsync(raw_buf[0]->p, (const char*)src, (size_t)sb_bytes(0), cudaMemcpyHostToDevice, c->copy_in));
-    CK(cudaEventRecord(c->ev_in[0], c->copy_in));
-  }
+  const Batches sb = plan_encode_batches(c, n_chunks, chunk_rows, row_bytes, itemsize, flags, !src_is_device || !dst_is_device);
+  const int n_sb = sb.count();
+  if (!src_is_device) { NEED(c->d_raw, (size_t)sb.max_in + 256); if (n_sb > 1) NEED(c->d_raw2, (size_t)sb.max_in + 256); }
+  if (!dst_is_device) { NEED(c->d_out, (size_t)sb.max_out + 256); if (n_sb > 1) NEED(c->d_out2, (size_t)sb.max_out + 256); }
+  auto sb_src = [&](int k) { return (const char*)src + chunk_rows[sb.first[k]] * row_bytes; };
+  auto sb_bytes = [&](int k) { return (size_t)((chunk_rows[sb.first[k + 1]] - chunk_rows[sb.first[k]]) * row_bytes); };
+  CopyPipe& io = c->io;
+  if (int r = io.start(c, src_is_device ? nullptr : &c->d_raw, &c->d_raw2, dst_is_device ? nullptr : &c->d_out, &c->d_out2, sb_src(0), sb_bytes(0)))
+    return r;
   for (int k = 0; k < n_sb; k++) {
-    const int c0 = sb_first[k], c1 = sb_first[k + 1];
-    const long long bbytes = sb_bytes(k);
-    const int nb = c1 - c0;
-    const long long row0 = chunk_rows[c0];
-    // tables
-    std::vector<ChunkDesc> cds(nb);
-    std::vector<DeflateSeg> segs;
-    std::vector<int> first(nb + 1);
-    int max_ns = 0, n_subs = 0;
-    long long bound = 0;
-    for (int i = 0; i < nb; i++) {
-      long long ns = chunk_rows[c0 + i + 1] - chunk_rows[c0 + i];
-      long long raw = ns * row_bytes;
-      long long seg = seg_size_for(c, ns, itemsize, flags);
-      int k = (int)((raw + seg - 1) / seg);
-      cds[i].elem_off = (chunk_rows[c0 + i] - row0) * nc;
-      cds[i].ns = (int)ns;
-      cds[i].first_seg = (int)segs.size();
-      cds[i].n_seg = k;
-      cds[i].pad_ = (int)seg;
-      first[i] = (int)segs.size();
-      max_ns = std::max(max_ns, (int)ns);
-      long long base = cds[i].elem_off * itemsize;
-      for (int j = 0; j < k; j++) {
-        DeflateSeg s;
-        s.in_off = base + (long long)j * seg;
-        s.tok_off = s.in_off;
-        s.in_len = (int)std::min<long long>(seg, raw - (long long)j * seg);
-        s.chunk = i;
-        s.flags = (j == 0 ? SEG_FIRST : 0) | (j == k - 1 ? SEG_LAST : 0);
-        s.sub_first = n_subs;
-        n_subs += idx_n_sub(s.in_len);
-        segs.push_back(s);
-      }
-      bound += chunk_bound(c, raw, seg);
-    }
-    first[nb] = (int)segs.size();
-    const int n_segs = (int)segs.size();
-    // table blob: [ChunkDesc nb][DeflateSeg n_segs][AdlerSeg n_segs][first nb+1]
-    size_t o_cd = 0, o_seg = (o_cd + nb * sizeof(ChunkDesc) + 255) & ~(size_t)255;
-    size_t o_as = (o_seg + n_segs * sizeof(DeflateSeg) + 255) & ~(size_t)255;
-    size_t o_first = (o_as + n_segs * sizeof(AdlerSeg) + 255) & ~(size_t)255;
-    size_t tab_bytes = o_first + (nb + 1) * sizeof(int);
-    NEED(c->h_tab, tab_bytes);
-    NEED(c->d_tab, tab_bytes);
-    char* h = (char*)c->h_tab.p;
-    memcpy(h + o_cd, cds.data(), nb * sizeof(ChunkDesc));
-    memcpy(h + o_seg, segs.data(), n_segs * sizeof(DeflateSeg));
-    AdlerSeg* as = (AdlerSeg*)(h + o_as);
-    for (int i = 0; i < n_segs; i++) { as[i].off = segs[i].in_off; as[i].len = segs[i].in_len; as[i].pad_ = 0; }
-    memcpy(h + o_first, first.data(), (nb + 1) * sizeof(int));
+    const int c0 = sb.first[k];
+    EncodeBatch b;
+    plan_encode_tables(c, chunk_rows, nc, itemsize, flags, c0, sb.first[k + 1], b);
+    const int nb = b.nb, n_segs = (int)b.segs.size();
+    if (int r = b.tab.stage(c)) return r;
     // scratch
-    NEED(c->d_T, (size_t)bbytes + 16384);
-    NEED(c->d_tok, (size_t)bbytes * 2 + 4096);
+    NEED(c->d_T, sb_bytes(k) + 16384);
+    NEED(c->d_tok, sb_bytes(k) * 2 + 4096);
     NEED(c->d_hist, (size_t)n_segs * HIST_STRIDE * 4);
     NEED(c->d_codes, (size_t)n_segs * CODE_STRIDE * 4);
     NEED(c->d_hdrs, (size_t)n_segs * HDR_WORDS * 4);
@@ -727,94 +893,34 @@ int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_
     NEED(c->d_seg_adler, (size_t)n_segs * 4);
     NEED(c->d_chunk_adler, (size_t)nb * 4);
     NEED(c->d_chunk_off, (size_t)(nb + 1) * 8);
-    NEED(c->d_subabs, (size_t)n_subs * 8 + 64);
-    NEED(c->d_subtok, (size_t)n_subs * 8 + 64);
+    NEED(c->d_subabs, (size_t)b.n_subs * 8 + 64);
+    NEED(c->d_subtok, (size_t)b.n_subs * 8 + 64);
     NEED(c->h_small, (size_t)(nb + 1) * 8);
-    const char* d = (const char*)c->d_tab.p;
-    const ChunkDesc* d_cd = (const ChunkDesc*)(d + o_cd);
-    const DeflateSeg* d_seg = (const DeflateSeg*)(d + o_seg);
-    const AdlerSeg* d_as = (const AdlerSeg*)(d + o_as);
-    const int* d_first = (const int*)(d + o_first);
 
     c->begin(0);
-    { int rc_ = small_copy(c, c->d_tab.p, h, tab_bytes); if (rc_) return rc_; }
+    if (int r = b.tab.upload(c)) return r;
     // only now queue the next sub-batch's upload: the copy engine serves transfers in submission order, so the small
     // table upload above must not sit behind it
-    if (!src_is_device && k + 1 < n_sb) {
-      CK(cudaMemcpyAsync(raw_buf[(k + 1) & 1]->p, (const char*)src + chunk_rows[sb_first[k + 1]] * row_bytes,
-                         (size_t)sb_bytes(k + 1), cudaMemcpyHostToDevice, c->copy_in));
-      CK(cudaEventRecord(c->ev_in[(k + 1) & 1], c->copy_in));
+    if (k + 1 < n_sb) {
+      if (int r = io.upload(c, k + 1, sb_src(k + 1), sb_bytes(k + 1))) return r;
     }
-    const void* raw = (const char*)src + row0 * row_bytes;
-    if (!src_is_device) {
-      CK(cudaStreamWaitEvent(c->stream, c->ev_in[k & 1], 0));
-      raw = raw_buf[k & 1]->p;
-    }
+    const void* raw = sb_src(k);
+    if (int r = io.input(c, k, raw)) return r;
     c->end();
-    unsigned char* outp;
-    if (dst_is_device) outp = (unsigned char*)dst + total_out;
-    else {
-      if (k >= 2) CK(cudaStreamWaitEvent(c->stream, c->ev_out[k & 1], 0));   // D2H of sub-batch k-2 has drained it
-      outp = (unsigned char*)out_buf[k & 1]->p;
-    }
-
-    c->begin(1);
-    int r = launch_fwd(c, itemsize, raw, c->d_T.p, d_cd, nb, max_ns, nc, flags);
-    if (r) return r;
-    c->end();
-    c->begin(3);
-    {
-      NEED(c->d_invstate, 256);
-      CK(cudaMemsetAsync(c->d_invstate.p, 0, 64, c->stream));    // the match finder's segment counter
-      int grid = std::min(n_segs, c->sm_count * c->lz_ctas_per_sm);
-      if (itemsize == 2) {
-        auto k = lz77_kernel<2, LZ_NT>;
-        MTS_LAUNCH(k, dim3(grid), dim3(LZ_NT + 32), (LzSmem<2, LZ_NT>::total), c->stream, (const unsigned char*)c->d_T.p, d_seg, n_segs, (unsigned short*)c->d_tok.p, (unsigned*)c->d_hist.p, (DeflateSegOut*)c->d_so.p, (unsigned*)c->d_seg_adler.p, c->write_index ? (unsigned long long*)c->d_subtok.p : (unsigned long long*)nullptr, (unsigned*)c->d_invstate.p);
-      } else {
-        auto k = lz77_kernel<1, LZ_NT>;
-        MTS_LAUNCH(k, dim3(grid), dim3(LZ_NT + 32), (LzSmem<1, LZ_NT>::total), c->stream, (const unsigned char*)c->d_T.p, d_seg, n_segs, (unsigned short*)c->d_tok.p, (unsigned*)c->d_hist.p, (DeflateSegOut*)c->d_so.p, (unsigned*)c->d_seg_adler.p, c->write_index ? (unsigned long long*)c->d_subtok.p : (unsigned long long*)nullptr, (unsigned*)c->d_invstate.p);
-      }
-      CKL();
-      c->launches++;
-    }
-    c->end();
-    c->begin(4);
-    // the match finder left each segment's adler32 (it streams every byte of T anyway): fold them per chunk
-    MTS_LAUNCH(adler_combine_kernel, dim3((nb + 127) / 128), dim3(128), 0, c->stream, d_as, (const uint32_t*)c->d_seg_adler.p, d_first, nb, (uint32_t*)c->d_chunk_adler.p);
-    CKL();
-    c->launches++;
-    MTS_LAUNCH(huff_kernel, dim3(n_segs), dim3(32), 0, c->stream, d_seg, n_segs, (unsigned*)c->d_hist.p, (unsigned*)c->d_codes.p, (unsigned*)c->d_hdrs.p, (DeflateSegOut*)c->d_so.p);
-    CKL();
-    MTS_LAUNCH(scan_kernel, dim3(1), dim3(1024), 0, c->stream, d_seg, n_segs, (DeflateSegOut*)c->d_so.p, (long long*)c->d_chunk_off.p, nb, d_cd, (int)c->write_index);
-    CKL();
-    c->launches += 2;
-    c->end();
-    c->begin(5);
-    auto ek = itemsize == 2 ? encode_kernel<true> : encode_kernel<false>;
-    MTS_LAUNCH(ek, dim3(n_segs), dim3(ENC_THREADS), 0, c->stream, (const unsigned char*)c->d_T.p, d_seg, n_segs, (const unsigned short*)c->d_tok.p, (const unsigned*)c->d_codes.p, (const unsigned*)c->d_hdrs.p, (const DeflateSegOut*)c->d_so.p, (const unsigned*)c->d_chunk_adler.p, outp, (const unsigned long long*)c->d_subtok.p, c->write_index ? (unsigned long long*)c->d_subabs.p : (unsigned long long*)nullptr);
-    CKL();
-    c->launches++;
-    if (c->write_index) {
-      MTS_LAUNCH(trailer_kernel, dim3(nb), dim3(128), 0, c->stream, d_seg, (const DeflateSegOut*)c->d_so.p, d_cd,
-                 (const long long*)c->d_chunk_off.p, (const unsigned long long*)c->d_subabs.p, outp,
-                 (unsigned)(LZ_NT * (itemsize == 2 ? 2 : 1)));
-      CKL();
-      c->launches++;
-    }
-    c->end();
-    { int rc_ = small_copy(c, c->h_small.p, c->d_chunk_off.p, (size_t)(nb + 1) * 8); if (rc_) return rc_; }
-    CK(cudaStreamSynchronize(c->stream));
-    const long long* co = (const long long*)c->h_small.p;
-    if (co[nb] > bound) return fail(c, MTSB_E_CAPACITY, "internal: sub-batch output %lld exceeds bound %lld", co[nb], bound);
+    void* outp = (unsigned char*)dst + total_out;
+    if (int r = io.output(c, k, outp)) return r;
+    if (int r = launch_encode(c, b, raw, nc, itemsize, flags, (unsigned char*)outp)) return r;
+    ReadBack rb(c);
+    rb.add(c->d_chunk_off.p, (size_t)(nb + 1) * 8);
+    if (int r = rb.sync()) return r;
+    const long long* co = rb.get<long long>(0);
+    if (co[nb] > b.bound) return fail(c, MTSB_E_CAPACITY, "internal: sub-batch output %lld exceeds bound %lld", co[nb], b.bound);
     for (int i = 0; i < nb; i++) out_offsets[c0 + i + 1] = total_out + co[i + 1];
-    if (!dst_is_device) {
-      // the kernels of this sub-batch are complete (synchronised above): drain it on the copy-out stream
-      CK(cudaMemcpyAsync((char*)dst + total_out, outp, (size_t)co[nb], cudaMemcpyDeviceToHost, c->copy_out));
-      CK(cudaEventRecord(c->ev_out[k & 1], c->copy_out));
-    }
+    // the kernels of this sub-batch are complete (synchronised above): drain it on the copy-out stream
+    if (int r = io.download(c, k, (char*)dst + total_out, (size_t)co[nb])) return r;
     total_out += co[nb];
   }
-  if (!dst_is_device) CK(cudaStreamSynchronize(c->copy_out));
+  if (int r = io.finish(c)) return r;
   c->collect_timing();
   return 0;
 }
@@ -863,6 +969,211 @@ static int fetch_ranges(mtsb_ctx* c, const unsigned char* comp, int comp_is_devi
 
 static uint32_t rd32(const unsigned char* p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
 
+// The arguments of one mtsb_decompress_chunks call
+struct DecodeArgs {
+  const unsigned char* comp; int comp_is_device; const long long* comp_offsets;
+  int n_chunks; const long long* chunk_rows; int nc, itemsize, flags;
+  void* dst; int dst_is_device; long long row_bytes;
+};
+
+// What read_indexes found behind a chunk's zlib stream (the index formats are written by trailer_kernel, deflate.cuh).
+struct ChunkIndex {
+  int n_seg = 0;                 // segments; 0: no usable index, the chunk is decoded as one plain zlib stream
+  bool v2 = false;               // second format
+  unsigned step = 0;             // second format: the step bytes of its fast path, 0 where the fast path cannot be taken
+  long long seg_bytes = 0;       // output bytes of every segment but the last
+  long long sub_bytes = 0;       // second format: bytes of the sub-block table and the {sub-block bytes, step bytes} words
+  uint32_t adler = 0;            // stored adler32 of the chunk's transformed bytes
+  long long tab_off = 0;         // second format: where the sub-block table starts, from the start of the chunk
+  const unsigned char* lens = nullptr;   // the n_seg segment lengths (in the buffer read_indexes filled)
+};
+
+// Reads the index behind every chunk's zlib stream in two rounds: the 16-byte tails, then the adler32, sub-block table
+// and lengths of the chunks whose tail is plausible.  An index is only used when its lengths tile the stream body
+// exactly and match its checksum word; `bytes` holds what the records point to.
+static int read_indexes(mtsb_ctx* c, const DecodeArgs& a, std::vector<ChunkIndex>& ix, std::vector<unsigned char>& bytes) {
+  ix.assign(a.n_chunks, ChunkIndex());
+  std::vector<long long> off, pos;
+  std::vector<int> len, who;
+  std::vector<unsigned char> tails;
+  for (int i = 0; i < a.n_chunks; i++) {
+    long long l = a.comp_offsets[i + 1] - a.comp_offsets[i];
+    if (l >= 2 + 6 + 4 + INDEX_TAIL && !c->ignore_index) { off.push_back(a.comp_offsets[i + 1] - INDEX_TAIL); len.push_back(INDEX_TAIL); who.push_back(i); }
+  }
+  if (int r = fetch_ranges(c, a.comp, a.comp_is_device, off, len, tails, pos)) return r;
+  std::vector<int> who2;
+  std::vector<uint32_t> sum_word(a.n_chunks, 0);
+  off.clear();
+  len.clear();
+  for (size_t j = 0; j < who.size(); j++) {
+    const unsigned char* t = tails.data() + pos[j];
+    int i = who[j];
+    long long l = a.comp_offsets[i + 1] - a.comp_offsets[i];
+    long long raw = (a.chunk_rows[i + 1] - a.chunk_rows[i]) * a.row_bytes;
+    uint32_t sb = rd32(t), k = rd32(t + 4), magic = rd32(t + 8);
+    if ((magic != IDX_MAGIC_V1 && magic != IDX_MAGIC_V2) || sb == 0 || k == 0) continue;
+    if ((long long)k != (raw + sb - 1) / sb) continue;
+    // second format: the sub-block table lies before the k lengths, {sub-block bytes, step bytes} after them
+    long long extra = 0;
+    if (magic == IDX_MAGIC_V2) {
+      long long full = raw / sb, rem = raw - full * sb;
+      extra = 8 + 4 * (full * idx_n_sub(sb) + (rem ? idx_n_sub(rem) : 0));
+    }
+    if (8 + 4ll * k + INDEX_TAIL + extra >= l) continue;
+    ChunkIndex& x = ix[i];
+    x.n_seg = (int)k; x.seg_bytes = sb; x.sub_bytes = extra; x.v2 = magic == IDX_MAGIC_V2;
+    x.tab_off = l - INDEX_TAIL - 4ll * k - extra;
+    sum_word[i] = rd32(t + 12);
+    off.push_back(a.comp_offsets[i + 1] - INDEX_TAIL - 4ll * k - extra - 4);   // adler32 | [sub table] | k lengths | [2 words]
+    len.push_back((int)(4 * k + 4 + extra));
+    who2.push_back(i);
+  }
+  if (int r = fetch_ranges(c, a.comp, a.comp_is_device, off, len, bytes, pos)) return r;
+  // validate: lengths must tile the stream body exactly, and match the checksum word
+  for (size_t j = 0; j < who2.size(); j++) {
+    const int i = who2[j];
+    ChunkIndex& x = ix[i];
+    const unsigned char* p = bytes.data() + pos[j];
+    long long l = a.comp_offsets[i + 1] - a.comp_offsets[i];
+    unsigned long long sum = 0;
+    bool ok = true;
+    const unsigned char* lens = p + 4 + (x.v2 ? x.sub_bytes - 8 : 0);    // after the adler32 and the sub-block table
+    for (int q = 0; q < x.n_seg; q++) { uint32_t v = rd32(lens + 4 * q); if (v == 0) ok = false; sum += v; }
+    if (!ok || (long long)sum != l - 8 - 4ll * x.n_seg - INDEX_TAIL - x.sub_bytes || (uint32_t)sum != sum_word[i]) { x = ChunkIndex(); continue; }
+    x.adler = ((uint32_t)p[0] << 24) | (p[1] << 16) | (p[2] << 8) | p[3];
+    x.lens = lens;
+    if (x.v2) {
+      // the fast path needs the sub-block size this build uses and a sane step size; otherwise only the segment lengths are used
+      const uint32_t subb = rd32(lens + 4 * x.n_seg), stepb = rd32(lens + 4 * x.n_seg + 4);
+      const bool fast = subb == (uint32_t)IDX_SUB_BYTES && stepb >= 256 && stepb <= (uint32_t)IDX_SUB_BYTES / 2 && (stepb & (stepb - 1)) == 0;
+      x.step = fast ? stepb : 0;
+    }
+  }
+  return 0;
+}
+
+// Decompress sub-batches.  A sub-batch must also hold enough independent streams to fill the GPU: chunks without a
+// segment index (e.g. reference-written ones) are ONE serial stream each, so they are batched by count (up to 16 GiB of
+// output).  Device-resident calls have nothing to overlap with: they take the largest sub-batches (measured on 600
+// chunks: 2 GiB 62 GB/s, 4 GiB 75, 8 GiB 88, one 13.9 GB batch 96 — fewer, fuller waves of the block kernels).
+static Batches plan_decode_batches(const mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix) {
+  const bool host_io = !a.comp_is_device || !a.dst_is_device;
+  const long long min_streams = 8ll * c->sm_count, hard_limit = std::max<long long>(c->batch_bytes, 16ll << 30);
+  const long long sb_limit = host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : hard_limit;
+  // index-less chunks with host buffers: equal sub-batches of about par_batch_bytes
+  long long par_limit = std::max(sb_limit, c->par_batch_bytes);
+  bool small_first = false;                 // several sub-batches of index-less chunks: start with a small one
+  {
+    long long total_par = 0, max_cb = 0;
+    for (int i = 0; i < a.n_chunks; i++)
+      if (!ix[i].n_seg) { long long cb = (a.chunk_rows[i + 1] - a.chunk_rows[i]) * a.row_bytes; total_par += cb; max_cb = std::max(max_cb, cb); }
+    const long long n_par = std::max<long long>(1, (total_par + par_limit / 2) / par_limit);
+    par_limit = (total_par + n_par - 1) / n_par + max_cb;
+    small_first = n_par > 1;
+  }
+  Batches sb;
+  for (int i0 = 0; i0 < a.n_chunks;) {
+    sb.first.push_back(i0);
+    int i1 = i0;
+    long long bb = 0, streams = 0;
+    while (i1 < a.n_chunks && i1 - i0 < 60000) {
+      long long cb = (a.chunk_rows[i1 + 1] - a.chunk_rows[i1]) * a.row_bytes;
+      if (i1 > i0 && bb + cb > hard_limit) break;
+      // index-less chunks decoded block-parallel have thousands of independent blocks: with host buffers they are
+      // batched by bytes so that copies overlap the decode of the neighbouring sub-batches
+      const bool par_b = host_io && c->par_inflate && !ix[i1].n_seg;
+      // (the first sub-batch is a quarter of the others: its decode is the one thing the download cannot overlap)
+      if (i1 > i0 && par_b && bb + cb > ((i0 == 0 && small_first) ? par_limit / 4 : par_limit)) break;
+      if (i1 > i0 && !par_b && bb + cb > sb_limit && streams >= min_streams) break;
+      bb += cb; streams += ix[i1].n_seg ? ix[i1].n_seg : 1; i1++;
+    }
+    sb.max_out = std::max(sb.max_out, bb);
+    sb.max_in = std::max(sb.max_in, a.comp_offsets[i1] - a.comp_offsets[i0]);
+    i0 = i1;
+  }
+  sb.first.push_back(a.n_chunks);
+  return sb;
+}
+
+// One decompress sub-batch: its chunks and their inflate segments, which segments each decode phase takes, and what
+// the phases return
+struct DecodeBatch {
+  int c0 = 0, nb = 0, max_ns = 0;
+  std::vector<ChunkDesc> cds;
+  std::vector<InflateSeg> segs;
+  std::vector<int> first;        // chunk i's segments: [first[i], first[i + 1])
+  std::vector<int> whole;        // the segments that are a whole index-less chunk (plain zlib streams)
+  std::vector<int> v2_ids;       // the segments the second-format kernels take, described by v2 ...
+  std::vector<SegV2> v2;
+  std::vector<uint32_t> v2_ad;   // ... and the adler32 of each that they produced (v2_ok)
+  std::vector<char> v2_ok;
+  std::vector<uint32_t> adler;   // per chunk: the adler32 of its transformed bytes where it is known on the host (have_adler)
+  std::vector<char> have_adler;
+  std::vector<AdlerSeg> as;      // the bytes the adler kernels sum for the other chunks: chunk i's [as_first[i], as_first[i + 1])
+  std::vector<int> as_first;
+};
+
+static void plan_segments(const mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, int c0, int c1,
+                          DecodeBatch& b) {
+  const long long row0 = a.chunk_rows[c0], comp0 = a.comp_offsets[c0];
+  b.c0 = c0;
+  b.nb = c1 - c0;
+  b.cds.resize(b.nb);
+  b.first.resize(b.nb + 1);
+  for (int i = 0; i < b.nb; i++) {
+    const int g = c0 + i;
+    const ChunkIndex& x = ix[g];
+    long long ns = a.chunk_rows[g + 1] - a.chunk_rows[g], raw = ns * a.row_bytes;
+    ChunkDesc& cd = b.cds[i];
+    cd.elem_off = (a.chunk_rows[g] - row0) * a.nc;
+    cd.ns = (int)ns; cd.first_seg = 0; cd.n_seg = 0; cd.pad_ = 0;
+    b.max_ns = std::max(b.max_ns, (int)ns);
+    long long tbase = cd.elem_off * a.itemsize;
+    long long cbase = a.comp_offsets[g] - comp0, clen = a.comp_offsets[g + 1] - a.comp_offsets[g];
+    b.first[i] = (int)b.segs.size();
+    if (!x.n_seg) {
+      InflateSeg s;
+      s.in_off = cbase; s.in_len = (int)clen; s.out_off = tbase; s.out_len = (int)raw; s.flags = INF_ZLIB;
+      s.start_bit = 0; s.opos0 = 0; s.pad_ = 0;
+      b.whole.push_back((int)b.segs.size());
+      b.segs.push_back(s);
+      continue;
+    }
+    long long pos = cbase + 2;
+    long long tab = cbase + x.tab_off;   // the chunk's sub-block table (second format)
+    for (int j = 0; j < x.n_seg; j++) {
+      InflateSeg s;
+      s.in_off = pos; s.in_len = (int)rd32(x.lens + 4 * j);
+      s.out_off = tbase + (long long)j * x.seg_bytes;
+      s.out_len = (int)std::min<long long>(x.seg_bytes, raw - (long long)j * x.seg_bytes);
+      s.flags = 0; s.start_bit = 0; s.opos0 = 0; s.pad_ = 0;
+      if (x.step && c->seg_v2 && c->par_inflate && s.in_len < (1 << 28)) {
+        SegV2 v;
+        v.in_off = s.in_off; v.out_off = s.out_off; v.tab_off = tab; v.in_len = s.in_len; v.out_len = s.out_len;
+        v.sub_first = 0; v.step_bytes = x.step;
+        b.v2.push_back(v);
+        b.v2_ids.push_back((int)b.segs.size());
+      }
+      tab += 4ll * idx_n_sub(s.out_len);
+      pos += s.in_len;
+      b.segs.push_back(s);
+    }
+  }
+  b.first[b.nb] = (int)b.segs.size();
+}
+
+// Records the block-parallel result `r` of segment `s`: unless no block of it was resolved or its tokens were
+// inconsistent (then the serial kernel decodes it from its start), `s` becomes the tail that is left, with `flags`.
+static bool resume_tail(mtsb_ctx* c, InflateSeg& s, const ParRes& r, int flags) {
+  c->par_chained += r.n_done;
+  if (r.n_done == 0 || (r.flags & 2)) return false;
+  s.flags = flags;
+  s.start_bit = r.tail_bit;
+  s.opos0 = r.tail_out;
+  c->par_resumed++;
+  return true;
+}
+
 // The block-parallel decoder for the streams `ps` (segs[ids[i]] each).  blks == nullptr: plain zlib streams, the
 // blocks are searched for on the device (find -> validate into per-stream buckets -> sort).  Otherwise blks holds one
 // known block per stream (the indexed segments of GPU-written chunks).  No host round trip between the kernels: one
@@ -870,7 +1181,7 @@ static uint32_t rd32(const unsigned char* p) { return p[0] | (p[1] << 8) | (p[2]
 // rewritten as INF_RESUME tails; the others are left untouched (full serial decode).
 static int par_decode(mtsb_ctx* c, const unsigned char* dcomp, std::vector<InflateSeg>& segs, const std::vector<int>& ids,
                       const std::vector<ParStream>& ps, const std::vector<ParBlk>* blks, long long in_total, int max_in,
-                      unsigned char* dT, int zflag) {
+                      unsigned char* dT) {
   const int ns = (int)ps.size();
   if (ns == 0) return 0;
   // bucket of candidate blocks per stream: zlib level 6 closes a block about every 29 KB of output here; streams with
@@ -901,13 +1212,13 @@ static int par_decode(mtsb_ctx* c, const unsigned char* dcomp, std::vector<Infla
   NEED(c->h_tab, o_blk + (blks ? n_slots * sizeof(ParBlk) : 0) + 64);
   NEED(c->h_small, 4096 + (size_t)ns * (sizeof(ParRes) + 4) + 64);
   memcpy(c->h_tab.p, ps.data(), (size_t)ns * sizeof(ParStream));
-  { int r = small_copy(c, c->d_pstreams.p, c->h_tab.p, (size_t)ns * sizeof(ParStream)); if (r) return r; }
+  if (int r = small_copy(c, c->d_pstreams.p, c->h_tab.p, (size_t)ns * sizeof(ParStream))) return r;
   CK(cudaMemsetAsync(c->d_pcount.p, 0, 256, c->stream));           // [0] survivors, [4..5] token cursor
   const ParStream* d_ps = (const ParStream*)c->d_pstreams.p;
   unsigned* d_cnt = (unsigned*)c->d_pcount.p;
   if (blks) {
     memcpy((char*)c->h_tab.p + o_blk, blks->data(), n_slots * sizeof(ParBlk));
-    { int r = small_copy(c, c->d_plist.p, (char*)c->h_tab.p + o_blk, n_slots * sizeof(ParBlk)); if (r) return r; }
+    if (int r = small_copy(c, c->d_plist.p, (char*)c->h_tab.p + o_blk, n_slots * sizeof(ParBlk))) return r;
   } else {
     NEED(c->d_surv, surv_cap * 8);
     NEED(c->d_cand, o_keys + n_slots * 4);
@@ -962,26 +1273,22 @@ static int par_decode(mtsb_ctx* c, const unsigned char* dcomp, std::vector<Infla
     c->launches++;
   }
   c->launches++;
-  char* hs = (char*)c->h_small.p;
-  { int r = small_copy(c, hs, c->d_pcount.p, 64); if (r) return r; }
-  { int r = small_copy(c, hs + 4096, c->d_pbad.p, (size_t)ns * sizeof(ParRes)); if (r) return r; }
-  const size_t o_bc = 4096 + (((size_t)ns * sizeof(ParRes) + 15) & ~(size_t)15);
-  if (!blks) { int r = small_copy(c, hs + o_bc, c->d_cand.p, (size_t)ns * 4); if (r) return r; }
-  CK(cudaStreamSynchronize(c->stream));
+  ReadBack rb(c);
+  rb.add(c->d_pcount.p, 64);
+  rb.add(c->d_pbad.p, (size_t)ns * sizeof(ParRes));
+  if (!blks) rb.add(c->d_cand.p, (size_t)ns * 4);
+  if (int r = rb.sync()) return r;
   if (!blks) {
-    c->par_stats[0] += ((const unsigned*)hs)[0];
-    for (int i = 0; i < ns; i++) c->par_stats[1] += ((const unsigned*)(hs + o_bc))[i];
+    c->par_survivors += rb.get<unsigned>(0)[0];
+    const unsigned* bcount = rb.get<unsigned>(2);
+    for (int i = 0; i < ns; i++) c->par_candidates += bcount[i];
   }
-  const ParRes* res = (const ParRes*)(hs + 4096);
+  const int zflag = blks ? 0 : INF_ZLIB;
+  const ParRes* res = rb.get<ParRes>(1);
   for (int sidx = 0; sidx < ns; sidx++) {
     const ParRes& r = res[sidx];
-    c->par_stats[2] += r.n_done;
-    if (r.n_done == 0 || (r.flags & 2)) continue;              // full serial decode of this stream
     InflateSeg& s = segs[ids[sidx]];
-    s.flags = zflag | INF_RESUME | ((r.flags & 1) ? INF_NO_BLOCKS : 0);
-    s.start_bit = r.tail_bit;
-    s.opos0 = r.tail_out;
-    c->par_stats[3]++;
+    if (!resume_tail(c, s, r, zflag | INF_RESUME | ((r.flags & 1) ? INF_NO_BLOCKS : 0))) continue;
     if ((r.flags & 4) && zflag && r.tail_out == (unsigned)s.out_len && (size_t)ids[sidx] < c->lz_adler.size()) {
       c->lz_adler[ids[sidx]] = r.adler;          // the whole stream went through par_lz_kernel: its adler32 is known
       c->lz_adler_have[ids[sidx]] = 1;
@@ -990,27 +1297,30 @@ static int par_decode(mtsb_ctx* c, const unsigned char* dcomp, std::vector<Infla
   return 0;
 }
 
-// The indexed segments of GPU-written chunks (`ids`: indices into segs): every segment is one dynamic block at bit 0
-// followed by the empty stored block that byte-aligns the next segment (deflate.cuh), so the blocks are known without
-// any search; a segment stored uncompressed simply fails the header parse and stays serial.
-static int par_phase_indexed(mtsb_ctx* c, const unsigned char* dcomp, std::vector<InflateSeg>& segs, const std::vector<int>& ids,
-                             unsigned char* dT) {
+// Block-parallel decode of the segments `ids` (indices into segs) through par_decode.  indexed: the indexed segments of
+// GPU-written chunks: every segment is one dynamic block at bit 0 followed by the empty stored block that byte-aligns
+// the next segment (deflate.cuh), so the blocks are known without any search; a segment stored uncompressed simply
+// fails the header parse and stays serial.  Otherwise: whole plain zlib streams, whose blocks are searched for.
+static int par_phase(mtsb_ctx* c, const unsigned char* dcomp, std::vector<InflateSeg>& segs, const std::vector<int>& ids,
+                     bool indexed, unsigned char* dT) {
   const int ns = (int)ids.size();
   std::vector<ParStream> ps(ns);
-  std::vector<ParBlk> blks(ns);
+  std::vector<ParBlk> blks(indexed ? ns : 0);
   long long in_total = 0;
   int max_in = 0;
   for (int i = 0; i < ns; i++) {
     const InflateSeg& s = segs[ids[i]];
     ps[i].in_off = s.in_off; ps[i].out_off = s.out_off; ps[i].in_len = s.in_len; ps[i].out_len = s.out_len;
-    ps[i].first_bit = 0; ps[i].pad_ = 0;
-    ParBlk& b = blks[i];
-    b.stream = (unsigned)i; b.bit = 0; b.limit = (unsigned)s.in_len * 8u;
-    b.end_bit = 0; b.n_tok = 0; b.out_len = 0; b.flags = 0; b.pad_ = 0; b.tok_off = 0;
+    ps[i].first_bit = indexed ? 0 : 16; ps[i].pad_ = 0;     // (after the zlib header)
+    if (indexed) {
+      ParBlk& b = blks[i];
+      b.stream = (unsigned)i; b.bit = 0; b.limit = (unsigned)s.in_len * 8u;
+      b.end_bit = 0; b.n_tok = 0; b.out_len = 0; b.flags = 0; b.pad_ = 0; b.tok_off = 0;
+    }
     in_total += s.in_len;
     max_in = std::max(max_in, s.in_len);
   }
-  return par_decode(c, dcomp, segs, ids, ps, &blks, in_total, max_in, dT, 0);
+  return par_decode(c, dcomp, segs, ids, ps, indexed ? &blks : nullptr, in_total, max_in, dT);
 }
 
 // The indexed segments of chunks with the second index format: `ids` index into segs, v2[i] describes segs[ids[i]].
@@ -1038,7 +1348,7 @@ static int par_phase_v2(mtsb_ctx* c, const unsigned char* dcomp, std::vector<Inf
     NEED(c->h_tab, (size_t)ns * sizeof(SegV2) + 64);
     NEED(c->h_small, 4096 + (size_t)ns * (sizeof(ParRes) + 4) + 128);
     memcpy(c->h_tab.p, v2.data() + a, (size_t)ns * sizeof(SegV2));
-    { int r = small_copy(c, c->d_segv2.p, c->h_tab.p, (size_t)ns * sizeof(SegV2)); if (r) return r; }
+    if (int r = small_copy(c, c->d_segv2.p, c->h_tab.p, (size_t)ns * sizeof(SegV2))) return r;
     MTS_LAUNCH(seg_tokens_kernel, dim3(ns), dim3(32), 0, c->stream, dcomp, (const SegV2*)c->d_segv2.p, (unsigned*)c->d_tokens.p,
                (uint2*)c->d_btab.p, (SubOut*)c->d_subout.p, (ParRes*)c->d_pbad.p);
     CKL();
@@ -1047,44 +1357,215 @@ static int par_phase_v2(mtsb_ctx* c, const unsigned char* dcomp, std::vector<Inf
                (unsigned*)c->d_tadler.p);
     CKL();
     c->launches += 2;
-    char* hs = (char*)c->h_small.p;
-    const size_t o_ad = 4096 + (((size_t)ns * sizeof(ParRes) + 15) & ~(size_t)15);
-    { int r = small_copy(c, hs + 4096, c->d_pbad.p, (size_t)ns * sizeof(ParRes)); if (r) return r; }
-    { int r = small_copy(c, hs + o_ad, c->d_tadler.p, (size_t)ns * 4); if (r) return r; }
-    CK(cudaStreamSynchronize(c->stream));
-    const ParRes* res = (const ParRes*)(hs + 4096);
+    ReadBack rb(c);
+    rb.add(c->d_pbad.p, (size_t)ns * sizeof(ParRes));
+    rb.add(c->d_tadler.p, (size_t)ns * 4);
+    if (int r = rb.sync()) return r;
+    const ParRes* res = rb.get<ParRes>(0);
+    const uint32_t* ad = rb.get<uint32_t>(1);
     for (int i = 0; i < ns; i++) {
-      const ParRes& r = res[i];
-      c->par_stats[2] += r.n_done;
-      if (r.n_done == 0 || (r.flags & 2)) continue;             // full serial decode of this segment
+      if (!resume_tail(c, segs[ids[a + i]], res[i], INF_RESUME)) continue;
       seg_ok[a + i] = 1;
-      seg_ad[a + i] = ((const uint32_t*)(hs + o_ad))[i];
-      InflateSeg& sg = segs[ids[a + i]];
-      sg.flags = INF_RESUME;
-      sg.start_bit = r.tail_bit;
-      sg.opos0 = r.tail_out;
-      c->par_stats[3]++;
+      seg_ad[a + i] = ad[i];
     }
     a = b;
   }
   return 0;
 }
 
-// Block-parallel decode of the whole-stream segments `whole` (indices into segs): plain zlib streams.
-static int par_phase(mtsb_ctx* c, const unsigned char* dcomp, std::vector<InflateSeg>& segs, const std::vector<int>& whole,
-                     unsigned char* dT) {
-  const int ns = (int)whole.size();
-  std::vector<ParStream> ps(ns);
-  long long in_total = 0;
-  int max_in = 0;
-  for (int i = 0; i < ns; i++) {
-    const InflateSeg& s = segs[whole[i]];
-    ps[i].in_off = s.in_off; ps[i].out_off = s.out_off; ps[i].in_len = s.in_len; ps[i].out_len = s.out_len;
-    ps[i].first_bit = 16; ps[i].pad_ = 0;
-    in_total += s.in_len;
-    max_in = std::max(max_in, s.in_len);
+// (the block kernels address bits with 32-bit offsets: streams of 256 MB and more stay with the serial decoder)
+static const int PAR_MAX_IN = 1 << 28;
+
+// The segments the block kernels take as indexed ones: all but the whole streams, the segments the second-format
+// kernels turned into tails, and streams too long for them
+static std::vector<int> indexed_for_blocks(const DecodeBatch& b) {
+  std::vector<int> ids;
+  size_t wi = 0, vi = 0;
+  for (int j = 0; j < (int)b.segs.size(); j++) {
+    if (wi < b.whole.size() && b.whole[wi] == j) { wi++; continue; }
+    if (vi < b.v2_ids.size() && b.v2_ids[vi] == j) { vi++; if (b.segs[j].flags & INF_RESUME) continue; }
+    if (b.segs[j].in_len < PAR_MAX_IN) ids.push_back(j);
   }
-  return par_decode(c, dcomp, segs, whole, ps, nullptr, in_total, max_in, dT, INF_ZLIB);
+  return ids;
+}
+
+// The parallel decode phases of a sub-batch: plain streams, second-format segments, then the other indexed segments
+static int par_phases(mtsb_ctx* c, const unsigned char* dcomp, DecodeBatch& b) {
+  unsigned char* dT = (unsigned char*)c->d_T.p;
+  c->lz_adler.assign(b.segs.size(), 0);
+  c->lz_adler_have.assign(b.segs.size(), 0);
+  if (c->par_inflate && !b.whole.empty()) {
+    long long whole_in = 0;
+    std::vector<int> fit;
+    for (int w : b.whole) if (b.segs[w].in_len < PAR_MAX_IN) { whole_in += b.segs[w].in_len; fit.push_back(w); }
+    if (whole_in >= 65536) { int r = par_phase(c, dcomp, b.segs, fit, false, dT); if (r) return r; }
+  }
+  if (!b.v2_ids.empty()) { int r = par_phase_v2(c, dcomp, b.segs, b.v2_ids, b.v2, dT, b.v2_ad, b.v2_ok); if (r) return r; }
+  if (c->par_inflate && c->par_indexed && b.whole.size() < b.segs.size()) {
+    if (int r = par_phase(c, dcomp, b.segs, indexed_for_blocks(b), true, dT)) return r;
+  }
+  return 0;
+}
+
+// adler32 of A | B from adler32(A), adler32(B) and the length of B
+static uint32_t adler32_combine(uint32_t a, uint32_t b, uint32_t len_b) {
+  const uint32_t s1a = a & 0xffff, s2a = a >> 16, s1b = b & 0xffff, s2b = b >> 16;
+  const uint32_t s1 = (s1a + s1b + ADLER_BASE - 1) % ADLER_BASE;
+  const unsigned long long t = (unsigned long long)(len_b % ADLER_BASE) * ((s1a + ADLER_BASE - 1) % ADLER_BASE);
+  return ((uint32_t)((s2a + s2b + t) % ADLER_BASE) << 16) | s1;
+}
+
+// adler32 of each chunk's transformed bytes: folded on the host from the segments' sums where the second-format
+// kernels produced every segment of the chunk, taken from par_lz_kernel where it produced a plain stream completely,
+// summed by the adler kernels (b.as) otherwise
+static void fold_adlers(const mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, DecodeBatch& b) {
+  const int ASEG = 1 << 16;
+  b.adler.assign(b.nb, 0);
+  b.have_adler.assign(b.nb, 0);
+  b.as_first.resize(b.nb + 1);
+  size_t vi = 0;
+  for (int i = 0; i < b.nb; i++) {
+    bool all = b.first[i + 1] > b.first[i];
+    uint32_t ad = 1;
+    for (int j = b.first[i]; j < b.first[i + 1]; j++) {
+      while (vi < b.v2_ids.size() && b.v2_ids[vi] < j) vi++;
+      if (vi < b.v2_ids.size() && b.v2_ids[vi] == j && b.v2_ok[vi]) ad = adler32_combine(ad, b.v2_ad[vi], (uint32_t)b.segs[j].out_len);
+      else { all = false; break; }
+    }
+    if (!ix[b.c0 + i].n_seg && b.first[i + 1] == b.first[i] + 1 && c->lz_adler_have[b.first[i]]) {
+      all = true; ad = c->lz_adler[b.first[i]];          // a plain stream that par_lz_kernel produced completely
+    }
+    if (all) { b.have_adler[i] = 1; b.adler[i] = ad; }
+    const long long raw = (long long)b.cds[i].ns * a.row_bytes, tbase = b.cds[i].elem_off * a.itemsize;
+    b.as_first[i] = (int)b.as.size();
+    if (!all) for (long long o = 0; o < raw; o += ASEG) b.as.push_back(AdlerSeg{tbase + o, (int)std::min<long long>(ASEG, raw - o), 0});
+  }
+  b.as_first[b.nb] = (int)b.as.size();
+}
+
+// The serial inflate kernel over the segments (d_segs: their table on the device): it decodes the segments and tails
+// the parallel phases left, checks every segment's end and writes its status and, for zlib streams, the trailer's adler32
+static int serial_inflate(mtsb_ctx* c, const unsigned char* dcomp, const std::vector<InflateSeg>& segs, const InflateSeg* d_segs) {
+  const int n_segs = (int)segs.size();
+  // segments the second-format kernels finished completely need nothing from the serial kernel
+  int n_serial = 0;
+  for (const InflateSeg& sg : segs)
+    if (!((sg.flags & INF_RESUME) && !(sg.flags & INF_ZLIB) && sg.opos0 >= (unsigned)sg.out_len)) n_serial++;
+  if (!n_serial) {
+    CK(cudaMemsetAsync(c->d_status.p, 0, (size_t)n_segs * 4, c->stream));
+  } else if (n_segs >= 6 * c->sm_count) {
+    // many short streams: global-memory window, 2 warps per CTA, up to 64 warps per SM
+    auto k = inflate_kernel<false, 2>;
+    MTS_LAUNCH(k, dim3((n_segs + 1) / 2), dim3(64), 0, c->stream, dcomp, d_segs, n_segs, (unsigned char*)c->d_T.p, (int*)c->d_status.p, (unsigned*)c->d_tadler.p);
+    c->launches++;
+  } else {
+    // few long streams: shared-memory window, one warp per CTA
+    auto k = inflate_kernel<true, 1>;
+    MTS_LAUNCH(k, dim3(n_segs), dim3(32), 0, c->stream, dcomp, d_segs, n_segs, (unsigned char*)c->d_T.p, (int*)c->d_status.p, (unsigned*)c->d_tadler.p);
+    c->launches++;
+  }
+  CKL();
+  return 0;
+}
+
+// Each chunk's status: its first failing segment's, else INF_BAD_ADLER where the adler32 of its transformed bytes is not
+// the stored one (the index's, or the zlib trailer's the serial kernel read: ta).  st: the segments' statuses, ca: the
+// adler kernels' sums.  Returns whether a chunk failed.
+static bool chunk_verdicts(const DecodeBatch& b, const std::vector<ChunkIndex>& ix, const int* st, const uint32_t* ta,
+                           const uint32_t* ca, int* status) {
+  bool bad = false;
+  for (int i = 0; i < b.nb; i++) {
+    int s = 0;
+    for (int j = b.first[i]; j < b.first[i + 1] && !s; j++) s = st[j];
+    if (!s) {
+      const ChunkIndex& x = ix[b.c0 + i];
+      uint32_t want = x.n_seg ? x.adler : ta[b.first[i]];
+      if (want != (b.have_adler[i] ? b.adler[i] : ca[i])) s = INF_BAD_ADLER;
+    }
+    if (s) bad = true;
+    status[b.c0 + i] = s;
+  }
+  return bad;
+}
+
+// Sub-batch k: segments, parallel phases, serial inflate, adler32s, inverse transform, verdicts
+static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const Batches& sb, int k,
+                        int* status, bool& any_bad) {
+  CopyPipe& io = c->io;
+  const int c0 = sb.first[k], c1 = sb.first[k + 1];
+  const long long row0 = a.chunk_rows[c0], bbytes = (a.chunk_rows[c1] - row0) * a.row_bytes;
+  DecodeBatch b;
+  plan_segments(c, a, ix, c0, c1, b);
+  const int nb = b.nb, n_segs = (int)b.segs.size();
+  NEED(c->d_T, (size_t)bbytes + 16384);
+  c->begin(0);
+  if (k + 1 < sb.count()) {
+    const long long n0 = a.comp_offsets[sb.first[k + 1]], n1 = a.comp_offsets[sb.first[k + 2]];
+    if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0))) return r;
+  }
+  const void* in = a.comp + a.comp_offsets[c0];
+  if (int r = io.input(c, k, in)) return r;
+  const unsigned char* dcomp = (const unsigned char*)in;
+  c->end();
+  c->begin(2);
+  if (int r = par_phases(c, dcomp, b)) return r;
+  fold_adlers(c, a, ix, b);
+  TableBlob tab;
+  const size_t o_cd = tab.add(b.cds), o_seg = tab.add(b.segs), o_as = tab.add(b.as), o_first = tab.add(b.as_first);
+  if (int r = tab.stage(c)) return r;
+  const int n_as = (int)b.as.size();
+  NEED(c->d_status, (size_t)n_segs * 4);
+  NEED(c->d_tadler, (size_t)n_segs * 4);
+  NEED(c->d_seg_adler, (size_t)n_as * 4 + 64);
+  NEED(c->d_chunk_adler, (size_t)nb * 4);
+  NEED(c->h_small, (size_t)n_segs * 8 + (size_t)nb * 4 + 128);
+  const AdlerSeg* d_as = TableBlob::dev<AdlerSeg>(c, o_as);
+  if (int r = tab.upload(c)) return r;
+  if (int r = serial_inflate(c, dcomp, b.segs, TableBlob::dev<InflateSeg>(c, o_seg))) return r;
+  c->end();
+  c->begin(3);
+  if (n_as) {
+    MTS_LAUNCH(adler_partial_kernel, dim3(n_as), dim3(256), 0, c->stream, (const uint8_t*)c->d_T.p, d_as, (uint32_t*)c->d_seg_adler.p);
+    CKL();
+  }
+  MTS_LAUNCH(adler_combine_kernel, dim3((nb + 127) / 128), dim3(128), 0, c->stream, d_as, (const uint32_t*)c->d_seg_adler.p, TableBlob::dev<int>(c, o_first), nb, (uint32_t*)c->d_chunk_adler.p);
+  CKL();
+  c->launches += 2;
+  c->end();
+  void* outp = (char*)a.dst + row0 * a.row_bytes;
+  if (int r = io.output(c, k, outp)) return r;
+  c->begin(4);
+  if (int r = launch_inv(c, a.itemsize, c->d_T.p, outp, TableBlob::dev<ChunkDesc>(c, o_cd), nb, b.max_ns, a.nc, a.flags, (size_t)(bbytes / a.itemsize))) return r;
+  c->end();
+  ReadBack rb(c);
+  rb.add(c->d_status.p, (size_t)n_segs * 4);
+  rb.add(c->d_tadler.p, (size_t)n_segs * 4);
+  rb.add(c->d_chunk_adler.p, (size_t)nb * 4);
+  if (int r = rb.sync()) return r;
+  if (int r = io.download(c, k, (char*)a.dst + row0 * a.row_bytes, (size_t)bbytes)) return r;
+  if (chunk_verdicts(b, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), status)) any_bad = true;
+  return 0;
+}
+
+// A chunk that carries something that looks like an index but does not decode with it (bytes after a foreign zlib
+// stream that happen to pass the index checks) is still a valid chunk for zlib, which ignores what follows the stream:
+// each such chunk is decoded again as a plain stream before it is called corrupt.  any_bad: whether a chunk stays bad.
+static int redecode_misled(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, int* status, bool& any_bad) {
+  any_bad = false;
+  for (int i = 0; i < a.n_chunks; i++) {
+    if (!status[i]) continue;
+    if (!ix[i].n_seg) { any_bad = true; continue; }
+    const long long one_off[2] = {0, a.comp_offsets[i + 1] - a.comp_offsets[i]}, one_rows[2] = {0, a.chunk_rows[i + 1] - a.chunk_rows[i]};
+    int st = 0;
+    c->ignore_index = true;
+    const int rc = mtsb_decompress_chunks(c, a.comp + a.comp_offsets[i], a.comp_is_device, one_off, 1, one_rows, a.nc, a.itemsize,
+                                          a.flags, (char*)a.dst + a.chunk_rows[i] * a.row_bytes, a.dst_is_device, &st);
+    c->ignore_index = false;
+    if (rc != 0 && rc != MTSB_E_CORRUPT) return rc;
+    status[i] = st;
+    if (st) any_bad = true;
+  }
+  return 0;
 }
 
 int mtsb_decompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, const long long* comp_offsets,
@@ -1098,360 +1579,35 @@ int mtsb_decompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, c
   }
   cudaSetDevice(c->device);
   c->reset_timing();
-  for (long long& v : c->par_stats) v = 0;
-  const unsigned char* comp = (const unsigned char*)comp_;
-  const long long row_bytes = (long long)nc * itemsize;
+  c->par_survivors = c->par_candidates = c->par_chained = c->par_resumed = 0;
+  const DecodeArgs a{(const unsigned char*)comp_, comp_is_device, comp_offsets, n_chunks, chunk_rows, nc, itemsize, flags, dst,
+                     dst_is_device, (long long)nc * itemsize};
 
   // ---- plan: look for the segment index after each chunk's zlib stream
   c->begin(1);
-  std::vector<int> nseg(n_chunks, 0);
-  std::vector<long long> segb(n_chunks, 0), idx_extra(n_chunks, 0);
-  std::vector<char> idx_v2(n_chunks, 0);
-  std::vector<unsigned> idx_step(n_chunks, 0);
-  std::vector<unsigned char> tails, idx;
-  std::vector<long long> tpos, ipos;
-  {
-    std::vector<long long> off;
-    std::vector<int> len;
-    std::vector<int> who;
-    for (int i = 0; i < n_chunks; i++) {
-      long long l = comp_offsets[i + 1] - comp_offsets[i];
-      if (l >= 2 + 6 + 4 + INDEX_TAIL && !c->ignore_index) { off.push_back(comp_offsets[i + 1] - INDEX_TAIL); len.push_back(INDEX_TAIL); who.push_back(i); }
-    }
-    int r = fetch_ranges(c, comp, comp_is_device, off, len, tails, tpos);
-    if (r) return r;
-    std::vector<long long> off2, tail_by_chunk(n_chunks, -1);
-    std::vector<int> len2;
-    std::vector<int> who2;
-    for (size_t j = 0; j < who.size(); j++) {
-      const unsigned char* t = tails.data() + tpos[j];
-      int i = who[j];
-      tail_by_chunk[i] = tpos[j];
-      long long l = comp_offsets[i + 1] - comp_offsets[i];
-      long long raw = (chunk_rows[i + 1] - chunk_rows[i]) * row_bytes;
-      uint32_t sb = rd32(t), k = rd32(t + 4), magic = rd32(t + 8);
-      if ((magic != IDX_MAGIC_V1 && magic != IDX_MAGIC_V2) || sb == 0 || k == 0) continue;
-      if ((long long)k != (raw + sb - 1) / sb) continue;
-      // second format: {sub-block bytes, step bytes} and the sub-block table lie before the k lengths
-      long long extra = 0;
-      if (magic == IDX_MAGIC_V2) {
-        long long full = raw / sb, rem = raw - full * sb;
-        extra = 8 + 4 * (full * idx_n_sub(sb) + (rem ? idx_n_sub(rem) : 0));
-      }
-      if (8 + 4ll * k + INDEX_TAIL + extra >= l) continue;
-      nseg[i] = (int)k; segb[i] = sb; idx_extra[i] = extra; idx_v2[i] = magic == IDX_MAGIC_V2;
-      off2.push_back(comp_offsets[i + 1] - INDEX_TAIL - 4ll * k - extra - 4);   // adler32 | [sub table] | k lengths | [2 words]
-      len2.push_back((int)(4 * k + 4 + extra));
-      who2.push_back(i);
-    }
-    r = fetch_ranges(c, comp, comp_is_device, off2, len2, idx, ipos);
-    if (r) return r;
-    // validate: lengths must tile the stream body exactly, and match the checksum word
-    std::vector<long long> ipos_by_chunk(n_chunks, -1);
-    for (size_t j = 0; j < who2.size(); j++) {
-      int i = who2[j];
-      const unsigned char* p = idx.data() + ipos[j];
-      const unsigned char* t = tails.data() + tail_by_chunk[i];
-      long long l = comp_offsets[i + 1] - comp_offsets[i];
-      unsigned long long sum = 0;
-      bool ok = true;
-      const unsigned char* lens = p + 4 + (idx_v2[i] ? idx_extra[i] - 8 : 0);    // after the adler32 and the sub-block table
-      for (int q = 0; q < nseg[i]; q++) { uint32_t v = rd32(lens + 4 * q); if (v == 0) ok = false; sum += v; }
-      if (!ok || (long long)sum != l - 8 - 4ll * nseg[i] - INDEX_TAIL - idx_extra[i] || (uint32_t)sum != rd32(t + 12)) { nseg[i] = 0; continue; }
-      if (idx_v2[i]) {
-        // the fast path needs the sub-block size this build uses and a sane step size; otherwise only the segment lengths are used
-        const uint32_t subb = rd32(lens + 4 * nseg[i]), stepb = rd32(lens + 4 * nseg[i] + 4);
-        const bool fast = subb == (uint32_t)IDX_SUB_BYTES && stepb >= 256 && stepb <= (uint32_t)IDX_SUB_BYTES / 2 && (stepb & (stepb - 1)) == 0;
-        idx_step[i] = fast ? stepb : 0;
-      }
-      ipos_by_chunk[i] = ipos[j];
-    }
-    for (int i = 0; i < n_chunks; i++) if (nseg[i] && ipos_by_chunk[i] < 0) nseg[i] = 0;
-    tpos.assign(ipos_by_chunk.begin(), ipos_by_chunk.end());   // reuse: tpos[i] = position of chunk i's index in idx
-  }
+  std::vector<ChunkIndex> ix;
+  std::vector<unsigned char> ix_bytes;
+  if (int r = read_indexes(c, a, ix, ix_bytes)) return r;
   c->end();
 
-  if (chunk_status) for (int i = 0; i < n_chunks; i++) chunk_status[i] = 0;
+  // every chunk's status, also when the caller does not ask for them
+  std::vector<int> own_status(chunk_status ? 0 : n_chunks);
+  int* status = chunk_status ? chunk_status : own_status.data();
+  for (int i = 0; i < n_chunks; i++) status[i] = 0;
+  const Batches sb = plan_decode_batches(c, a, ix);
+  const int n_sb = sb.count();
+  if (!comp_is_device) { NEED(c->d_comp, (size_t)sb.max_in + 256); if (n_sb > 1) NEED(c->d_comp2, (size_t)sb.max_in + 256); }
+  if (!dst_is_device) { NEED(c->d_out, (size_t)sb.max_out + 256); if (n_sb > 1) NEED(c->d_out2, (size_t)sb.max_out + 256); }
+  if (int r = c->io.start(c, comp_is_device ? nullptr : &c->d_comp, &c->d_comp2, dst_is_device ? nullptr : &c->d_out, &c->d_out2,
+                          a.comp + comp_offsets[0], (size_t)(comp_offsets[sb.first[1]] - comp_offsets[0])))
+    return r;
   bool any_bad = false;
-  const bool host_io = !comp_is_device || !dst_is_device;
-  // a sub-batch must also hold enough independent streams to fill the GPU: chunks without a segment index (e.g.
-  // reference-written ones) are ONE serial stream each, so they are batched by count (up to 16 GiB of output).
-  // Device-resident calls have nothing to overlap with: they take the largest sub-batches (measured on 600 chunks:
-  // 2 GiB 62 GB/s, 4 GiB 75, 8 GiB 88, one 13.9 GB batch 96 — fewer, fuller waves of the block kernels)
-  const long long min_streams = 8ll * c->sm_count, hard_limit = std::max<long long>(c->batch_bytes, 16ll << 30);
-  const long long sb_limit = host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : hard_limit;
-  // index-less chunks with host buffers: equal sub-batches of about par_batch_bytes
-  long long par_limit = std::max(sb_limit, c->par_batch_bytes);
-  bool small_first = false;                 // several sub-batches of index-less chunks: start with a small one
-  {
-    long long total_par = 0, max_cb = 0;
-    for (int i = 0; i < n_chunks; i++)
-      if (!nseg[i]) { long long cb = (chunk_rows[i + 1] - chunk_rows[i]) * row_bytes; total_par += cb; max_cb = std::max(max_cb, cb); }
-    const long long n_par = std::max<long long>(1, (total_par + par_limit / 2) / par_limit);
-    par_limit = (total_par + n_par - 1) / n_par + max_cb;
-    small_first = n_par > 1;
-  }
-  std::vector<int> sb_first;
-  long long max_sb_bytes = 0, max_sb_comp = 0;
-  for (int a = 0; a < n_chunks;) {
-    sb_first.push_back(a);
-    int b = a;
-    long long bb = 0, streams = 0;
-    while (b < n_chunks && b - a < 60000) {
-      long long cb = (chunk_rows[b + 1] - chunk_rows[b]) * row_bytes;
-      if (b > a && bb + cb > hard_limit) break;
-      // index-less chunks decoded block-parallel have thousands of independent blocks: with host buffers they are
-      // batched by bytes so that copies overlap the decode of the neighbouring sub-batches
-      const bool par_b = host_io && c->par_inflate && !nseg[b];
-      // (the first sub-batch is a quarter of the others: its decode is the one thing the download cannot overlap)
-      if (b > a && par_b && bb + cb > ((a == 0 && small_first) ? par_limit / 4 : par_limit)) break;
-      if (b > a && !par_b && bb + cb > sb_limit && streams >= min_streams) break;
-      bb += cb; streams += nseg[b] ? nseg[b] : 1; b++;
-    }
-    max_sb_bytes = std::max(max_sb_bytes, bb);
-    max_sb_comp = std::max(max_sb_comp, comp_offsets[b] - comp_offsets[a]);
-    a = b;
-  }
-  sb_first.push_back(n_chunks);
-  const int n_sb = (int)sb_first.size() - 1;
-  Buf* comp_buf[2] = {&c->d_comp, &c->d_comp2};
-  Buf* out_buf[2] = {&c->d_out, &c->d_out2};
-  if (!comp_is_device) { NEED(c->d_comp, (size_t)max_sb_comp + 256); if (n_sb > 1) NEED(c->d_comp2, (size_t)max_sb_comp + 256); }
-  if (!dst_is_device) { NEED(c->d_out, (size_t)max_sb_bytes + 256); if (n_sb > 1) NEED(c->d_out2, (size_t)max_sb_bytes + 256); }
-  if (!comp_is_device) {
-    CK(cudaEventRecord(c->ev_done, c->stream));
-    CK(cudaStreamWaitEvent(c->copy_in, c->ev_done, 0));
-    CK(cudaMemcpyAsync(comp_buf[0]->p, comp + comp_offsets[0], (size_t)(comp_offsets[sb_first[1]] - comp_offsets[0]),
-                       cudaMemcpyHostToDevice, c->copy_in));
-    CK(cudaEventRecord(c->ev_in[0], c->copy_in));
-  }
-  for (int k = 0; k < n_sb; k++) {
-    const int c0 = sb_first[k], c1 = sb_first[k + 1];
-    const long long bbytes = (chunk_rows[c1] - chunk_rows[c0]) * row_bytes;
-    const int nb = c1 - c0;
-    const long long row0 = chunk_rows[c0];
-    const long long comp0 = comp_offsets[c0], comp_bytes = comp_offsets[c1] - comp0;
-    std::vector<ChunkDesc> cds(nb);
-    std::vector<InflateSeg> segs;
-    std::vector<AdlerSeg> as;
-    std::vector<int> first(nb + 1), first_inf(nb + 1), whole, v2_ids;
-    std::vector<SegV2> v2;
-    std::vector<uint32_t> want_adler(nb, 0);
-    int max_ns = 0;
-    const int ASEG = 1 << 16;
-    for (int i = 0; i < nb; i++) {
-      int g = c0 + i;
-      long long ns = chunk_rows[g + 1] - chunk_rows[g], raw = ns * row_bytes;
-      cds[i].elem_off = (chunk_rows[g] - row0) * nc;
-      cds[i].ns = (int)ns; cds[i].first_seg = 0; cds[i].n_seg = 0; cds[i].pad_ = 0;
-      max_ns = std::max(max_ns, (int)ns);
-      long long tbase = cds[i].elem_off * itemsize;
-      long long cbase = comp_offsets[g] - comp0, clen = comp_offsets[g + 1] - comp_offsets[g];
-      first_inf[i] = (int)segs.size();
-      if (nseg[g]) {
-        const unsigned char* p = idx.data() + tpos[g];
-        want_adler[i] = ((uint32_t)p[0] << 24) | (p[1] << 16) | (p[2] << 8) | p[3];
-        const unsigned char* lens = p + 4 + (idx_v2[g] ? idx_extra[g] - 8 : 0);
-        long long pos = cbase + 2;
-        long long tab = cbase + clen - INDEX_TAIL - 4ll * nseg[g] - idx_extra[g];   // the chunk's sub-block table (second format)
-        for (int j = 0; j < nseg[g]; j++) {
-          InflateSeg s;
-          s.in_off = pos; s.in_len = (int)rd32(lens + 4 * j);
-          s.out_off = tbase + (long long)j * segb[g];
-          s.out_len = (int)std::min<long long>(segb[g], raw - (long long)j * segb[g]);
-          s.flags = 0; s.start_bit = 0; s.opos0 = 0; s.pad_ = 0;
-          if (idx_step[g] && c->seg_v2 && c->par_inflate && s.in_len < (1 << 28)) {
-            SegV2 v;
-            v.in_off = s.in_off; v.out_off = s.out_off; v.tab_off = tab; v.in_len = s.in_len; v.out_len = s.out_len;
-            v.sub_first = 0; v.step_bytes = idx_step[g];
-            v2.push_back(v);
-            v2_ids.push_back((int)segs.size());
-          }
-          tab += 4ll * idx_n_sub(s.out_len);
-          pos += s.in_len;
-          segs.push_back(s);
-        }
-      } else {
-        InflateSeg s;
-        s.in_off = cbase; s.in_len = (int)clen; s.out_off = tbase; s.out_len = (int)raw; s.flags = INF_ZLIB;
-        s.start_bit = 0; s.opos0 = 0; s.pad_ = 0;
-        whole.push_back((int)segs.size());
-        segs.push_back(s);
-      }
-    }
-    first_inf[nb] = (int)segs.size();
-    const int n_segs = (int)segs.size();
-    NEED(c->d_T, (size_t)bbytes + 16384);
-    c->begin(0);
-    if (!comp_is_device && k + 1 < n_sb) {
-      const int a = sb_first[k + 1], b = sb_first[k + 2];
-      CK(cudaMemcpyAsync(comp_buf[(k + 1) & 1]->p, comp + comp_offsets[a], (size_t)(comp_offsets[b] - comp_offsets[a]),
-                         cudaMemcpyHostToDevice, c->copy_in));
-      CK(cudaEventRecord(c->ev_in[(k + 1) & 1], c->copy_in));
-    }
-    const unsigned char* dcomp = comp + comp0;
-    if (!comp_is_device) {
-      CK(cudaStreamWaitEvent(c->stream, c->ev_in[k & 1], 0));
-      dcomp = (const unsigned char*)comp_buf[k & 1]->p;
-    }
-    c->end();
-    c->begin(2);
-    c->lz_adler.assign(n_segs, 0);
-    c->lz_adler_have.assign(n_segs, 0);
-    // (the block kernels address bits with 32-bit offsets: streams of 256 MB and more stay with the serial decoder)
-    const int PAR_MAX_IN = 1 << 28;
-    if (c->par_inflate && !whole.empty()) {
-      long long whole_in = 0;
-      std::vector<int> fit;
-      for (int w : whole) if (segs[w].in_len < PAR_MAX_IN) { whole_in += segs[w].in_len; fit.push_back(w); }
-      if (whole_in >= 65536) { int r = par_phase(c, dcomp, segs, fit, (unsigned char*)c->d_T.p); if (r) return r; }
-    }
-    std::vector<uint32_t> v2_ad;
-    std::vector<char> v2_ok;
-    if (!v2_ids.empty()) { int r = par_phase_v2(c, dcomp, segs, v2_ids, v2, (unsigned char*)c->d_T.p, v2_ad, v2_ok); if (r) return r; }
-    if (c->par_inflate && c->par_indexed && (int)whole.size() < n_segs) {
-      std::vector<int> ids;
-      size_t wi = 0, vi = 0;
-      for (int j = 0; j < n_segs; j++) {
-        if (wi < whole.size() && whole[wi] == j) { wi++; continue; }
-        if (vi < v2_ids.size() && v2_ids[vi] == j) { vi++; if (segs[j].flags & INF_RESUME) continue; }   // done by the second-format kernels
-        if (segs[j].in_len < PAR_MAX_IN) ids.push_back(j);
-      }
-      int r = par_phase_indexed(c, dcomp, segs, ids, (unsigned char*)c->d_T.p);
-      if (r) return r;
-    }
-    // adler32 of each chunk's transformed bytes: folded on the host from the segments' sums where the second-format
-    // kernels produced every segment of the chunk, taken from par_lz_kernel where it produced a plain stream completely,
-    // computed by the adler kernels otherwise
-    std::vector<uint32_t> host_adler(nb, 0);
-    std::vector<char> have_adler(nb, 0);
-    {
-      size_t vi = 0;
-      for (int i = 0; i < nb; i++) {
-        bool all = first_inf[i + 1] > first_inf[i];
-        uint32_t a = 1;
-        for (int j = first_inf[i]; j < first_inf[i + 1]; j++) {
-          while (vi < v2_ids.size() && v2_ids[vi] < j) vi++;
-          if (vi < v2_ids.size() && v2_ids[vi] == j && v2_ok[vi]) {
-            const uint32_t a2 = v2_ad[vi], len2 = (uint32_t)segs[j].out_len;
-            const uint32_t s1a = a & 0xffff, s2a = a >> 16, s1b = a2 & 0xffff, s2b = a2 >> 16;
-            const uint32_t s1 = (s1a + s1b + ADLER_BASE - 1) % ADLER_BASE;
-            const unsigned long long t = (unsigned long long)(len2 % ADLER_BASE) * ((s1a + ADLER_BASE - 1) % ADLER_BASE);
-            a = ((uint32_t)((s2a + s2b + t) % ADLER_BASE) << 16) | s1;
-          } else { all = false; break; }
-        }
-        if (!nseg[c0 + i] && first_inf[i + 1] == first_inf[i] + 1 && c->lz_adler_have[first_inf[i]]) {
-          all = true; a = c->lz_adler[first_inf[i]];          // a plain stream that par_lz_kernel produced completely
-        }
-        if (all) { have_adler[i] = 1; host_adler[i] = a; }
-        const long long raw = (long long)cds[i].ns * row_bytes, tbase = cds[i].elem_off * itemsize;
-        first[i] = (int)as.size();
-        if (!all) for (long long o = 0; o < raw; o += ASEG) as.push_back(AdlerSeg{tbase + o, (int)std::min<long long>(ASEG, raw - o), 0});
-      }
-      first[nb] = (int)as.size();
-    }
-    const int n_as = (int)as.size();
-    size_t o_cd = 0, o_seg = (o_cd + nb * sizeof(ChunkDesc) + 255) & ~(size_t)255;
-    size_t o_as = (o_seg + n_segs * sizeof(InflateSeg) + 255) & ~(size_t)255;
-    size_t o_first = (o_as + n_as * sizeof(AdlerSeg) + 255) & ~(size_t)255;
-    size_t tab_bytes = o_first + (nb + 1) * sizeof(int);
-    NEED(c->h_tab, tab_bytes);
-    NEED(c->d_tab, tab_bytes);
-    char* h = (char*)c->h_tab.p;
-    memcpy(h + o_cd, cds.data(), nb * sizeof(ChunkDesc));
-    memcpy(h + o_seg, segs.data(), n_segs * sizeof(InflateSeg));
-    memcpy(h + o_as, as.data(), n_as * sizeof(AdlerSeg));
-    memcpy(h + o_first, first.data(), (nb + 1) * sizeof(int));
-    NEED(c->d_status, (size_t)n_segs * 4);
-    NEED(c->d_tadler, (size_t)n_segs * 4);
-    NEED(c->d_seg_adler, (size_t)n_as * 4 + 64);
-    NEED(c->d_chunk_adler, (size_t)nb * 4);
-    NEED(c->h_small, (size_t)n_segs * 8 + (size_t)nb * 4 + 128);
-    const char* d = (const char*)c->d_tab.p;
-    const ChunkDesc* d_cd = (const ChunkDesc*)(d + o_cd);
-    { int rc_ = small_copy(c, c->d_tab.p, h, tab_bytes); if (rc_) return rc_; }
-    // segments the second-format kernels finished completely need nothing from the serial kernel
-    int n_serial = 0;
-    for (const InflateSeg& sg : segs)
-      if (!((sg.flags & INF_RESUME) && !(sg.flags & INF_ZLIB) && sg.opos0 >= (unsigned)sg.out_len)) n_serial++;
-    if (!n_serial) {
-      CK(cudaMemsetAsync(c->d_status.p, 0, (size_t)n_segs * 4, c->stream));
-    } else if (n_segs >= 6 * c->sm_count) {
-      // many short streams: global-memory window, 2 warps per CTA, up to 64 warps per SM
-      auto k = inflate_kernel<false, 2>;
-      MTS_LAUNCH(k, dim3((n_segs + 1) / 2), dim3(64), 0, c->stream, dcomp, (const InflateSeg*)(d + o_seg), n_segs, (unsigned char*)c->d_T.p, (int*)c->d_status.p, (unsigned*)c->d_tadler.p);
-      c->launches++;
-    } else {
-      // few long streams: shared-memory window, one warp per CTA
-      auto k = inflate_kernel<true, 1>;
-      MTS_LAUNCH(k, dim3(n_segs), dim3(32), 0, c->stream, dcomp, (const InflateSeg*)(d + o_seg), n_segs, (unsigned char*)c->d_T.p, (int*)c->d_status.p, (unsigned*)c->d_tadler.p);
-      c->launches++;
-    }
-    CKL();
-    c->end();
-    c->begin(3);
-    if (n_as) {
-      MTS_LAUNCH(adler_partial_kernel, dim3(n_as), dim3(256), 0, c->stream, (const uint8_t*)c->d_T.p, (const AdlerSeg*)(d + o_as), (uint32_t*)c->d_seg_adler.p);
-      CKL();
-    }
-    MTS_LAUNCH(adler_combine_kernel, dim3((nb + 127) / 128), dim3(128), 0, c->stream, (const AdlerSeg*)(d + o_as), (const uint32_t*)c->d_seg_adler.p, (const int*)(d + o_first), nb, (uint32_t*)c->d_chunk_adler.p);
-    CKL();
-    c->launches += 2;
-    c->end();
-    void* outp;
-    if (dst_is_device) outp = (char*)dst + row0 * row_bytes;
-    else {
-      if (k >= 2) CK(cudaStreamWaitEvent(c->stream, c->ev_out[k & 1], 0));   // D2H of sub-batch k-2 has drained it
-      outp = out_buf[k & 1]->p;
-    }
-    c->begin(4);
-    int r = launch_inv(c, itemsize, c->d_T.p, outp, d_cd, nb, max_ns, nc, flags, (size_t)(bbytes / itemsize));
-    if (r) return r;
-    c->end();
-    char* hs = (char*)c->h_small.p;
-    const size_t so_t = ((size_t)n_segs * 4 + 15) & ~(size_t)15, so_c = so_t + (((size_t)n_segs * 4 + 15) & ~(size_t)15);
-    { int rc_ = small_copy(c, hs, c->d_status.p, (size_t)n_segs * 4); if (rc_) return rc_; }
-    { int rc_ = small_copy(c, hs + so_t, c->d_tadler.p, (size_t)n_segs * 4); if (rc_) return rc_; }
-    { int rc_ = small_copy(c, hs + so_c, c->d_chunk_adler.p, (size_t)nb * 4); if (rc_) return rc_; }
-    CK(cudaStreamSynchronize(c->stream));
-    if (!dst_is_device) {
-      CK(cudaMemcpyAsync((char*)dst + row0 * row_bytes, outp, (size_t)bbytes, cudaMemcpyDeviceToHost, c->copy_out));
-      CK(cudaEventRecord(c->ev_out[k & 1], c->copy_out));
-    }
-    const int* st = (const int*)hs;
-    const uint32_t* ta = (const uint32_t*)(hs + so_t);
-    const uint32_t* ca = (const uint32_t*)(hs + so_c);
-    for (int i = 0; i < nb; i++) {
-      int s = 0;
-      for (int j = first_inf[i]; j < first_inf[i + 1] && !s; j++) s = st[j];
-      if (!s) {
-        uint32_t want = nseg[c0 + i] ? want_adler[i] : ta[first_inf[i]];
-        if (want != (have_adler[i] ? host_adler[i] : ca[i])) s = INF_BAD_ADLER;
-      }
-      if (s) any_bad = true;
-      if (chunk_status) chunk_status[c0 + i] = s;
-    }
-  }
-  if (!dst_is_device) CK(cudaStreamSynchronize(c->copy_out));
+  for (int k = 0; k < n_sb; k++)
+    if (int r = decode_batch(c, a, ix, sb, k, status, any_bad)) return r;
+  if (int r = c->io.finish(c)) return r;
   c->collect_timing();
   if (any_bad && chunk_status && !c->ignore_index) {
-    // A chunk that carries something that looks like an index but does not decode with it (bytes after a foreign zlib
-    // stream that happen to pass the index checks) is still a valid chunk for zlib, which ignores what follows the
-    // stream: decode it again as a plain stream before calling it corrupt.
-    any_bad = false;
-    for (int i = 0; i < n_chunks; i++) {
-      if (!chunk_status[i]) continue;
-      if (!nseg[i]) { any_bad = true; continue; }
-      const long long one_off[2] = {0, comp_offsets[i + 1] - comp_offsets[i]}, one_rows[2] = {0, chunk_rows[i + 1] - chunk_rows[i]};
-      int st = 0;
-      c->ignore_index = true;
-      const int rc = mtsb_decompress_chunks(c, comp + comp_offsets[i], comp_is_device, one_off, 1, one_rows, nc, itemsize, flags,
-                                            (char*)dst + chunk_rows[i] * row_bytes, dst_is_device, &st);
-      c->ignore_index = false;
-      if (rc != 0 && rc != MTSB_E_CORRUPT) return rc;
-      chunk_status[i] = st;
-      if (st) any_bad = true;
-    }
+    if (int r = redecode_misled(c, a, ix, status, any_bad)) return r;
   }
   if (any_bad) return fail(c, MTSB_E_CORRUPT, "at least one compressed chunk is corrupted");
   return 0;
