@@ -110,11 +110,25 @@ int mtsb_decompress_chunks(mtsb_ctx* ctx, const void* comp, int comp_is_device, 
                            int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags, void* dst,
                            int dst_is_device, int* chunk_status);
 
-/* Device-time (ms, CUDA events on the context's stream) of the stages of the last compress / decompress call:
+/* Integrity check — replaces the per-chunk compare of check() (mtscomp.py:866-888).  Chunk i is decoded exactly as
+ * mtsb_decompress_chunks decodes it and compared on the device with rows [chunk_rows[i], chunk_rows[i+1]) of the
+ * row-major array `ref` (host or device, itemsize-aligned); the decoded rows are not returned.  Integers: bit equality.
+ * MTSB_FLOAT: np.isclose(decoded, ref, rtol, atol) per element, evaluated as NumPy 2 evaluates it for Python-float
+ * tolerances: (|x - y| <= atol + rtol * |y| && isfinite(y)) || x == y in the element's precision, with atol and rtol
+ * rounded to it.  mismatches[i] / first_mismatch[i] (n_chunks host int64): elements that fail, and the element index
+ * within chunk i of the first one (-1: none).  chunk_status as in mtsb_decompress_chunks (never NULL here); a chunk
+ * that does not decode gets -1 in both arrays and the call returns MTSB_E_CORRUPT. */
+int mtsb_verify_chunks(mtsb_ctx* ctx, const void* comp, int comp_is_device, const long long* comp_offsets,
+                       int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags,
+                       const void* ref, int ref_is_device, double rtol, double atol,
+                       long long* mismatches, long long* first_mismatch, int* chunk_status);
+
+/* Device-time (ms, CUDA events on the context's stream) of the stages of the last compress / decompress / verify call:
  * out[0..7] = {h2d, transform, adler, lz77, huffman+scan, encode, d2h, total} for compress,
- *             {h2d, plan, inflate, adler, inverse, d2h, 0, total} for decompress.  Returns the number filled. */
+ *             {h2d, plan, inflate, adler, inverse, d2h, 0, total} for decompress,
+ *             {h2d, plan, inflate, adler, inverse, 0, compare, total} for verify.  Returns the number filled. */
 int mtsb_last_timings(mtsb_ctx* ctx, float* out, int n);
-/* Number of kernels launched by the last compress / decompress / transform call. */
+/* Number of kernels launched by the last compress / decompress / verify / transform call. */
 long long mtsb_last_launches(mtsb_ctx* ctx);
 
 /* Pinned host memory helpers (so that Python can stage file data without torch). */

@@ -26,7 +26,7 @@ E_CORRUPT = -5
 SYMBOLS = (
     'mtsb_version', 'mtsb_device_count', 'mtsb_create', 'mtsb_destroy', 'mtsb_last_error', 'mtsb_sync',
     'mtsb_set_param', 'mtsb_get_param', 'mtsb_compress_bound', 'mtsb_delta_transform', 'mtsb_inverse_transform',
-    'mtsb_compress_chunks', 'mtsb_decompress_chunks', 'mtsb_last_timings', 'mtsb_last_launches',
+    'mtsb_compress_chunks', 'mtsb_decompress_chunks', 'mtsb_verify_chunks', 'mtsb_last_timings', 'mtsb_last_launches',
     'mtsb_host_alloc', 'mtsb_host_free', 'mtsb_device_alloc', 'mtsb_device_free', 'mtsb_memcpy')
 
 
@@ -61,6 +61,8 @@ def _declare(lib):
     lib.mtsb_inverse_transform.argtypes = [vp, vp, i, ll, i, i, i, vp, i, C.POINTER(C.c_uint32)]
     lib.mtsb_compress_chunks.argtypes = [vp, vp, i, i, pll, i, i, i, vp, i, ll, pll]
     lib.mtsb_decompress_chunks.argtypes = [vp, vp, i, pll, i, pll, i, i, i, vp, i, C.POINTER(C.c_int)]
+    lib.mtsb_verify_chunks.argtypes = [vp, vp, i, pll, i, pll, i, i, i, vp, i, C.c_double, C.c_double, pll, pll,
+                                       C.POINTER(C.c_int)]
     lib.mtsb_last_timings.argtypes = [vp, C.POINTER(C.c_float), i]
     lib.mtsb_last_launches.argtypes = [vp]
     lib.mtsb_last_launches.restype = ll
@@ -236,6 +238,24 @@ class Codec:
                 self._check(rc)
         return status
 
+    def verify_ptr(self, comp, comp_is_device, comp_offsets, chunk_rows, nc, itemsize, flags, ref, ref_is_device,
+                   rtol, atol):
+        """Decode each chunk and compare it on the device with its rows of `ref` (mtsb_verify_chunks) ->
+        (status int32[n], mismatches int64[n], first_mismatch int64[n]); -1 in both counters where a chunk is corrupt."""
+        rows, offs = _i64(chunk_rows), _i64(comp_offsets)
+        n = len(rows) - 1
+        status = np.zeros(n, dtype=np.int32)
+        mism, first = np.zeros(n, dtype=np.int64), np.zeros(n, dtype=np.int64)
+        pll = C.POINTER(C.c_longlong)
+        with self.lock:
+            rc = self.lib.mtsb_verify_chunks(
+                self.ctx, C.c_void_p(comp), int(comp_is_device), offs.ctypes.data_as(pll), n,
+                rows.ctypes.data_as(pll), nc, itemsize, flags, C.c_void_p(ref), int(ref_is_device), float(rtol),
+                float(atol), mism.ctypes.data_as(pll), first.ctypes.data_as(pll), status.ctypes.data_as(C.POINTER(C.c_int)))
+            if rc != 0 and rc != E_CORRUPT:
+                self._check(rc)
+        return status, mism, first
+
     # -- NumPy conveniences (host arrays)
     def delta_transform(self, chunk, flags):
         chunk = np.ascontiguousarray(chunk)
@@ -280,6 +300,14 @@ class Codec:
         status = self.decompress_ptr(comp.ctypes.data, 0, comp_offsets, rows, nc, dtype.itemsize, _fl(flags, dtype),
                                      out.ctypes.data, 0)
         return out, status
+
+
+    def verify(self, comp, comp_offsets, chunk_rows, ref, flags, rtol=1e-5, atol=1e-16):
+        """comp: bytes-like; ref: C-contiguous (n_samples, nc) array -> (status, mismatches, first_mismatch)."""
+        ref = np.ascontiguousarray(ref)
+        comp = np.frombuffer(comp, dtype=np.uint8)
+        return self.verify_ptr(comp.ctypes.data, 0, comp_offsets, chunk_rows, ref.shape[1], ref.dtype.itemsize,
+                               _fl(flags, ref.dtype), ref.ctypes.data, 0, rtol, atol)
 
 
 _default = {}

@@ -10,7 +10,8 @@ CSRC = PKG / 'csrc'
 BUILD = PKG / '_build'
 LIB = BUILD / 'libmtscomp_b200.so'
 SOURCES = ['capi.cu']
-HEADERS = ['common.cuh', 'transform.cuh', 'deflate.cuh', 'inflate.cuh', 'inflate_par.cuh', 'inflate_seg.cuh', '../../include/mtscomp_b200.h']
+HEADERS = ['common.cuh', 'transform.cuh', 'deflate.cuh', 'inflate.cuh', 'inflate_par.cuh', 'inflate_seg.cuh', 'verify.cuh',
+           '../../include/mtscomp_b200.h']
 
 
 def _stale(target, deps):

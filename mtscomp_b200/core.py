@@ -33,6 +33,9 @@ from .rawio import load_raw_data
 
 _seek_lock = Lock()
 CRITICAL_ERROR_URL = "https://github.com/int-brain-lab/mtscomp/issues/new?title=Critical+error"
+CRITICAL_CHECK_FAILED = ("CRITICAL ERROR: automatic check failed when compressing the data. "
+                         "Report immediately to " + CRITICAL_ERROR_URL)
+CHECK_RTOL = 1e-5            # np.allclose's default, which the reference's check() uses for floats
 GPU_BATCH_CHUNKS = 64        # chunks handed to the GPU per call by Writer.write / Reader.tofile ...
 GPU_BATCH_BYTES = 256 << 20  # ... and at most this many raw bytes: the pinned staging (two raw + two compressed buffers in
                              # the Writer) stays near 1 GB -- pinning host memory costs about 0.7 s per GB on the B200 box
@@ -313,9 +316,7 @@ class Writer:
             try:
                 check(self.data, out, outmeta)
             except AssertionError:
-                raise RuntimeError(
-                    "CRITICAL ERROR: automatic check failed when compressing the data. "
-                    "Report immediately to " + CRITICAL_ERROR_URL)
+                raise RuntimeError(CRITICAL_CHECK_FAILED)
             logger.debug("Automatic integrity check after compression PASSED.")
         return ratio
 
@@ -496,11 +497,11 @@ class Reader:
         else:
             view[:] = np.frombuffer(self._pread(n, start), dtype=np.uint8)
 
-    def _stage_compressed(self, codec, spans):
-        """Read the .cbin ranges `spans` [(start, length)] back to back into the pinned 'r_comp' buffer (one read per
+    def _stage_compressed(self, codec, spans, name='r_comp'):
+        """Read the .cbin ranges `spans` [(start, length)] back to back into the pinned buffer `name` (one read per
         run of adjacent ranges) -> (buffer, offsets)."""
         offs = np.concatenate(([0], np.cumsum([length for _, length in spans]))).astype(np.int64)
-        buf = codec.host_buffer('r_comp', int(offs[-1]) + 64)
+        buf = codec.host_buffer(name, int(offs[-1]) + 64)
         k = 0
         while k < len(spans):
             j = k
@@ -780,26 +781,77 @@ class Reader:
 # High-level API
 # ------------------------------------------------------------------------------------------------------------------
 
+def _copy_rows(dst, src):
+    """dst[...] = src (same shape) with a few threads: np.copyto releases the GIL, and the source is usually a memory
+    map whose pages fault in as they are read."""
+    n = src.shape[0]
+    step = max(-(-n // 4), 1)
+    if src.nbytes < (4 << 20):
+        np.copyto(dst, src)
+        return
+    list(_read_pool().map(lambda a: np.copyto(dst[a:a + step], src[a:a + step]), range(0, n, step)))
+
+
+def _verify_range(reader, data, first, last):
+    """Check chunks [first, last) of the open `reader` against the rows of `data` on the GPU (mtsb_verify_chunks):
+    batches of _batch_ranges, whose compressed bytes and source rows are staged into pinned memory for batch k+1 while
+    the GPU verifies batch k.  Integers must be equal, floats np.isclose(rtol=CHECK_RTOL, atol=CHECK_ATOL).  Raises
+    IOError for a corrupt chunk or AssertionError for a mismatching one, whichever comes first in chunk order."""
+    dtype = _require_integer_dtype(reader.dtype)
+    codec = _codec_for(reader.config)
+    nc, b = reader.n_channels, reader.chunk_bounds
+    row_bytes = nc * dtype.itemsize
+    flags = _native._fl(reader._flags(), dtype)
+    ranges = list(_batch_ranges(b, row_bytes, first, last))
+
+    def stage(k):
+        # the Writer's staging buffers: pinned already when the check follows a write
+        lo, hi = ranges[k]
+        cbuf, offs = reader._stage_compressed(codec, [reader._span(i) for i in range(lo, hi)], 'w_comp%d' % (k & 1))
+        n = (b[hi] - b[lo]) * row_bytes
+        rbuf = codec.host_buffer('w_raw%d' % (k & 1), n)
+        _copy_rows(rbuf.array[:n].view(dtype).reshape(-1, nc), data[b[lo]:b[hi]])
+        return cbuf, offs, rbuf
+
+    with codec.stage_lock, ThreadPoolExecutor(1) as stager:
+        nxt = stager.submit(stage, 0) if ranges else None
+        try:
+            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Checking')):
+                cbuf, offs, rbuf = nxt.result()
+                nxt = stager.submit(stage, k + 1) if k + 1 < len(ranges) else None
+                status, mism, at = codec.verify_ptr(cbuf.ptr, 0, offs, reader._rows_of(range(lo, hi)), nc,
+                                                    dtype.itemsize, flags, rbuf.ptr, 0, CHECK_RTOL, CHECK_ATOL)
+                bad = np.flatnonzero((status != 0) | (mism != 0))
+                if not len(bad):
+                    continue
+                i = int(bad[0])
+                if status[i]:
+                    raise IOError("Compressed chunk #%d is corrupted." % (lo + i))
+                if nxt is not None:
+                    nxt.result()
+                    nxt = None
+                raise AssertionError(_mismatch_message(reader, data, lo + i, int(mism[i]), int(at[i])))
+        finally:
+            if nxt is not None:
+                nxt.exception()          # the stager is done with its buffers before they change hands
+
+
+def _mismatch_message(reader, data, idx, n_bad, at):
+    row, ch = divmod(at, reader.n_channels)
+    sample = reader.chunk_bounds[idx] + row
+    got = reader._decode([idx], [reader._span(idx)])[0][row, ch]
+    return ("chunk #%d does not match the data in %d element(s); the first is row %d (sample %d), channel %d: "
+            "decoded %r, expected %r" % (idx, n_bad, row, sample, ch, got.item(), data[sample, ch].item()))
+
+
 def check(data, out, outmeta):
-    """Decode every chunk and compare with `data` (reference mtscomp.py:866-888); AssertionError on mismatch."""
+    """Decode every chunk and compare it with `data` on the GPU (reference mtscomp.py:866-888): IOError for a corrupt
+    chunk, AssertionError for a mismatch, whichever chunk comes first."""
     unc = decompress(out, outmeta)
     try:
         dtype = _require_integer_dtype(unc.dtype)
-        codec = _codec_for(unc.config)
-        row_bytes = unc.n_channels * dtype.itemsize
         assert tuple(data.shape) == tuple(unc.shape) and data.dtype == dtype
-        with codec.stage_lock:
-            for lo, hi in tqdm(list(_batch_ranges(unc.chunk_bounds, row_bytes, 0, unc.n_chunks)), desc='Checking'):
-                ids = list(range(lo, hi))
-                buf = codec.host_buffer('r_out0', (unc.chunk_bounds[hi] - unc.chunk_bounds[lo]) * row_bytes)
-                rows = unc._decode_into(ids, [unc._span(i) for i in ids], buf.ptr, False)
-                got = buf.array[:int(rows[-1]) * row_bytes].view(dtype).reshape(-1, unc.n_channels)
-                expected = data[unc.chunk_bounds[lo]:unc.chunk_bounds[hi]]
-                assert got.shape == expected.shape
-                if np.issubdtype(dtype, np.integer):
-                    assert np.array_equal(got, expected)
-                else:
-                    assert np.allclose(got, expected, atol=CHECK_ATOL)
+        _verify_range(unc, data, 0, unc.n_chunks)
     finally:
         unc.close()
 

@@ -15,6 +15,7 @@
 #include "inflate_par.cuh"
 #include "inflate_seg.cuh"
 #include "transform.cuh"
+#include "verify.cuh"
 
 using namespace mts;
 
@@ -73,6 +74,7 @@ struct CopyPipe {
   cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr}, ev_done = nullptr;
   Buf* in[2] = {nullptr, nullptr};     // the buffer pairs of the call in progress
   Buf* out[2] = {nullptr, nullptr};
+  Buf* ref[2] = {nullptr, nullptr};
   CopyPipe() = default;
   CopyPipe(const CopyPipe&) = delete;
   bool create(cudaStream_t compute) {
@@ -89,23 +91,29 @@ struct CopyPipe {
     if (copy_in) cudaStreamDestroy(copy_in);
     if (copy_out) cudaStreamDestroy(copy_out);
   }
-  // takes the call's pairs (NEEDed by the caller) and queues the upload of sub-batch 0
-  int start(mtsb_ctx* c, Buf* in0, Buf* in1, Buf* out0, Buf* out1, const void* src0, size_t bytes0) {
-    in[0] = in0; in[1] = in1; out[0] = out0; out[1] = out1;
-    if (!in[0]) return 0;
+  // takes the call's pairs (NEEDed by the caller) and queues the upload of sub-batch 0.  ref0 / ref1: a second input
+  // pair (the reference rows of a verify call with a host reference), uploaded with the first and ready with it
+  int start(mtsb_ctx* c, Buf* in0, Buf* in1, Buf* out0, Buf* out1, const void* src0, size_t bytes0, Buf* ref0 = nullptr,
+            Buf* ref1 = nullptr, const void* ref_src0 = nullptr, size_t ref_bytes0 = 0) {
+    in[0] = in0; in[1] = in1; out[0] = out0; out[1] = out1; ref[0] = ref0; ref[1] = ref1;
+    if (!in[0] && !ref[0]) return 0;
     // the copy-in stream must not start before work already queued on the caller's stream (e.g. producing `src`)
     CK(cudaEventRecord(ev_done, stream));
     CK(cudaStreamWaitEvent(copy_in, ev_done, 0));
-    return upload(c, 0, src0, bytes0);
+    return upload(c, 0, src0, bytes0, ref_src0, ref_bytes0);
   }
-  int upload(mtsb_ctx* c, int k, const void* src, size_t bytes) {   // queues the upload of sub-batch k
-    if (!in[0]) return 0;
-    CK(cudaMemcpyAsync(in[k & 1]->p, src, bytes, cudaMemcpyHostToDevice, copy_in));
+  int upload(mtsb_ctx* c, int k, const void* src, size_t bytes, const void* ref_src = nullptr, size_t ref_bytes = 0) {
+    if (!in[0] && !ref[0]) return 0;                 // queues the upload of sub-batch k
+    if (in[0]) CK(cudaMemcpyAsync(in[k & 1]->p, src, bytes, cudaMemcpyHostToDevice, copy_in));
+    if (ref[0]) CK(cudaMemcpyAsync(ref[k & 1]->p, ref_src, ref_bytes, cudaMemcpyHostToDevice, copy_in));
     CK(cudaEventRecord(ev_in[k & 1], copy_in));
     return 0;
   }
-  int input(mtsb_ctx* c, int k, const void*& p) {   // p: sub-batch k's input, once its upload is done
-    if (in[0]) { CK(cudaStreamWaitEvent(stream, ev_in[k & 1], 0)); p = in[k & 1]->p; }
+  // p (and r, with a reference pair): sub-batch k's input, once its upload is done
+  int input(mtsb_ctx* c, int k, const void*& p, const void** r = nullptr) {
+    if (in[0] || ref[0]) CK(cudaStreamWaitEvent(stream, ev_in[k & 1], 0));
+    if (in[0]) p = in[k & 1]->p;
+    if (ref[0] && r) *r = ref[k & 1]->p;
     return 0;
   }
   int output(mtsb_ctx* c, int k, void*& p) {        // p: where sub-batch k's output goes, once it is free
@@ -160,6 +168,7 @@ struct mtsb_ctx {
   bool ignore_index = false;    // (internal) decode every chunk as a plain zlib stream: the retry of chunks whose index misled
   Buf d_raw, d_raw2, d_out2, d_comp2, d_T, d_tok, d_hist, d_codes, d_hdrs, d_tab, d_so, d_seg_adler, d_chunk_adler, d_chunk_off, d_out,
       d_partial, d_comp, d_status, d_tadler, d_gather, d_subabs, d_subtok, d_invstate, d_invcells;
+  Buf d_ref, d_ref2, d_vcount;     // verify: the reference rows of a host reference (a pair), the per-chunk counters
   int inv_cells_isz = 0;           // element size of the launch that last wrote the look-back cells
   long long inv_epoch = 0;         // epoch of the last inv_tile_kernel launch (tags its look-back cells)
   long long inv_order_block = 2;   // inv_tile_kernel: consecutive tiles of a chunk that get consecutive tickets
@@ -466,6 +475,37 @@ int launch_inv(mtsb_ctx* c, int isz, const void* tbuf, void* out, const ChunkDes
     case 8: return launch_inv_t<uint64_t>(c, tbuf, out, d_cd, n_chunks, max_ns, nc, flags);
   }
   return fail(c, MTSB_E_ARG, "itemsize %d not supported (1, 2, 4, 8)", isz);
+}
+
+// The compare of a verify sub-batch: decoded rows `dec` against reference rows `ref` (both from the sub-batch's first
+// row), per-chunk counters into d_vcount = [count nb][first nb]
+template <class T>
+int launch_verify_t(mtsb_ctx* c, const void* dec, const void* ref, const ChunkDesc* d_cd, int nb, int max_ns, int nc,
+                    double rtol, double atol) {
+  const long long tiles = ((long long)max_ns * nc * (long long)sizeof(T) + VERIFY_TILE_BYTES - 1) / VERIFY_TILE_BYTES;
+  unsigned long long* cnt = (unsigned long long*)c->d_vcount.p;
+  long long* fst = (long long*)c->d_vcount.p + nb;
+  CK(cudaMemsetAsync(cnt, 0, (size_t)nb * 8, c->stream));
+  CK(cudaMemsetAsync(fst, 0x7f, (size_t)nb * 8, c->stream));
+  auto k = verify_kernel<T>;
+  MTS_LAUNCH(k, dim3((unsigned)tiles, nb), dim3(VERIFY_THREADS), 0, c->stream, (const T*)dec, (const T*)ref, d_cd, nc, (T)rtol,
+             (T)atol, cnt, fst);
+  c->launches++;
+  CKL();
+  return 0;
+}
+int launch_verify(mtsb_ctx* c, int isz, int flags, const void* dec, const void* ref, const ChunkDesc* d_cd, int nb, int max_ns,
+                  int nc, double rtol, double atol) {
+  if (flags & FLAG_FLOAT) {
+    if (isz == 4) return launch_verify_t<float>(c, dec, ref, d_cd, nb, max_ns, nc, rtol, atol);
+    return launch_verify_t<double>(c, dec, ref, d_cd, nb, max_ns, nc, rtol, atol);
+  }
+  switch (isz) {
+    case 1: return launch_verify_t<uint8_t>(c, dec, ref, d_cd, nb, max_ns, nc, 0, 0);
+    case 2: return launch_verify_t<uint16_t>(c, dec, ref, d_cd, nb, max_ns, nc, 0, 0);
+    case 4: return launch_verify_t<uint32_t>(c, dec, ref, d_cd, nb, max_ns, nc, 0, 0);
+  }
+  return launch_verify_t<uint64_t>(c, dec, ref, d_cd, nb, max_ns, nc, 0, 0);
 }
 
 long long seg_size_for(const mtsb_ctx* c, long long ns, int itemsize, int flags) {
@@ -969,11 +1009,15 @@ static int fetch_ranges(mtsb_ctx* c, const unsigned char* comp, int comp_is_devi
 
 static uint32_t rd32(const unsigned char* p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
 
-// The arguments of one mtsb_decompress_chunks call
+// The arguments of one mtsb_decompress_chunks or mtsb_verify_chunks call (verify: the decoded rows go to scratch and are
+// compared with `ref`; dst is unused)
 struct DecodeArgs {
   const unsigned char* comp; int comp_is_device; const long long* comp_offsets;
   int n_chunks; const long long* chunk_rows; int nc, itemsize, flags;
   void* dst; int dst_is_device; long long row_bytes;
+  bool verify = false;
+  const void* ref = nullptr; int ref_is_device = 0; double rtol = 0, atol = 0;
+  long long* mismatches = nullptr; long long* first_mismatch = nullptr;
 };
 
 // What read_indexes found behind a chunk's zlib stream (the index formats are written by trailer_kernel, deflate.cuh).
@@ -1057,7 +1101,7 @@ static int read_indexes(mtsb_ctx* c, const DecodeArgs& a, std::vector<ChunkIndex
 // output).  Device-resident calls have nothing to overlap with: they take the largest sub-batches (measured on 600
 // chunks: 2 GiB 62 GB/s, 4 GiB 75, 8 GiB 88, one 13.9 GB batch 96 — fewer, fuller waves of the block kernels).
 static Batches plan_decode_batches(const mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix) {
-  const bool host_io = !a.comp_is_device || !a.dst_is_device;
+  const bool host_io = !a.comp_is_device || !(a.verify ? a.ref_is_device : a.dst_is_device);
   const long long min_streams = 8ll * c->sm_count, hard_limit = std::max<long long>(c->batch_bytes, 16ll << 30);
   const long long sb_limit = host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : hard_limit;
   // index-less chunks with host buffers: equal sub-batches of about par_batch_bytes
@@ -1488,7 +1532,16 @@ static bool chunk_verdicts(const DecodeBatch& b, const std::vector<ChunkIndex>& 
   return bad;
 }
 
-// Sub-batch k: segments, parallel phases, serial inflate, adler32s, inverse transform, verdicts
+// The rows of sub-batch k in the caller's `ref` (verify)
+static const void* ref_rows(const DecodeArgs& a, const Batches& sb, int k) {
+  return (const char*)a.ref + a.chunk_rows[sb.first[k]] * a.row_bytes;
+}
+static size_t batch_bytes_of(const DecodeArgs& a, const Batches& sb, int k) {
+  return (size_t)((a.chunk_rows[sb.first[k + 1]] - a.chunk_rows[sb.first[k]]) * a.row_bytes);
+}
+
+// Sub-batch k: segments, parallel phases, serial inflate, adler32s, inverse transform, verdicts.  Verify: the inverse
+// writes to scratch (d_out), the compare follows on the same stream and its counters come back with the verdicts.
 static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const Batches& sb, int k,
                         int* status, bool& any_bad) {
   CopyPipe& io = c->io;
@@ -1501,10 +1554,15 @@ static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<Chun
   c->begin(0);
   if (k + 1 < sb.count()) {
     const long long n0 = a.comp_offsets[sb.first[k + 1]], n1 = a.comp_offsets[sb.first[k + 2]];
-    if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0))) return r;
+    if (a.verify) {
+      if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0), ref_rows(a, sb, k + 1), batch_bytes_of(a, sb, k + 1))) return r;
+    } else if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0))) {
+      return r;
+    }
   }
   const void* in = a.comp + a.comp_offsets[c0];
-  if (int r = io.input(c, k, in)) return r;
+  const void* ref = a.verify ? ref_rows(a, sb, k) : nullptr;
+  if (int r = io.input(c, k, in, &ref)) return r;
   const unsigned char* dcomp = (const unsigned char*)in;
   c->end();
   c->begin(2);
@@ -1532,18 +1590,38 @@ static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<Chun
   CKL();
   c->launches += 2;
   c->end();
-  void* outp = (char*)a.dst + row0 * a.row_bytes;
-  if (int r = io.output(c, k, outp)) return r;
+  void* outp = a.verify ? c->d_out.p : (char*)a.dst + row0 * a.row_bytes;
+  if (!a.verify) {
+    if (int r = io.output(c, k, outp)) return r;
+  }
   c->begin(4);
   if (int r = launch_inv(c, a.itemsize, c->d_T.p, outp, TableBlob::dev<ChunkDesc>(c, o_cd), nb, b.max_ns, a.nc, a.flags, (size_t)(bbytes / a.itemsize))) return r;
   c->end();
+  if (a.verify) {
+    NEED(c->d_vcount, (size_t)nb * 16);
+    NEED(c->h_small, (size_t)n_segs * 8 + (size_t)nb * 20 + 160);
+    c->begin(6);
+    if (int r = launch_verify(c, a.itemsize, a.flags, outp, ref, TableBlob::dev<ChunkDesc>(c, o_cd), nb, b.max_ns, a.nc, a.rtol, a.atol)) return r;
+    c->end();
+  }
   ReadBack rb(c);
   rb.add(c->d_status.p, (size_t)n_segs * 4);
   rb.add(c->d_tadler.p, (size_t)n_segs * 4);
   rb.add(c->d_chunk_adler.p, (size_t)nb * 4);
+  if (a.verify) rb.add(c->d_vcount.p, (size_t)nb * 16);
   if (int r = rb.sync()) return r;
-  if (int r = io.download(c, k, (char*)a.dst + row0 * a.row_bytes, (size_t)bbytes)) return r;
+  if (!a.verify) {
+    if (int r = io.download(c, k, (char*)a.dst + row0 * a.row_bytes, (size_t)bbytes)) return r;
+  }
   if (chunk_verdicts(b, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), status)) any_bad = true;
+  if (a.verify) {
+    const long long* cnt = rb.get<long long>(3);
+    for (int i = 0; i < nb; i++) {
+      const bool ok = status[c0 + i] == 0;
+      a.mismatches[c0 + i] = ok ? cnt[i] : -1;
+      a.first_mismatch[c0 + i] = !ok || cnt[nb + i] == VERIFY_NONE ? -1 : cnt[nb + i];
+    }
+  }
   return 0;
 }
 
@@ -1558,8 +1636,12 @@ static int redecode_misled(mtsb_ctx* c, const DecodeArgs& a, const std::vector<C
     const long long one_off[2] = {0, a.comp_offsets[i + 1] - a.comp_offsets[i]}, one_rows[2] = {0, a.chunk_rows[i + 1] - a.chunk_rows[i]};
     int st = 0;
     c->ignore_index = true;
-    const int rc = mtsb_decompress_chunks(c, a.comp + a.comp_offsets[i], a.comp_is_device, one_off, 1, one_rows, a.nc, a.itemsize,
-                                          a.flags, (char*)a.dst + a.chunk_rows[i] * a.row_bytes, a.dst_is_device, &st);
+    const int rc = a.verify
+        ? mtsb_verify_chunks(c, a.comp + a.comp_offsets[i], a.comp_is_device, one_off, 1, one_rows, a.nc, a.itemsize, a.flags,
+                             (const char*)a.ref + a.chunk_rows[i] * a.row_bytes, a.ref_is_device, a.rtol, a.atol,
+                             a.mismatches + i, a.first_mismatch + i, &st)
+        : mtsb_decompress_chunks(c, a.comp + a.comp_offsets[i], a.comp_is_device, one_off, 1, one_rows, a.nc, a.itemsize,
+                                 a.flags, (char*)a.dst + a.chunk_rows[i] * a.row_bytes, a.dst_is_device, &st);
     c->ignore_index = false;
     if (rc != 0 && rc != MTSB_E_CORRUPT) return rc;
     status[i] = st;
@@ -1568,20 +1650,15 @@ static int redecode_misled(mtsb_ctx* c, const DecodeArgs& a, const std::vector<C
   return 0;
 }
 
-int mtsb_decompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, const long long* comp_offsets,
-                           int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags, void* dst,
-                           int dst_is_device, int* chunk_status) {
-  if (!valid_common(c, n_chunks, chunk_rows, nc, itemsize) || !comp_ || !comp_offsets || !dst)
-    return fail(c, MTSB_E_ARG, "decompress_chunks: bad arguments");
-  for (int i = 0; i < n_chunks; i++) {
-    long long l = comp_offsets[i + 1] - comp_offsets[i];
-    if (l < 1 || l > 0x7fffffffll) return fail(c, MTSB_E_ARG, "decompress_chunks: bad compressed length of chunk %d", i);
+// The body both batch decode entry points share: plan, sub-batches through the copy pipeline, retry of misled chunks
+static int decode_call(mtsb_ctx* c, const char* name, const DecodeArgs& a, int* chunk_status) {
+  for (int i = 0; i < a.n_chunks; i++) {
+    long long l = a.comp_offsets[i + 1] - a.comp_offsets[i];
+    if (l < 1 || l > 0x7fffffffll) return fail(c, MTSB_E_ARG, "%s: bad compressed length of chunk %d", name, i);
   }
   cudaSetDevice(c->device);
   c->reset_timing();
   c->par_survivors = c->par_candidates = c->par_chained = c->par_resumed = 0;
-  const DecodeArgs a{(const unsigned char*)comp_, comp_is_device, comp_offsets, n_chunks, chunk_rows, nc, itemsize, flags, dst,
-                     dst_is_device, (long long)nc * itemsize};
 
   // ---- plan: look for the segment index after each chunk's zlib stream
   c->begin(1);
@@ -1591,16 +1668,23 @@ int mtsb_decompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, c
   c->end();
 
   // every chunk's status, also when the caller does not ask for them
-  std::vector<int> own_status(chunk_status ? 0 : n_chunks);
+  std::vector<int> own_status(chunk_status ? 0 : a.n_chunks);
   int* status = chunk_status ? chunk_status : own_status.data();
-  for (int i = 0; i < n_chunks; i++) status[i] = 0;
+  for (int i = 0; i < a.n_chunks; i++) status[i] = 0;
   const Batches sb = plan_decode_batches(c, a, ix);
   const int n_sb = sb.count();
-  if (!comp_is_device) { NEED(c->d_comp, (size_t)sb.max_in + 256); if (n_sb > 1) NEED(c->d_comp2, (size_t)sb.max_in + 256); }
-  if (!dst_is_device) { NEED(c->d_out, (size_t)sb.max_out + 256); if (n_sb > 1) NEED(c->d_out2, (size_t)sb.max_out + 256); }
-  if (int r = c->io.start(c, comp_is_device ? nullptr : &c->d_comp, &c->d_comp2, dst_is_device ? nullptr : &c->d_out, &c->d_out2,
-                          a.comp + comp_offsets[0], (size_t)(comp_offsets[sb.first[1]] - comp_offsets[0])))
-    return r;
+  if (!a.comp_is_device) { NEED(c->d_comp, (size_t)sb.max_in + 256); if (n_sb > 1) NEED(c->d_comp2, (size_t)sb.max_in + 256); }
+  const bool host_rows = a.verify ? !a.ref_is_device : !a.dst_is_device;
+  if (host_rows || a.verify) NEED(c->d_out, (size_t)sb.max_out + 256);   // verify: the decoded rows, one buffer
+  if (host_rows && !a.verify && n_sb > 1) NEED(c->d_out2, (size_t)sb.max_out + 256);
+  if (host_rows && a.verify) { NEED(c->d_ref, (size_t)sb.max_out + 256); if (n_sb > 1) NEED(c->d_ref2, (size_t)sb.max_out + 256); }
+  const void* comp0 = a.comp + a.comp_offsets[0];
+  const size_t comp_bytes0 = (size_t)(a.comp_offsets[sb.first[1]] - a.comp_offsets[0]);
+  Buf* in0 = a.comp_is_device ? nullptr : &c->d_comp;
+  int r0 = a.verify ? c->io.start(c, in0, &c->d_comp2, nullptr, nullptr, comp0, comp_bytes0, host_rows ? &c->d_ref : nullptr,
+                                  &c->d_ref2, ref_rows(a, sb, 0), batch_bytes_of(a, sb, 0))
+                    : c->io.start(c, in0, &c->d_comp2, host_rows ? &c->d_out : nullptr, &c->d_out2, comp0, comp_bytes0);
+  if (r0) return r0;
   bool any_bad = false;
   for (int k = 0; k < n_sb; k++)
     if (int r = decode_batch(c, a, ix, sb, k, status, any_bad)) return r;
@@ -1611,6 +1695,30 @@ int mtsb_decompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, c
   }
   if (any_bad) return fail(c, MTSB_E_CORRUPT, "at least one compressed chunk is corrupted");
   return 0;
+}
+
+int mtsb_decompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, const long long* comp_offsets,
+                           int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags, void* dst,
+                           int dst_is_device, int* chunk_status) {
+  if (!valid_common(c, n_chunks, chunk_rows, nc, itemsize) || !comp_ || !comp_offsets || !dst)
+    return fail(c, MTSB_E_ARG, "decompress_chunks: bad arguments");
+  const DecodeArgs a{(const unsigned char*)comp_, comp_is_device, comp_offsets, n_chunks, chunk_rows, nc, itemsize, flags, dst,
+                     dst_is_device, (long long)nc * itemsize};
+  return decode_call(c, "decompress_chunks", a, chunk_status);
+}
+
+int mtsb_verify_chunks(mtsb_ctx* c, const void* comp, int comp_is_device, const long long* comp_offsets, int n_chunks,
+                       const long long* chunk_rows, int nc, int itemsize, int flags, const void* ref, int ref_is_device,
+                       double rtol, double atol, long long* mismatches, long long* first_mismatch, int* chunk_status) {
+  if (!valid_common(c, n_chunks, chunk_rows, nc, itemsize) || !comp || !comp_offsets || !ref || !mismatches ||
+      !first_mismatch || !chunk_status || ((size_t)ref % (size_t)itemsize) || ((flags & FLAG_FLOAT) && itemsize != 4 && itemsize != 8))
+    return fail(c, MTSB_E_ARG, "verify_chunks: bad arguments");
+  DecodeArgs a{(const unsigned char*)comp, comp_is_device, comp_offsets, n_chunks, chunk_rows, nc, itemsize, flags, nullptr,
+               0, (long long)nc * itemsize};
+  a.verify = true;
+  a.ref = ref; a.ref_is_device = ref_is_device; a.rtol = rtol; a.atol = atol;
+  a.mismatches = mismatches; a.first_mismatch = first_mismatch;
+  return decode_call(c, "verify_chunks", a, chunk_status);
 }
 
 }  // extern "C"

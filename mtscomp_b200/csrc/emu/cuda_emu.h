@@ -13,6 +13,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -267,6 +268,14 @@ static inline unsigned __byte_perm(unsigned x, unsigned y, unsigned s) {
 }
 static inline unsigned __umulhi(unsigned a, unsigned b) { return (unsigned)(((uint64_t)a * b) >> 32); }
 template <class T> static inline T __ldg(const T* p) { return *p; }
+
+// ---------------------------------------------------------------- IEEE operations rounded one at a time (no contraction)
+static inline float __fadd_rn(float a, float b) { return a + b; }
+static inline float __fsub_rn(float a, float b) { return a - b; }
+static inline float __fmul_rn(float a, float b) { return a * b; }
+static inline double __dadd_rn(double a, double b) { return a + b; }
+static inline double __dsub_rn(double a, double b) { return a - b; }
+static inline double __dmul_rn(double a, double b) { return a * b; }
 using std::max;
 using std::min;
 static inline unsigned min(unsigned a, int b) { return a < (unsigned)b ? a : (unsigned)b; }

@@ -58,6 +58,16 @@ def compress_sharded(codec, data, chunk_bounds, flags, rank, world, group=None):
     return comp, assemble_offsets(all_sizes), rank_base_offsets(all_sizes)[rank] if world > 1 else 0
 
 
+def gather_objects(obj, group=None):
+    """Every rank's `obj`, in rank order, on all ranks (one object all-gather; [obj] without a process group)."""
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized()):
+        return [obj]
+    out = [None] * dist.get_world_size(group)
+    dist.all_gather_object(out, obj, group=group)
+    return out
+
+
 def _barrier(group=None):
     import torch.distributed as dist
     if dist.is_available() and dist.is_initialized():
@@ -65,7 +75,7 @@ def _barrier(group=None):
 
 
 def write_sharded(data_path, out, outmeta, rank, world, sample_rate=None, n_channels=None, dtype=None, group=None,
-                  hash_raw=True, codec=None, **config):
+                  hash_raw=True, codec=None, check_after_compress=False, before_check=None, **config):
     """ONE `.cbin` + `.ch` written by `world` ranks (one GPU each): every rank memory-maps the raw file, compresses its
     contiguous chunk range (shard_range) on its GPU, the per-chunk sizes are gathered on the host, and each rank writes
     its packed streams at its base offset with pwrite (reference mtscomp.py:453-486 builds the same offset table
@@ -73,11 +83,16 @@ def write_sharded(data_path, out, outmeta, rank, world, sample_rate=None, n_chan
     and the compressed file — and writes the `.ch`.  Returns (chunk_offsets, seconds spent compressing on this rank).
 
     `codec` is for tests (anything with compress_ptr-free `compress(data, rows, flags)`); by default the rank's
-    `_native.Codec` is used through the Writer's own batching."""
+    `_native.Codec` is used through the Writer's own batching.
+
+    check_after_compress (off by default here): once the file is complete, each rank calls `before_check(writer)` and
+    verifies its own chunk range of the written .cbin against its memory map on its GPU.  The verdicts are gathered, so
+    that every rank raises the same error when any rank's check failed: the CRITICAL ERROR RuntimeError of
+    Writer.write for a mismatch, IOError for a corrupt chunk (the first failure in chunk order decides)."""
     import time
     from . import _native
     from .core import Writer, _batch_ranges, _require_integer_dtype
-    w = Writer(quiet=True, check_after_compress=False, **config)
+    w = Writer(quiet=True, check_after_compress=check_after_compress, before_check=before_check, **config)
     w.open(data_path, sample_rate=sample_rate, n_channels=n_channels, dtype=dtype)
     dt = _require_integer_dtype(w.dtype)
     b, nc, isz = w.chunk_bounds, w.n_channels, dt.itemsize
@@ -147,6 +162,38 @@ def write_sharded(data_path, out, outmeta, rank, world, sample_rate=None, n_chan
         with open(outmeta, 'w') as f:
             json.dump(meta, f, indent=2, sort_keys=True)
     pool.shutdown()
-    w.close()
     _barrier(group)
+    if check_after_compress:
+        _check_shard(w, out, outmeta, first, last, group)
+    w.close()
     return offsets, secs
+
+
+def _check_shard(w, out, outmeta, first, last, group=None):
+    """The post-write check of write_sharded on chunks [first, last): every rank takes part in the gather whatever its
+    own check did, so no rank waits in a collective for a rank that raised."""
+    from .core import CRITICAL_CHECK_FAILED, Reader, _verify_range
+    verdict = None
+    try:
+        w.before_check(w)
+        r = Reader(quiet=True, device=w.config.get('device', None))
+        r.open(out, outmeta)
+        try:
+            _verify_range(r, w.data, first, last)
+        finally:
+            r.close()
+    except AssertionError as e:
+        verdict = ('mismatch', str(e))
+    except IOError as e:
+        verdict = ('corrupt', str(e))
+    except Exception as e:
+        verdict = ('error', '%s: %s' % (type(e).__name__, e))
+    failed = [v for v in gather_objects(verdict, group) if v is not None]
+    if not failed:
+        return
+    kind, msg = failed[0]
+    if kind == 'mismatch':
+        raise RuntimeError(CRITICAL_CHECK_FAILED + " (" + msg + ")")
+    if kind == 'corrupt':
+        raise IOError(msg)
+    raise RuntimeError("the check after a sharded write failed on a rank: " + msg)
