@@ -123,12 +123,35 @@ int mtsb_verify_chunks(mtsb_ctx* ctx, const void* comp, int comp_is_device, cons
                        const void* ref, int ref_is_device, double rtol, double atol,
                        long long* mismatches, long long* first_mismatch, int* chunk_status);
 
-/* Device-time (ms, CUDA events on the context's stream) of the stages of the last compress / decompress / verify call:
+/* Re-encode: chunk i is the zlib stream comp[comp_offsets[i] : comp_offsets[i+1]], as mtsb_decompress_chunks takes it.
+ * It is inflated on the device to its transformed bytes, and those bytes are deflated again exactly as
+ * mtsb_compress_chunks deflates a chunk with the context's current parameters (write_index, seg_bytes, ...).  There is no
+ * inverse or forward transform.  The new stream inflates to the same bytes, so it has the same adler32 and decodes to
+ * exactly what chunk i decodes to.  Output: packed at dst, out_offsets as in mtsb_compress_chunks; dst_capacity must be
+ * >= the sum of mtsb_compress_bound.  flags: the file's, as for mtsb_decompress_chunks (the ORDER_C bit sets the
+ * encoder's segments).  chunk_status as in mtsb_decompress_chunks, never NULL.  A chunk that does not decode makes the
+ * call return MTSB_E_CORRUPT, and dst / out_offsets are then undefined.  If the bytes the encoder read do not have
+ * the adler32 the decode accepted for a chunk, the call returns MTSB_E_CUDA with an "internal:" message naming it.
+ * Sub-batches hold at most "batch_bytes" raw bytes ("host_batch_bytes" when comp or dst is host memory).  Peak device
+ * scratch: about 3 bytes per raw byte of the largest sub-batch (the transformed bytes and the match finder's tokens),
+ * plus the decoder's scratch, which is about 9.6 bytes per compressed byte of plain zlib streams (2 bytes per raw byte
+ * more for a sub-batch of 16 streams or fewer) and about 2.3 bytes per raw byte of indexed ones; with host buffers, two
+ * compressed inputs and two output bounds on top.  For AP-like int16 data (0.38 compressed bytes per raw byte) that is
+ * about 7 bytes per raw byte, 14 GiB at the default batch_bytes. */
+int mtsb_recompress_chunks(mtsb_ctx* ctx, const void* comp, int comp_is_device, const long long* comp_offsets,
+                           int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags,
+                           void* dst, int dst_is_device, long long dst_capacity, long long* out_offsets,
+                           int* chunk_status);
+
+/* Device-time (ms, CUDA events on the context's stream) of the stages of the last compress / decompress / verify /
+ * recompress call:
  * out[0..7] = {h2d, transform, adler, lz77, huffman+scan, encode, d2h, total} for compress,
  *             {h2d, plan, inflate, adler, inverse, d2h, 0, total} for decompress,
- *             {h2d, plan, inflate, adler, inverse, 0, compare, total} for verify.  Returns the number filled. */
+ *             {h2d, plan, inflate, adler, inverse, 0, compare, total} for verify,
+ *             {h2d, plan, inflate, adler, lz77, adler+huffman+scan+encode+trailer, 0, total} for recompress (its
+ *             downloads overlap the next sub-batch on a copy stream and are not timed).  Returns the number filled. */
 int mtsb_last_timings(mtsb_ctx* ctx, float* out, int n);
-/* Number of kernels launched by the last compress / decompress / verify / transform call. */
+/* Number of kernels launched by the last compress / decompress / verify / recompress / transform call. */
 long long mtsb_last_launches(mtsb_ctx* ctx);
 
 /* Pinned host memory helpers (so that Python can stage file data without torch). */

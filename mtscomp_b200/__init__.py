@@ -10,9 +10,9 @@ from .config import (  # noqa: F401
     Bunch, CHECK_ATOL, DEFAULT_CONFIG, FORMAT_VERSION, add_default_handler, config_path, read_config, write_config)
 from .rawio import load_raw_data  # noqa: F401
 from .core import (  # noqa: F401
-    Reader, Writer, check, compress, cumsum_along_axis, decompress, diff_along_axis)
+    Reader, Writer, check, compress, cumsum_along_axis, decompress, diff_along_axis, recompress)
 from .cli import (  # noqa: F401
-    _args_to_config, mtschop, mtscomp, mtscomp_parser, mtsdecomp, mtsdecomp_parser, mtsdesc)
+    _args_to_config, mtschop, mtscomp, mtscomp_parser, mtsdecomp, mtsdecomp_parser, mtsdesc, mtsrecomp)
 
 __version__ = '0.1.0'
 __all__ = ('load_raw_data', 'Writer', 'Reader', 'compress', 'decompress')

@@ -26,7 +26,8 @@ E_CORRUPT = -5
 SYMBOLS = (
     'mtsb_version', 'mtsb_device_count', 'mtsb_create', 'mtsb_destroy', 'mtsb_last_error', 'mtsb_sync',
     'mtsb_set_param', 'mtsb_get_param', 'mtsb_compress_bound', 'mtsb_delta_transform', 'mtsb_inverse_transform',
-    'mtsb_compress_chunks', 'mtsb_decompress_chunks', 'mtsb_verify_chunks', 'mtsb_last_timings', 'mtsb_last_launches',
+    'mtsb_compress_chunks', 'mtsb_decompress_chunks', 'mtsb_verify_chunks', 'mtsb_recompress_chunks',
+    'mtsb_last_timings', 'mtsb_last_launches',
     'mtsb_host_alloc', 'mtsb_host_free', 'mtsb_device_alloc', 'mtsb_device_free', 'mtsb_memcpy')
 
 
@@ -63,6 +64,7 @@ def _declare(lib):
     lib.mtsb_decompress_chunks.argtypes = [vp, vp, i, pll, i, pll, i, i, i, vp, i, C.POINTER(C.c_int)]
     lib.mtsb_verify_chunks.argtypes = [vp, vp, i, pll, i, pll, i, i, i, vp, i, C.c_double, C.c_double, pll, pll,
                                        C.POINTER(C.c_int)]
+    lib.mtsb_recompress_chunks.argtypes = [vp, vp, i, pll, i, pll, i, i, i, vp, i, ll, pll, C.POINTER(C.c_int)]
     lib.mtsb_last_timings.argtypes = [vp, C.POINTER(C.c_float), i]
     lib.mtsb_last_launches.argtypes = [vp]
     lib.mtsb_last_launches.restype = ll
@@ -256,6 +258,25 @@ class Codec:
                 self._check(rc)
         return status, mism, first
 
+    def recompress_ptr(self, comp, comp_is_device, comp_offsets, chunk_rows, nc, itemsize, flags, dst, dst_is_device,
+                       dst_capacity):
+        """Inflate each chunk to its transformed bytes and deflate them again with the codec's current parameters
+        (mtsb_recompress_chunks) -> (out_offsets int64[n+1], status int32[n]).  Where a status is non-zero the output
+        is undefined."""
+        rows, offs = _i64(chunk_rows), _i64(comp_offsets)
+        n = len(rows) - 1
+        out = np.zeros(n + 1, dtype=np.int64)
+        status = np.zeros(n, dtype=np.int32)
+        pll = C.POINTER(C.c_longlong)
+        with self.lock:
+            rc = self.lib.mtsb_recompress_chunks(
+                self.ctx, C.c_void_p(comp), int(comp_is_device), offs.ctypes.data_as(pll), n,
+                rows.ctypes.data_as(pll), nc, itemsize, flags, C.c_void_p(dst), int(dst_is_device), int(dst_capacity),
+                out.ctypes.data_as(pll), status.ctypes.data_as(C.POINTER(C.c_int)))
+            if rc != 0 and rc != E_CORRUPT:
+                self._check(rc)
+        return out, status
+
     # -- NumPy conveniences (host arrays)
     def delta_transform(self, chunk, flags):
         chunk = np.ascontiguousarray(chunk)
@@ -308,6 +329,19 @@ class Codec:
         comp = np.frombuffer(comp, dtype=np.uint8)
         return self.verify_ptr(comp.ctypes.data, 0, comp_offsets, chunk_rows, ref.shape[1], ref.dtype.itemsize,
                                _fl(flags, ref.dtype), ref.ctypes.data, 0, rtol, atol)
+
+    def recompress(self, comp, comp_offsets, chunk_rows, nc, dtype, flags):
+        """comp: bytes-like -> (bytes-like uint8 array, offsets int64[n+1], status int32[n])."""
+        dtype = np.dtype(dtype)
+        comp = np.frombuffer(comp, dtype=np.uint8)
+        rows = _i64(chunk_rows)
+        flags = _fl(flags, dtype)
+        cap = sum(self.compress_bound(int(rows[i + 1] - rows[i]), nc, dtype.itemsize, flags)
+                  for i in range(len(rows) - 1))
+        dst = np.empty(cap, dtype=np.uint8)
+        offs, status = self.recompress_ptr(comp.ctypes.data, 0, comp_offsets, rows, nc, dtype.itemsize, flags,
+                                           dst.ctypes.data, 0, cap)
+        return dst[:int(offs[-1])], offs, status
 
 
 _default = {}

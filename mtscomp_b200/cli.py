@@ -1,5 +1,5 @@
 # -*- coding: utf-8 -*-
-"""Command-line front-ends mtscomp / mtsdecomp / mtsdesc / mtschop (reference mtscomp.py:1004-1179)."""
+"""Command-line front-ends mtscomp / mtsdecomp / mtsdesc / mtschop (reference mtscomp.py:1004-1179) and mtsrecomp."""
 
 import argparse
 import sys
@@ -7,7 +7,7 @@ import sys
 import numpy as np
 
 from .config import add_default_handler, read_config, write_config
-from .core import Reader, compress, decompress
+from .core import Reader, compress, decompress, recompress
 
 
 def exception_handler(exception_type, exception, traceback, debug_hook=sys.excepthook):  # pragma: no cover
@@ -112,3 +112,25 @@ def mtschop(args=None):
     r.open(pargs.cdata)
     r.chop(pargs.n_chunks, pargs.out)
     r.close()
+
+
+def mtsrecomp(args=None):
+    """Re-encode a compressed file on the GPU, with or without the segment index, without decompressing it."""
+    sys.excepthook = exception_handler
+    parser = argparse.ArgumentParser(
+        description='Re-encode a compressed file on the GPU from its chunks\' inflated bytes: adds the segment index '
+                    'that speeds up decoding (or strips it with --no-index). The new file decodes to exactly what the '
+                    'input decodes to.')
+    parser.add_argument('cdata', type=str, help='path to the input compressed binary file (.cbin)')
+    parser.add_argument('cmeta', type=str, nargs='?', help='path to the input compression metadata JSON file (.ch)')
+    parser.add_argument('-o', '--out', type=str, required=True, help='path to the output compressed file (.cbin)')
+    parser.add_argument('--outmeta', type=str, help='path to the output metadata file (.ch, default: next to --out)')
+    parser.add_argument('--no-index', action='store_true', help='write one plain zlib stream per chunk, no index')
+    parser.add_argument('--overwrite', '-f', action='store_true', help='overwrite existing output')
+    _shared_options(parser)
+    pargs = parser.parse_args(args or sys.argv[1:])
+    add_default_handler('DEBUG' if pargs.debug else 'INFO')
+    # store_false: True means the flag was absent -> keep the configured default
+    check_after = None if pargs.no_check is True else False
+    return recompress(pargs.cdata, pargs.cmeta, out=pargs.out, outmeta=pargs.outmeta, write_index=not pargs.no_index,
+                      overwrite=pargs.overwrite, n_threads=pargs.cpus, check_after_compress=check_after)

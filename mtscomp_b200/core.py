@@ -866,6 +866,148 @@ def compress(path, out=None, outmeta=None, sample_rate=None, n_channels=None, dt
     return ratio
 
 
+def _recompress_batches(r, fb, ranges, flags, write_index, quiet):
+    """Recompress the open Reader `r` batch by batch into the file `fb` -> (chunk_offsets, SHA-1 of the written bytes).
+    While the GPU recompresses batch k, a worker stages batch k+1's .cbin bytes into pinned memory and another writes
+    and hashes batch k-1's output."""
+    codec = _codec_for(r.config)
+    nc, b, isz = r.n_channels, r.chunk_bounds, r.dtype.itemsize
+    sha1 = hashlib.sha1()
+    offsets = [0]
+
+    def stage(k):
+        lo, hi = ranges[k]
+        return r._stage_compressed(codec, [r._span(i) for i in range(lo, hi)], 'rc_in%d' % (k & 1))
+
+    def write_and_hash(comp):
+        fb.write(comp)
+        sha1.update(comp)
+
+    with codec.stage_lock, _codec_param(codec, 'write_index', write_index), \
+            ThreadPoolExecutor(1) as stager, ThreadPoolExecutor(1) as writer:
+        # (the bound depends on write_index: computed with it set)
+        caps = [sum(codec.compress_bound(b[i + 1] - b[i], nc, isz, flags) for i in range(lo, hi)) for lo, hi in ranges]
+        out_bufs = [codec.host_buffer('rc_out%d' % i, max(caps)) for i in (0, 1)]
+        nxt = stager.submit(stage, 0)
+        pending = [None, None]
+        try:
+            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Recompressing', disable=quiet)):
+                slot = k & 1
+                cbuf, coffs = nxt.result()
+                nxt = stager.submit(stage, k + 1) if k + 1 < len(ranges) else None
+                if pending[slot] is not None:         # the slot's previous batch has been written
+                    pending[slot].result()
+                offs, status = codec.recompress_ptr(cbuf.ptr, 0, coffs, r._rows_of(range(lo, hi)), nc, isz, flags,
+                                                    out_bufs[slot].ptr, 0, caps[k])
+                r._raise_if_corrupt(status, list(range(lo, hi)))
+                base = offsets[-1]
+                offsets.extend(int(base + o) for o in offs[1:])
+                pending[slot] = writer.submit(write_and_hash, out_bufs[slot].array[:int(offs[-1])])
+            for f in pending:
+                if f is not None:
+                    f.result()
+        finally:
+            if nxt is not None:
+                nxt.exception()          # the stager is done with its buffer before the exception propagates
+    return offsets, sha1
+
+
+def _check_recompressed(src, new, ranges, quiet):
+    """Both Readers' chunks decode to the same bits: each batch of `src` is decoded into device memory and `new`'s
+    chunks are verified against it (mtsb_verify_chunks, reference on the device).  Both calls use the integer flags
+    of the element width: the modular inverse transform is a bijection, so equal integer decodes mean equal inflated
+    bytes, which makes the check exact for floats too (NaN payloads included)."""
+    codec = _codec_for(src.config)
+    nc, b, isz = src.n_channels, src.chunk_bounds, src.dtype.itemsize
+    row_bytes = nc * isz
+    flags = src._flags()                          # no MTSB_FLOAT
+    block = _DeviceBlock(codec, max((b[hi] - b[lo]) * row_bytes for lo, hi in ranges) + 256)
+
+    def stage(k):
+        lo, hi = ranges[k]
+        ids = range(lo, hi)
+        return (src._stage_compressed(codec, [src._span(i) for i in ids], 'rc_in%d' % (k & 1)),
+                new._stage_compressed(codec, [new._span(i) for i in ids], 'rc_chk%d' % (k & 1)))
+
+    with codec.stage_lock, ThreadPoolExecutor(1) as stager:
+        nxt = stager.submit(stage, 0)
+        try:
+            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Checking', disable=quiet)):
+                (sbuf, soffs), (nbuf, noffs) = nxt.result()
+                nxt = stager.submit(stage, k + 1) if k + 1 < len(ranges) else None
+                ids = list(range(lo, hi))
+                rows = src._rows_of(ids)
+                src._raise_if_corrupt(codec.decompress_ptr(sbuf.ptr, 0, soffs, rows, nc, isz, flags, block.ptr, 1), ids)
+                status, mism, _ = codec.verify_ptr(nbuf.ptr, 0, noffs, rows, nc, isz, flags, block.ptr, 1, 0., 0.)
+                bad = np.flatnonzero((status != 0) | (mism != 0))
+                if len(bad):
+                    raise RuntimeError("recompressed chunk #%d does not decode to what the source chunk decodes to"
+                                       % ids[int(bad[0])])
+        finally:
+            if nxt is not None:
+                nxt.exception()
+
+
+def recompress(cdata, cmeta=None, out=None, outmeta=None, write_index=True, overwrite=False, quiet=False, **kwargs):
+    """Re-encode a compressed dataset on the GPU into `out` (.cbin) + `outmeta` (.ch, default: next to `out`), with
+    (write_index=True) or without the in-band segment index; returns compressed/raw size ratio.
+
+    Every chunk's zlib stream is inflated to its transformed bytes and deflated again; the samples are never
+    reconstructed, so the new file decodes to exactly what the source decodes to, for floats too.  The .ch keeps every
+    key of the source's but `chunk_offsets` and `sha1_compressed`.  Unless check_after_compress is off, every new chunk
+    is then checked against its source chunk on the GPU.  On failure the new .cbin is removed and no .ch is written."""
+    if out is None:
+        raise ValueError("The output path must be specified.")
+    out = Path(out)
+    outmeta = Path(outmeta) if outmeta else out.with_suffix('.ch')
+    r = Reader(quiet=quiet, **kwargs)
+    r.open(cdata, cmeta)
+    try:
+        src_cbin = Path(r.cdata.name)
+        src_ch = Path(cmeta) if isinstance(cmeta, (str, Path)) else src_cbin.with_suffix('.ch')
+        for p, s in ((out, src_cbin), (outmeta, src_ch)):
+            if p.resolve() == s.resolve() or (p.exists() and s.exists() and op.samefile(p, s)):
+                raise ValueError("Cannot recompress %s in place: %s is a source file." % (src_cbin, p))
+        for p in (out, outmeta):
+            if p.exists() and not overwrite:
+                raise ValueError(
+                    "The output file %s already exists, use --overwrite or specify another output path." % p)
+        dtype = _require_integer_dtype(r.dtype)
+        flags = _native._fl(r._flags(), dtype)
+        ranges = list(_batch_ranges(r.chunk_bounds, r.n_channels * dtype.itemsize, 0, r.n_chunks))
+        for p in (out, outmeta):
+            if p.exists():
+                p.unlink()
+        out.parent.mkdir(exist_ok=True, parents=True)
+        try:
+            with open(out, 'wb') as fb:
+                offsets, sha1 = _recompress_batches(r, fb, ranges, flags, write_index, quiet)
+                csize = fb.tell()
+            assert offsets[-1] == csize
+            meta = dict(r.cmeta)
+            meta['chunk_offsets'] = offsets
+            meta['sha1_compressed'] = sha1.hexdigest()
+            if r.config.check_after_compress:
+                new = Reader(quiet=quiet, **kwargs)
+                new.open(out, meta)
+                try:
+                    _check_recompressed(r, new, ranges, quiet)
+                finally:
+                    new.close()
+                logger.debug("Automatic integrity check after recompression PASSED.")
+        except BaseException:
+            if out.exists():
+                out.unlink()
+            raise
+        with open(outmeta, 'w') as f:
+            json.dump(meta, f, indent=2, sort_keys=True)
+        ratio = csize / (r.n_samples * r.n_channels * dtype.itemsize)
+        logger.info("Wrote %s (%.1f GB, -%.3f%%).", out, csize / 1024 ** 3, 100 - 100 * ratio)
+        return ratio
+    finally:
+        r.close()
+
+
 def decompress(cdata, cmeta=None, out=None, write_output=False, overwrite=False, **kwargs):
     """Open a compressed dataset, optionally writing the decompressed file; returns the Reader
     (reference mtscomp.py:961-997)."""

@@ -763,9 +763,9 @@ int mtsb_inverse_transform(mtsb_ctx* c, const void* src, int src_is_device, long
 // Compress sub-batches: bounded by batch_bytes; smaller when a host buffer is involved so that copies pipeline with
 // kernels.  Device-resident calls have nothing to overlap with: one large sub-batch keeps the persistent match-finder
 // CTAs busy to the end (measured on 600 chunks: 2 GiB 99.9, 4 GiB 100.6, one 13.9 GB batch 101.7 GB/s).
+// sb_limit: raw bytes per sub-batch (a single larger chunk forms its own)
 static Batches plan_encode_batches(const mtsb_ctx* c, int n_chunks, const long long* chunk_rows, long long row_bytes,
-                                   int itemsize, int flags, bool host_io) {
-  const long long sb_limit = host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : std::max<long long>(c->batch_bytes, 16ll << 30);
+                                   int itemsize, int flags, long long sb_limit) {
   Batches sb;
   for (int a = 0; a < n_chunks;) {
     sb.first.push_back(a);
@@ -840,7 +840,9 @@ static void plan_encode_tables(const mtsb_ctx* c, const long long* chunk_rows, i
 }
 
 // The kernels that encode one sub-batch (its tables uploaded): forward transform of `raw` into d_T, match finder,
-// per-chunk adler32, Huffman tables, output offsets (d_chunk_off), encoder and, with write_index, the index trailers
+// per-chunk adler32, Huffman tables, output offsets (d_chunk_off), encoder and, with write_index, the index trailers.
+// raw == nullptr: d_T already holds the transformed bytes (recompress), there is no transform, and the stages are timed
+// in recompress's slots (lz77 4, the rest 5).
 static int launch_encode(mtsb_ctx* c, const EncodeBatch& b, const void* raw, int nc, int itemsize, int flags,
                          unsigned char* outp) {
   const int nb = b.nb, n_segs = (int)b.segs.size();
@@ -848,10 +850,12 @@ static int launch_encode(mtsb_ctx* c, const EncodeBatch& b, const void* raw, int
   const DeflateSeg* d_seg = TableBlob::dev<DeflateSeg>(c, b.o_seg);
   const AdlerSeg* d_as = TableBlob::dev<AdlerSeg>(c, b.o_as);
   const int* d_first = TableBlob::dev<int>(c, b.o_first);
-  c->begin(1);
-  if (int r = launch_fwd(c, itemsize, raw, c->d_T.p, d_cd, nb, b.max_ns, nc, flags)) return r;
-  c->end();
-  c->begin(3);
+  if (raw) {
+    c->begin(1);
+    if (int r = launch_fwd(c, itemsize, raw, c->d_T.p, d_cd, nb, b.max_ns, nc, flags)) return r;
+    c->end();
+  }
+  c->begin(raw ? 3 : 4);
   {
     NEED(c->d_invstate, 256);
     CK(cudaMemsetAsync(c->d_invstate.p, 0, 64, c->stream));    // the match finder's segment counter
@@ -863,7 +867,7 @@ static int launch_encode(mtsb_ctx* c, const EncodeBatch& b, const void* raw, int
     c->launches++;
   }
   c->end();
-  c->begin(4);
+  c->begin(raw ? 4 : 5);
   // the match finder left each segment's adler32 (it streams every byte of T anyway): fold them per chunk
   MTS_LAUNCH(adler_combine_kernel, dim3((nb + 127) / 128), dim3(128), 0, c->stream, d_as, (const uint32_t*)c->d_seg_adler.p, d_first, nb, (uint32_t*)c->d_chunk_adler.p);
   CKL();
@@ -908,7 +912,9 @@ int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_
 
   out_offsets[0] = 0;
   long long total_out = 0;
-  const Batches sb = plan_encode_batches(c, n_chunks, chunk_rows, row_bytes, itemsize, flags, !src_is_device || !dst_is_device);
+  const bool host_io = !src_is_device || !dst_is_device;
+  const Batches sb = plan_encode_batches(c, n_chunks, chunk_rows, row_bytes, itemsize, flags,
+                                         host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : std::max<long long>(c->batch_bytes, 16ll << 30));
   const int n_sb = sb.count();
   if (!src_is_device) { NEED(c->d_raw, (size_t)sb.max_in + 256); if (n_sb > 1) NEED(c->d_raw2, (size_t)sb.max_in + 256); }
   if (!dst_is_device) { NEED(c->d_out, (size_t)sb.max_out + 256); if (n_sb > 1) NEED(c->d_out2, (size_t)sb.max_out + 256); }
@@ -1155,11 +1161,14 @@ struct DecodeBatch {
   std::vector<char> have_adler;
   std::vector<AdlerSeg> as;      // the bytes the adler kernels sum for the other chunks: chunk i's [as_first[i], as_first[i + 1])
   std::vector<int> as_first;
+  size_t o_cd = 0;               // where inflate_stages put the ChunkDesc table in d_tab
 };
 
+// Chunks [c0, c1) placed in d_T and in the device copy of the compressed bytes relative to chunk `base` (<= c0): the
+// first chunk of the sub-batch whose buffers they are in
 static void plan_segments(const mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, int c0, int c1,
-                          DecodeBatch& b) {
-  const long long row0 = a.chunk_rows[c0], comp0 = a.comp_offsets[c0];
+                          DecodeBatch& b, int base) {
+  const long long row0 = a.chunk_rows[base], comp0 = a.comp_offsets[base];
   b.c0 = c0;
   b.nb = c1 - c0;
   b.cds.resize(b.nb);
@@ -1514,9 +1523,10 @@ static int serial_inflate(mtsb_ctx* c, const unsigned char* dcomp, const std::ve
 
 // Each chunk's status: its first failing segment's, else INF_BAD_ADLER where the adler32 of its transformed bytes is not
 // the stored one (the index's, or the zlib trailer's the serial kernel read: ta).  st: the segments' statuses, ca: the
-// adler kernels' sums.  Returns whether a chunk failed.
+// adler kernels' sums.  accepted (may be null): per chunk, the stored adler32 that a good chunk matched.  Returns
+// whether a chunk failed.
 static bool chunk_verdicts(const DecodeBatch& b, const std::vector<ChunkIndex>& ix, const int* st, const uint32_t* ta,
-                           const uint32_t* ca, int* status) {
+                           const uint32_t* ca, int* status, uint32_t* accepted = nullptr) {
   bool bad = false;
   for (int i = 0; i < b.nb; i++) {
     int s = 0;
@@ -1525,6 +1535,7 @@ static bool chunk_verdicts(const DecodeBatch& b, const std::vector<ChunkIndex>& 
       const ChunkIndex& x = ix[b.c0 + i];
       uint32_t want = x.n_seg ? x.adler : ta[b.first[i]];
       if (want != (b.have_adler[i] ? b.adler[i] : ca[i])) s = INF_BAD_ADLER;
+      if (accepted) accepted[i] = want;
     }
     if (s) bad = true;
     status[b.c0 + i] = s;
@@ -1540,36 +1551,18 @@ static size_t batch_bytes_of(const DecodeArgs& a, const Batches& sb, int k) {
   return (size_t)((a.chunk_rows[sb.first[k + 1]] - a.chunk_rows[sb.first[k]]) * a.row_bytes);
 }
 
-// Sub-batch k: segments, parallel phases, serial inflate, adler32s, inverse transform, verdicts.  Verify: the inverse
-// writes to scratch (d_out), the compare follows on the same stream and its counters come back with the verdicts.
-static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const Batches& sb, int k,
-                        int* status, bool& any_bad) {
-  CopyPipe& io = c->io;
-  const int c0 = sb.first[k], c1 = sb.first[k + 1];
-  const long long row0 = a.chunk_rows[c0], bbytes = (a.chunk_rows[c1] - row0) * a.row_bytes;
-  DecodeBatch b;
-  plan_segments(c, a, ix, c0, c1, b);
+// The decode stages that fill d_T for the planned segments of b (dcomp: the device copy of their compressed bytes):
+// parallel phases, serial inflate, adler32s.  The statuses, trailer adler32s and sums are left in d_status, d_tadler
+// and d_chunk_adler for chunk_verdicts.
+static int inflate_stages(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const unsigned char* dcomp,
+                          DecodeBatch& b) {
   const int nb = b.nb, n_segs = (int)b.segs.size();
-  NEED(c->d_T, (size_t)bbytes + 16384);
-  c->begin(0);
-  if (k + 1 < sb.count()) {
-    const long long n0 = a.comp_offsets[sb.first[k + 1]], n1 = a.comp_offsets[sb.first[k + 2]];
-    if (a.verify) {
-      if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0), ref_rows(a, sb, k + 1), batch_bytes_of(a, sb, k + 1))) return r;
-    } else if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0))) {
-      return r;
-    }
-  }
-  const void* in = a.comp + a.comp_offsets[c0];
-  const void* ref = a.verify ? ref_rows(a, sb, k) : nullptr;
-  if (int r = io.input(c, k, in, &ref)) return r;
-  const unsigned char* dcomp = (const unsigned char*)in;
-  c->end();
   c->begin(2);
   if (int r = par_phases(c, dcomp, b)) return r;
   fold_adlers(c, a, ix, b);
   TableBlob tab;
   const size_t o_cd = tab.add(b.cds), o_seg = tab.add(b.segs), o_as = tab.add(b.as), o_first = tab.add(b.as_first);
+  b.o_cd = o_cd;
   if (int r = tab.stage(c)) return r;
   const int n_as = (int)b.as.size();
   NEED(c->d_status, (size_t)n_segs * 4);
@@ -1590,6 +1583,47 @@ static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<Chun
   CKL();
   c->launches += 2;
   c->end();
+  return 0;
+}
+
+// Sub-batch k up to the filled d_T: its segments, the upload of sub-batch k+1 (and, verify, its reference rows), the
+// wait for its own input (dcomp; ref: its reference rows), inflate_stages
+static int inflate_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const Batches& sb, int k,
+                         DecodeBatch& b, const unsigned char*& dcomp, const void*& ref) {
+  CopyPipe& io = c->io;
+  const int c0 = sb.first[k], c1 = sb.first[k + 1];
+  const long long row0 = a.chunk_rows[c0], bbytes = (a.chunk_rows[c1] - row0) * a.row_bytes;
+  plan_segments(c, a, ix, c0, c1, b, c0);
+  NEED(c->d_T, (size_t)bbytes + 16384);
+  c->begin(0);
+  if (k + 1 < sb.count()) {
+    const long long n0 = a.comp_offsets[sb.first[k + 1]], n1 = a.comp_offsets[sb.first[k + 2]];
+    if (a.verify) {
+      if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0), ref_rows(a, sb, k + 1), batch_bytes_of(a, sb, k + 1))) return r;
+    } else if (int r = io.upload(c, k + 1, a.comp + n0, (size_t)(n1 - n0))) {
+      return r;
+    }
+  }
+  const void* in = a.comp + a.comp_offsets[c0];
+  ref = a.verify ? ref_rows(a, sb, k) : nullptr;
+  if (int r = io.input(c, k, in, &ref)) return r;
+  dcomp = (const unsigned char*)in;
+  c->end();
+  return inflate_stages(c, a, ix, dcomp, b);
+}
+
+// Sub-batch k: inflate_batch, inverse transform, verdicts.  Verify: the inverse writes to scratch (d_out), the compare
+// follows on the same stream and its counters come back with the verdicts.
+static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const Batches& sb, int k,
+                        int* status, bool& any_bad) {
+  CopyPipe& io = c->io;
+  DecodeBatch b;
+  const unsigned char* dcomp = nullptr;
+  const void* ref = nullptr;
+  if (int r = inflate_batch(c, a, ix, sb, k, b, dcomp, ref)) return r;
+  const int c0 = b.c0, nb = b.nb, n_segs = (int)b.segs.size();
+  const long long row0 = a.chunk_rows[c0], bbytes = (a.chunk_rows[sb.first[k + 1]] - row0) * a.row_bytes;
+  const size_t o_cd = b.o_cd;
   void* outp = a.verify ? c->d_out.p : (char*)a.dst + row0 * a.row_bytes;
   if (!a.verify) {
     if (int r = io.output(c, k, outp)) return r;
@@ -1719,6 +1753,134 @@ int mtsb_verify_chunks(mtsb_ctx* c, const void* comp, int comp_is_device, const 
   a.ref = ref; a.ref_is_device = ref_is_device; a.rtol = rtol; a.atol = atol;
   a.mismatches = mismatches; a.first_mismatch = first_mismatch;
   return decode_call(c, "verify_chunks", a, chunk_status);
+}
+
+// =============================================================================================== recompress
+// Inflate sub-batch k into d_T (the decode stages, no inverse transform), then deflate d_T again (the encode stages, no
+// forward transform).  The decode and the encode scratch are used one after the other on one stream, so a sub-batch is
+// bounded like a compress sub-batch: batch_bytes of raw bytes, host_batch_bytes with a host buffer.
+int mtsb_recompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, const long long* comp_offsets,
+                           int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags, void* dst,
+                           int dst_is_device, long long dst_capacity, long long* out_offsets, int* chunk_status) {
+  if (!valid_common(c, n_chunks, chunk_rows, nc, itemsize) || !comp_ || !comp_offsets || !dst || !out_offsets || !chunk_status)
+    return fail(c, MTSB_E_ARG, "recompress_chunks: bad arguments");
+  for (int i = 0; i < n_chunks; i++) {
+    long long l = comp_offsets[i + 1] - comp_offsets[i];
+    if (l < 1 || l > 0x7fffffffll) return fail(c, MTSB_E_ARG, "recompress_chunks: bad compressed length of chunk %d", i);
+  }
+  cudaSetDevice(c->device);
+  c->reset_timing();
+  c->par_survivors = c->par_candidates = c->par_chained = c->par_resumed = 0;
+  const long long row_bytes = (long long)nc * itemsize;
+  long long need = 0;
+  for (int i = 0; i < n_chunks; i++) {
+    long long ns = chunk_rows[i + 1] - chunk_rows[i];
+    need += chunk_bound(c, ns * row_bytes, seg_size_for(c, ns, itemsize, flags));
+  }
+  if (dst_capacity < need) return fail(c, MTSB_E_CAPACITY, "dst_capacity %lld < bound %lld", dst_capacity, need);
+  const DecodeArgs a{(const unsigned char*)comp_, comp_is_device, comp_offsets, n_chunks, chunk_rows, nc, itemsize, flags,
+                     nullptr, 0, row_bytes};
+
+  c->begin(1);
+  std::vector<ChunkIndex> ix;
+  std::vector<unsigned char> ix_bytes;
+  if (int r = read_indexes(c, a, ix, ix_bytes)) return r;
+  c->end();
+  for (int i = 0; i < n_chunks; i++) chunk_status[i] = 0;
+
+  const bool host_io = !comp_is_device || !dst_is_device;
+  const Batches sb = plan_encode_batches(c, n_chunks, chunk_rows, row_bytes, itemsize, flags,
+                                         host_io ? std::min(c->batch_bytes, c->host_batch_bytes) : c->batch_bytes);
+  const int n_sb = sb.count();
+  long long max_comp = 0;
+  for (int k = 0; k < n_sb; k++) max_comp = std::max(max_comp, comp_offsets[sb.first[k + 1]] - comp_offsets[sb.first[k]]);
+  if (!comp_is_device) { NEED(c->d_comp, (size_t)max_comp + 256); if (n_sb > 1) NEED(c->d_comp2, (size_t)max_comp + 256); }
+  if (!dst_is_device) { NEED(c->d_out, (size_t)sb.max_out + 256); if (n_sb > 1) NEED(c->d_out2, (size_t)sb.max_out + 256); }
+  CopyPipe& io = c->io;
+  if (int r = io.start(c, comp_is_device ? nullptr : &c->d_comp, &c->d_comp2, dst_is_device ? nullptr : &c->d_out, &c->d_out2,
+                       a.comp + comp_offsets[0], (size_t)(comp_offsets[sb.first[1]] - comp_offsets[0])))
+    return r;
+  out_offsets[0] = 0;
+  long long total_out = 0;
+  bool any_bad = false;
+  for (int k = 0; k < n_sb; k++) {
+    const int c0 = sb.first[k], c1 = sb.first[k + 1];
+    // ---- decode half: inflate into d_T, verdicts
+    DecodeBatch b;
+    const unsigned char* dcomp = nullptr;
+    const void* unused_ref = nullptr;
+    if (int r = inflate_batch(c, a, ix, sb, k, b, dcomp, unused_ref)) return r;
+    std::vector<uint32_t> adler(b.nb, 0);     // the adler32 each good chunk's stored checksum confirmed
+    {
+      const int n_segs = (int)b.segs.size();
+      ReadBack rb(c);
+      rb.add(c->d_status.p, (size_t)n_segs * 4);
+      rb.add(c->d_tadler.p, (size_t)n_segs * 4);
+      rb.add(c->d_chunk_adler.p, (size_t)b.nb * 4);
+      if (int r = rb.sync()) return r;
+      chunk_verdicts(b, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), chunk_status, adler.data());
+    }
+    // a chunk whose index misled the decoder (see redecode_misled) is inflated again as a plain stream, alone, into its
+    // own place in d_T, before anything of the sub-batch is encoded
+    for (int i = c0; i < c1; i++) {
+      if (!chunk_status[i] || !ix[i].n_seg) continue;
+      ix[i] = ChunkIndex();
+      DecodeBatch one;
+      plan_segments(c, a, ix, i, i + 1, one, c0);
+      if (int r = inflate_stages(c, a, ix, dcomp, one)) return r;
+      ReadBack rb(c);
+      rb.add(c->d_status.p, 4);
+      rb.add(c->d_tadler.p, 4);
+      rb.add(c->d_chunk_adler.p, 4);
+      if (int r = rb.sync()) return r;
+      chunk_verdicts(one, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), chunk_status, &adler[i - c0]);
+    }
+    for (int i = c0; i < c1; i++) if (chunk_status[i]) any_bad = true;
+    if (any_bad) continue;          // the output is undefined: only the statuses of the remaining chunks are wanted
+
+    // ---- encode half: deflate d_T as mtsb_compress_chunks does
+    EncodeBatch e;
+    plan_encode_tables(c, chunk_rows, nc, itemsize, flags, c0, c1, e);
+    const int nb = e.nb, n_segs = (int)e.segs.size();
+    const size_t bbytes = (size_t)((chunk_rows[c1] - chunk_rows[c0]) * row_bytes);
+    if (int r = e.tab.stage(c)) return r;
+    NEED(c->d_tok, bbytes * 2 + 4096);
+    NEED(c->d_hist, (size_t)n_segs * HIST_STRIDE * 4);
+    NEED(c->d_codes, (size_t)n_segs * CODE_STRIDE * 4);
+    NEED(c->d_hdrs, (size_t)n_segs * HDR_WORDS * 4);
+    NEED(c->d_so, (size_t)n_segs * sizeof(DeflateSegOut));
+    NEED(c->d_seg_adler, (size_t)n_segs * 4);
+    NEED(c->d_chunk_adler, (size_t)nb * 4);
+    NEED(c->d_chunk_off, (size_t)(nb + 1) * 8);
+    NEED(c->d_subabs, (size_t)e.n_subs * 8 + 64);
+    NEED(c->d_subtok, (size_t)e.n_subs * 8 + 64);
+    NEED(c->h_small, (size_t)(nb + 1) * 8 + (size_t)nb * 4 + 64);
+    c->begin(0);
+    if (int r = e.tab.upload(c)) return r;
+    c->end();
+    void* outp = (unsigned char*)dst + total_out;
+    if (int r = io.output(c, k, outp)) return r;
+    if (int r = launch_encode(c, e, nullptr, nc, itemsize, flags, (unsigned char*)outp)) return r;
+    ReadBack rb(c);
+    rb.add(c->d_chunk_off.p, (size_t)(nb + 1) * 8);
+    rb.add(c->d_chunk_adler.p, (size_t)nb * 4);
+    if (int r = rb.sync()) return r;
+    const long long* co = rb.get<long long>(0);
+    const uint32_t* enc_adler = rb.get<uint32_t>(1);
+    if (co[nb] > e.bound) return fail(c, MTSB_E_CAPACITY, "internal: sub-batch output %lld exceeds bound %lld", co[nb], e.bound);
+    // the match finder summed the bytes it read: they must be the bytes the decode stages produced and checked
+    for (int i = 0; i < nb; i++)
+      if (enc_adler[i] != adler[i])
+        return fail(c, MTSB_E_CUDA, "internal: chunk %d: the encoder read bytes with adler32 %08x, the inflated ones have %08x",
+                    c0 + i, enc_adler[i], adler[i]);
+    for (int i = 0; i < nb; i++) out_offsets[c0 + i + 1] = total_out + co[i + 1];
+    if (int r = io.download(c, k, (char*)dst + total_out, (size_t)co[nb])) return r;
+    total_out += co[nb];
+  }
+  if (int r = io.finish(c)) return r;
+  c->collect_timing();
+  if (any_bad) return fail(c, MTSB_E_CORRUPT, "at least one compressed chunk is corrupted");
+  return 0;
 }
 
 }  // extern "C"
