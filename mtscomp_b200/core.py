@@ -14,10 +14,11 @@ ignores trailing bytes), which lets the GPU Reader decode a chunk's segments in 
 
 import bisect
 from collections import OrderedDict
-from functools import lru_cache
+from functools import lru_cache, partial
 import contextlib
 import hashlib
 import json
+from concurrent import futures
 from concurrent.futures import ThreadPoolExecutor
 import os
 import os.path as op
@@ -97,6 +98,41 @@ def _batch_ranges(bounds, row_bytes, first, last):
             hi += 1
         yield lo, hi
         lo = hi
+
+
+def _pipeline(n, stage, run, finish=None, lanes=0, desc=None, quiet=False):
+    """Run batches 0..n-1 of a whole-file operation, the caller holding codec.stage_lock.  Batch k uses the pinned
+    buffers of slot k & 1.  stage(k, slot) fills them with host reads on a stager thread, one batch ahead; run(k, slot,
+    staged) makes the GPU call and raises the operation's own errors; finish(k, slot, result) returns the batch's
+    finisher work, whose callable i runs on lane i: one thread per lane keeps each lane in batch order (the updates of
+    one SHA-1), and the lanes run side by side.  stage(k) waits for batch k-2's finisher work, which shares its slot.
+    On an error every worker is done before it propagates, and the earliest failing batch's error is raised."""
+    fins = []                                   # fins[k]: batch k's finisher futures
+
+    def stage_after(k):
+        for f in fins[k - 2] if k >= 2 else ():
+            f.result()                          # batch k-2 shares the slot; its failure stops the pipeline here
+        return stage(k, k & 1)
+
+    with ThreadPoolExecutor(1, 'mtsb-stage') as stager, contextlib.ExitStack() as stack:
+        pools = [stack.enter_context(ThreadPoolExecutor(1, 'mtsb-finish')) for _ in range(lanes)]
+        k, nxt = 0, (stager.submit(stage_after, 0) if n else None)
+        try:
+            for k in tqdm(range(n), desc=desc, disable=quiet):
+                staged = nxt.result()
+                nxt = stager.submit(stage_after, k + 1) if k + 1 < n else None
+                result = run(k, k & 1, staged)
+                work = finish(k, k & 1, result) if finish else ()
+                fins.append([pool.submit(fn) for pool, fn in zip(pools, work)])
+            for fs in fins:
+                for f in fs:
+                    f.result()
+        except BaseException as e:
+            futures.wait(([nxt] if nxt else []) + [f for fs in fins for f in fs])
+            earlier = [f.exception() for fs in fins[:k] for f in fs if f.exception() is not None]
+            if earlier and earlier[0] is not e:
+                raise earlier[0] from None
+            raise
 
 
 def _check_chunk_limits(bounds, n_channels, itemsize):
@@ -256,6 +292,37 @@ class Writer:
         """Single-chunk form of the seam, same return shape as the reference's (mtscomp.py:375-397)."""
         return chunk_idx, self.compress_batch(chunk_idx, chunk_idx + 1)[chunk_idx]
 
+    def _compress_range(self, first, last, finish, lanes):
+        """Compress chunks [first, last) on the _pipeline: stage reads a batch's rows from the memory map straight into
+        pinned w_raw%d, run packs them into pinned w_comp%d, and finish(raw, offsets, comp) gets views of both buffers
+        and the batch's chunk offsets and returns the batch's finisher work."""
+        dtype = _require_integer_dtype(self.dtype)
+        codec = _codec_for(self.config)
+        flags = _native._fl(self._flags(), dtype)
+        nc, isz, b = self.n_channels, dtype.itemsize, self.chunk_bounds
+        ranges = list(_batch_ranges(b, nc * isz, first, last))
+
+        def stage(k, slot):
+            lo, hi = ranges[k]
+            raw = raw_bufs[slot].array[:(b[hi] - b[lo]) * nc * isz]
+            np.copyto(raw.view(dtype).reshape(-1, nc), self.data[b[lo]:b[hi], :])
+            return raw
+
+        def run(k, slot, raw):
+            lo, hi = ranges[k]
+            rows = np.asarray(b[lo:hi + 1], dtype=np.int64) - b[lo]
+            offs = codec.compress_ptr(raw_bufs[slot].ptr, 0, rows, nc, isz, flags, comp_bufs[slot].ptr, 0, caps[k])
+            return raw, offs, comp_bufs[slot].array[:int(offs[-1])]
+
+        # write_index=False (Writer / compress() keyword, or "write_index" in ~/.mtscomp) gives exactly the reference's
+        # .cbin layout, one zlib stream per chunk and nothing else; the default appends the in-band index to each chunk.
+        with codec.stage_lock, _codec_param(codec, 'write_index', self.config.get('write_index')):
+            # (the bound depends on write_index: computed with it set)
+            caps = [sum(codec.compress_bound(b[i + 1] - b[i], nc, isz, flags) for i in range(lo, hi)) for lo, hi in ranges]
+            raw_bufs = [codec.host_buffer('w_raw%d' % i, max((b[hi] - b[lo]) * nc * isz for lo, hi in ranges)) for i in (0, 1)]
+            comp_bufs = [codec.host_buffer('w_comp%d' % i, max(caps)) for i in (0, 1)]
+            _pipeline(len(ranges), stage, run, lambda k, slot, res: finish(*res), lanes, 'Compressing', self.quiet)
+
     def write(self, out, outmeta):
         """Write `.cbin` and `.ch`; returns csize / raw size (reference mtscomp.py:425-507, SURVEY G7)."""
         if not out:
@@ -265,46 +332,21 @@ class Writer:
         Path(out).parent.mkdir(exist_ok=True, parents=True)
         self.chunk_offsets = [0]
         logger.info("Starting compression on the GPU.")
-        dtype = _require_integer_dtype(self.dtype)
-        codec = _codec_for(self.config)
-        flags = _native._fl(self._flags(), dtype)
-        nc, isz, b = self.n_channels, dtype.itemsize, self.chunk_bounds
-        ranges = list(_batch_ranges(b, nc * isz, 0, self.n_chunks))
-        caps = [sum(codec.compress_bound(b[i + 1] - b[i], nc, isz, flags) for i in range(lo, hi)) for lo, hi in ranges]
-        # Batches go through two pairs of PINNED staging buffers: the memory map is read straight into one (no
-        # intermediate copy), the codec fills the other with the packed streams, and while the GPU works on batch k+1 two
-        # workers finish batch k: one feeds the raw bytes to its SHA-1, the other writes and hashes the compressed bytes.
-        # The two digests the .ch format demands run at 1-2 GB/s per core and are the ceiling of this method.
-        def _write_and_hash(fb, comp):
+
+        # while the GPU works on batch k+1, two lanes finish batch k: one feeds the raw bytes to its SHA-1, the other
+        # writes and hashes the compressed bytes.  The two digests the .ch format demands run at 1-2 GB/s per core and
+        # are the ceiling of this method.
+        def write_and_hash(comp):
             fb.write(comp)
             self.sha1_compressed.update(comp)
 
-        # write_index=False (Writer / compress() keyword, or "write_index" in ~/.mtscomp) gives exactly the reference's
-        # .cbin layout, one zlib stream per chunk and nothing else; the default appends the in-band index to each chunk.
-        with codec.stage_lock, _codec_param(codec, 'write_index', self.config.get('write_index')), open(out, 'wb') as fb, \
-                ThreadPoolExecutor(1) as raw_worker, ThreadPoolExecutor(1) as out_worker:
-            if self.config.get('write_index') is not None:
-                caps = [sum(codec.compress_bound(b[i + 1] - b[i], nc, isz, flags) for i in range(lo, hi)) for lo, hi in ranges]
-            raw_bufs = [codec.host_buffer('w_raw%d' % i, max((b[hi] - b[lo]) * nc * isz for lo, hi in ranges)) for i in (0, 1)]
-            comp_bufs = [codec.host_buffer('w_comp%d' % i, max(caps)) for i in (0, 1)]
-            pending = [[], []]
-            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Compressing', disable=self.quiet)):
-                slot = k & 1
-                for f in pending[slot]:                # the slot's previous batch has been hashed and written
-                    f.result()
-                n_raw = (b[hi] - b[lo]) * nc * isz
-                raw = raw_bufs[slot].array[:n_raw]
-                np.copyto(raw.view(dtype).reshape(-1, nc), self.data[b[lo]:b[hi], :])
-                rows = np.asarray(b[lo:hi + 1], dtype=np.int64) - b[lo]
-                offs = codec.compress_ptr(raw_bufs[slot].ptr, 0, rows, nc, isz, flags, comp_bufs[slot].ptr, 0, caps[k])
-                base = self.chunk_offsets[-1]
-                self.chunk_offsets.extend(int(base + o) for o in offs[1:])
-                comp = comp_bufs[slot].array[:int(offs[-1])]
-                pending[slot] = [raw_worker.submit(self.sha1_uncompressed.update, raw),
-                                 out_worker.submit(_write_and_hash, fb, comp)]
-            for fs in pending:
-                for f in fs:
-                    f.result()
+        def finish(raw, offs, comp):
+            base = self.chunk_offsets[-1]
+            self.chunk_offsets.extend(int(base + o) for o in offs[1:])
+            return partial(self.sha1_uncompressed.update, raw), partial(write_and_hash, comp)
+
+        with open(out, 'wb') as fb:
+            self._compress_range(0, self.n_chunks, finish, 2)
             csize = fb.tell()
         assert self.chunk_offsets[-1] == csize
         ratio = csize / self.file_size
@@ -697,38 +739,41 @@ class Reader:
         dtype = _require_integer_dtype(self.dtype)
         codec = _codec_for(self.config)
         row_bytes = self.n_channels * dtype.itemsize
-        ranges = list(_batch_ranges(self.chunk_bounds, row_bytes, 0, self.n_chunks))
-        # two pinned output buffers: the GPU decodes batch k+1 into one while eight workers copy batch k from the other
+        flags = _native._fl(self._flags(), dtype)
+        b = self.chunk_bounds
+        ranges = list(_batch_ranges(b, row_bytes, 0, self.n_chunks))
+
+        def stage(k, slot):
+            lo, hi = ranges[k]
+            return self._stage_compressed(codec, [self._span(i) for i in range(lo, hi)], 'w_comp%d' % slot)
+
+        def run(k, slot, staged):
+            (cbuf, offs), (lo, hi) = staged, ranges[k]
+            status = codec.decompress_ptr(cbuf.ptr, 0, offs, self._rows_of(range(lo, hi)), self.n_channels,
+                                          dtype.itemsize, flags, bufs[slot].ptr, 0)
+            self._raise_if_corrupt(status, list(range(lo, hi)))
+
+        def finish(k, slot, _):
+            lo, hi = ranges[k]
+            pos, n, src = b[lo] * row_bytes, (b[hi] - b[lo]) * row_bytes, bufs[slot].array
+            step = max(-(-n // 8), 1 << 20)
+            return [partial(np.copyto, mm[pos + a:pos + min(a + step, n)], src[a:min(a + step, n)])
+                    for a in range(0, n, step)]
+
+        # two pinned output buffers: the GPU decodes batch k+1 into one while eight lanes copy batch k from the other
         # into a shared mapping of the output file.  (write() and pwrite() serialise on the file's write lock and run
         # at the speed of one page-cache copy — 3.5 GB/s on the bench box's tmpfs, four pwrite threads 4.3, four
         # mapping threads 5.6, eight 6.8 (tools/file_write_probe.py);
         # stores through a mapping only take per-page locks.  As with write(), nothing is fsync'ed.)
-        total = self.chunk_bounds[-1] * row_bytes
-        with codec.stage_lock, open(out, 'w+b') as fb, ThreadPoolExecutor(8) as writer:
+        total = b[-1] * row_bytes
+        with codec.stage_lock, open(out, 'w+b') as fb:
             fb.truncate(total)
             mm = np.memmap(fb, dtype=np.uint8, mode='r+', shape=(total,)) if total else None
-            n_max = max((self.chunk_bounds[hi] - self.chunk_bounds[lo]) * row_bytes for lo, hi in ranges)
+            n_max = max((b[hi] - b[lo]) * row_bytes for lo, hi in ranges)
             bufs = [codec.host_buffer('r_out%d' % i, n_max) for i in (0, 1)]
-            pending = [[], []]
-            dsize = 0
-            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Decompressing', disable=self.quiet)):
-                slot = k & 1
-                for f in pending[slot]:
-                    f.result()
-                ids = list(range(lo, hi))
-                rows = self._decode_into(ids, [self._span(i) for i in ids], bufs[slot].ptr, False)
-                n = int(rows[-1]) * row_bytes
-                src = bufs[slot].array
-                step = max(-(-n // 8), 1 << 20)
-                pending[slot] = [writer.submit(np.copyto, mm[dsize + a:dsize + min(a + step, n)], src[a:min(a + step, n)])
-                                 for a in range(0, n, step)]
-                dsize += n
-            for fs in pending:
-                for f in fs:
-                    f.result()
+            _pipeline(len(ranges), stage, run, finish, 8, 'Decompressing', self.quiet)
             del mm
-        assert dsize == self.chunk_bounds[-1] * self.n_channels * self.dtype.itemsize
-        logger.info("Wrote %s (%.1f GB).", out, dsize / 1024 ** 3)
+        logger.info("Wrote %s (%.1f GB).", out, total / 1024 ** 3)
         if self.check_after_decompress:
             decompressed = load_raw_data(out, n_channels=self.n_channels, dtype=self.dtype)
             check(decompressed, self.cdata, self.cmeta)
@@ -804,36 +849,28 @@ def _verify_range(reader, data, first, last):
     flags = _native._fl(reader._flags(), dtype)
     ranges = list(_batch_ranges(b, row_bytes, first, last))
 
-    def stage(k):
+    def stage(k, slot):
         # the Writer's staging buffers: pinned already when the check follows a write
         lo, hi = ranges[k]
-        cbuf, offs = reader._stage_compressed(codec, [reader._span(i) for i in range(lo, hi)], 'w_comp%d' % (k & 1))
+        cbuf, offs = reader._stage_compressed(codec, [reader._span(i) for i in range(lo, hi)], 'w_comp%d' % slot)
         n = (b[hi] - b[lo]) * row_bytes
-        rbuf = codec.host_buffer('w_raw%d' % (k & 1), n)
+        rbuf = codec.host_buffer('w_raw%d' % slot, n)
         _copy_rows(rbuf.array[:n].view(dtype).reshape(-1, nc), data[b[lo]:b[hi]])
         return cbuf, offs, rbuf
 
-    with codec.stage_lock, ThreadPoolExecutor(1) as stager:
-        nxt = stager.submit(stage, 0) if ranges else None
-        try:
-            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Checking')):
-                cbuf, offs, rbuf = nxt.result()
-                nxt = stager.submit(stage, k + 1) if k + 1 < len(ranges) else None
-                status, mism, at = codec.verify_ptr(cbuf.ptr, 0, offs, reader._rows_of(range(lo, hi)), nc,
-                                                    dtype.itemsize, flags, rbuf.ptr, 0, CHECK_RTOL, CHECK_ATOL)
-                bad = np.flatnonzero((status != 0) | (mism != 0))
-                if not len(bad):
-                    continue
-                i = int(bad[0])
-                if status[i]:
-                    raise IOError("Compressed chunk #%d is corrupted." % (lo + i))
-                if nxt is not None:
-                    nxt.result()
-                    nxt = None
-                raise AssertionError(_mismatch_message(reader, data, lo + i, int(mism[i]), int(at[i])))
-        finally:
-            if nxt is not None:
-                nxt.exception()          # the stager is done with its buffers before they change hands
+    def run(k, slot, staged):
+        (lo, hi), (cbuf, offs, rbuf) = ranges[k], staged
+        status, mism, at = codec.verify_ptr(cbuf.ptr, 0, offs, reader._rows_of(range(lo, hi)), nc, dtype.itemsize,
+                                            flags, rbuf.ptr, 0, CHECK_RTOL, CHECK_ATOL)
+        bad = np.flatnonzero((status != 0) | (mism != 0))
+        if len(bad):
+            i = int(bad[0])
+            if status[i]:
+                raise IOError("Compressed chunk #%d is corrupted." % (lo + i))
+            raise AssertionError(_mismatch_message(reader, data, lo + i, int(mism[i]), int(at[i])))
+
+    with codec.stage_lock:
+        _pipeline(len(ranges), stage, run, desc='Checking')
 
 
 def _mismatch_message(reader, data, idx, n_bad, at):
@@ -875,40 +912,31 @@ def _recompress_batches(r, fb, ranges, flags, write_index, quiet):
     sha1 = hashlib.sha1()
     offsets = [0]
 
-    def stage(k):
+    def stage(k, slot):
         lo, hi = ranges[k]
-        return r._stage_compressed(codec, [r._span(i) for i in range(lo, hi)], 'rc_in%d' % (k & 1))
+        return r._stage_compressed(codec, [r._span(i) for i in range(lo, hi)], 'rc_in%d' % slot)
+
+    def run(k, slot, staged):
+        (lo, hi), (cbuf, coffs) = ranges[k], staged
+        offs, status = codec.recompress_ptr(cbuf.ptr, 0, coffs, r._rows_of(range(lo, hi)), nc, isz, flags,
+                                            out_bufs[slot].ptr, 0, caps[k])
+        r._raise_if_corrupt(status, list(range(lo, hi)))
+        return offs
 
     def write_and_hash(comp):
         fb.write(comp)
         sha1.update(comp)
 
-    with codec.stage_lock, _codec_param(codec, 'write_index', write_index), \
-            ThreadPoolExecutor(1) as stager, ThreadPoolExecutor(1) as writer:
+    def finish(k, slot, offs):
+        base = offsets[-1]
+        offsets.extend(int(base + o) for o in offs[1:])
+        return partial(write_and_hash, out_bufs[slot].array[:int(offs[-1])]),
+
+    with codec.stage_lock, _codec_param(codec, 'write_index', write_index):
         # (the bound depends on write_index: computed with it set)
         caps = [sum(codec.compress_bound(b[i + 1] - b[i], nc, isz, flags) for i in range(lo, hi)) for lo, hi in ranges]
         out_bufs = [codec.host_buffer('rc_out%d' % i, max(caps)) for i in (0, 1)]
-        nxt = stager.submit(stage, 0)
-        pending = [None, None]
-        try:
-            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Recompressing', disable=quiet)):
-                slot = k & 1
-                cbuf, coffs = nxt.result()
-                nxt = stager.submit(stage, k + 1) if k + 1 < len(ranges) else None
-                if pending[slot] is not None:         # the slot's previous batch has been written
-                    pending[slot].result()
-                offs, status = codec.recompress_ptr(cbuf.ptr, 0, coffs, r._rows_of(range(lo, hi)), nc, isz, flags,
-                                                    out_bufs[slot].ptr, 0, caps[k])
-                r._raise_if_corrupt(status, list(range(lo, hi)))
-                base = offsets[-1]
-                offsets.extend(int(base + o) for o in offs[1:])
-                pending[slot] = writer.submit(write_and_hash, out_bufs[slot].array[:int(offs[-1])])
-            for f in pending:
-                if f is not None:
-                    f.result()
-        finally:
-            if nxt is not None:
-                nxt.exception()          # the stager is done with its buffer before the exception propagates
+        _pipeline(len(ranges), stage, run, finish, 1, 'Recompressing', quiet)
     return offsets, sha1
 
 
@@ -923,29 +951,24 @@ def _check_recompressed(src, new, ranges, quiet):
     flags = src._flags()                          # no MTSB_FLOAT
     block = _DeviceBlock(codec, max((b[hi] - b[lo]) * row_bytes for lo, hi in ranges) + 256)
 
-    def stage(k):
+    def stage(k, slot):
         lo, hi = ranges[k]
         ids = range(lo, hi)
-        return (src._stage_compressed(codec, [src._span(i) for i in ids], 'rc_in%d' % (k & 1)),
-                new._stage_compressed(codec, [new._span(i) for i in ids], 'rc_chk%d' % (k & 1)))
+        return (src._stage_compressed(codec, [src._span(i) for i in ids], 'rc_in%d' % slot),
+                new._stage_compressed(codec, [new._span(i) for i in ids], 'rc_chk%d' % slot))
 
-    with codec.stage_lock, ThreadPoolExecutor(1) as stager:
-        nxt = stager.submit(stage, 0)
-        try:
-            for k, (lo, hi) in enumerate(tqdm(ranges, desc='Checking', disable=quiet)):
-                (sbuf, soffs), (nbuf, noffs) = nxt.result()
-                nxt = stager.submit(stage, k + 1) if k + 1 < len(ranges) else None
-                ids = list(range(lo, hi))
-                rows = src._rows_of(ids)
-                src._raise_if_corrupt(codec.decompress_ptr(sbuf.ptr, 0, soffs, rows, nc, isz, flags, block.ptr, 1), ids)
-                status, mism, _ = codec.verify_ptr(nbuf.ptr, 0, noffs, rows, nc, isz, flags, block.ptr, 1, 0., 0.)
-                bad = np.flatnonzero((status != 0) | (mism != 0))
-                if len(bad):
-                    raise RuntimeError("recompressed chunk #%d does not decode to what the source chunk decodes to"
-                                       % ids[int(bad[0])])
-        finally:
-            if nxt is not None:
-                nxt.exception()
+    def run(k, slot, staged):
+        ids, ((sbuf, soffs), (nbuf, noffs)) = list(range(*ranges[k])), staged
+        rows = src._rows_of(ids)
+        src._raise_if_corrupt(codec.decompress_ptr(sbuf.ptr, 0, soffs, rows, nc, isz, flags, block.ptr, 1), ids)
+        status, mism, _ = codec.verify_ptr(nbuf.ptr, 0, noffs, rows, nc, isz, flags, block.ptr, 1, 0., 0.)
+        bad = np.flatnonzero((status != 0) | (mism != 0))
+        if len(bad):
+            raise RuntimeError("recompressed chunk #%d does not decode to what the source chunk decodes to"
+                               % ids[int(bad[0])])
+
+    with codec.stage_lock:
+        _pipeline(len(ranges), stage, run, desc='Checking', quiet=quiet)
 
 
 def recompress(cdata, cmeta=None, out=None, outmeta=None, write_index=True, overwrite=False, quiet=False, **kwargs):

@@ -797,8 +797,11 @@ struct EncodeBatch {
   size_t o_cd = 0, o_seg = 0, o_as = 0, o_first = 0;
 };
 
-static void plan_encode_tables(const mtsb_ctx* c, const long long* chunk_rows, int nc, int itemsize, int flags, int c0,
-                               int c1, EncodeBatch& b) {
+// The part of encode sub-batch [c0, c1) before its table upload: plan and stage the tables, size the scratch.
+// inflated: d_T already holds the sub-batch's transformed bytes (recompress), and h_small also takes the encoder's
+// per-chunk adler32s.
+static int plan_encode_sub_batch(mtsb_ctx* c, const long long* chunk_rows, int nc, int itemsize, int flags, int c0,
+                                 int c1, bool inflated, EncodeBatch& b) {
   const long long row_bytes = (long long)nc * itemsize, row0 = chunk_rows[c0];
   b.nb = c1 - c0;
   b.cds.resize(b.nb);
@@ -837,6 +840,22 @@ static void plan_encode_tables(const mtsb_ctx* c, const long long* chunk_rows, i
   b.o_seg = b.tab.add(b.segs);
   b.o_as = b.tab.add(b.as);
   b.o_first = b.tab.add(b.first);
+  const int nb = b.nb, n_segs = (int)b.segs.size();
+  const size_t bbytes = (size_t)((chunk_rows[c1] - row0) * row_bytes);
+  if (int r = b.tab.stage(c)) return r;
+  if (!inflated) NEED(c->d_T, bbytes + 16384);
+  NEED(c->d_tok, bbytes * 2 + 4096);
+  NEED(c->d_hist, (size_t)n_segs * HIST_STRIDE * 4);
+  NEED(c->d_codes, (size_t)n_segs * CODE_STRIDE * 4);
+  NEED(c->d_hdrs, (size_t)n_segs * HDR_WORDS * 4);
+  NEED(c->d_so, (size_t)n_segs * sizeof(DeflateSegOut));
+  NEED(c->d_seg_adler, (size_t)n_segs * 4);
+  NEED(c->d_chunk_adler, (size_t)nb * 4);
+  NEED(c->d_chunk_off, (size_t)(nb + 1) * 8);
+  NEED(c->d_subabs, (size_t)b.n_subs * 8 + 64);
+  NEED(c->d_subtok, (size_t)b.n_subs * 8 + 64);
+  NEED(c->h_small, (size_t)(nb + 1) * 8 + (inflated ? (size_t)nb * 4 + 64 : 0));
+  return 0;
 }
 
 // The kernels that encode one sub-batch (its tables uploaded): forward transform of `raw` into d_T, match finder,
@@ -894,6 +913,45 @@ static int launch_encode(mtsb_ctx* c, const EncodeBatch& b, const void* raw, int
   return 0;
 }
 
+// The rest of encode sub-batch k, its tables uploaded and its input ready: launch_encode into the copy pipeline's
+// output, read back the chunk offsets, fill out_offsets and queue the download to dst + total_out, which it advances.
+// want_adler (recompress): the adler32 each chunk's inflated bytes had, which the encoder's sums must equal.
+static int encode_sub_batch(mtsb_ctx* c, const EncodeBatch& b, int k, int c0, const void* raw, int nc, int itemsize,
+                            int flags, const uint32_t* want_adler, void* dst, long long& total_out, long long* out_offsets) {
+  const int nb = b.nb;
+  void* outp = (unsigned char*)dst + total_out;
+  if (int r = c->io.output(c, k, outp)) return r;
+  if (int r = launch_encode(c, b, raw, nc, itemsize, flags, (unsigned char*)outp)) return r;
+  ReadBack rb(c);
+  rb.add(c->d_chunk_off.p, (size_t)(nb + 1) * 8);
+  if (want_adler) rb.add(c->d_chunk_adler.p, (size_t)nb * 4);
+  if (int r = rb.sync()) return r;
+  const long long* co = rb.get<long long>(0);
+  if (co[nb] > b.bound) return fail(c, MTSB_E_CAPACITY, "internal: sub-batch output %lld exceeds bound %lld", co[nb], b.bound);
+  // the match finder summed the bytes it read: they must be the bytes the decode stages produced and checked
+  for (int i = 0; want_adler && i < nb; i++)
+    if (rb.get<uint32_t>(1)[i] != want_adler[i])
+      return fail(c, MTSB_E_CUDA, "internal: chunk %d: the encoder read bytes with adler32 %08x, the inflated ones have %08x",
+                  c0 + i, rb.get<uint32_t>(1)[i], want_adler[i]);
+  for (int i = 0; i < nb; i++) out_offsets[c0 + i + 1] = total_out + co[i + 1];
+  // the kernels of this sub-batch are complete (synchronised above): drain it on the copy-out stream
+  if (int r = c->io.download(c, k, (char*)dst + total_out, (size_t)co[nb])) return r;
+  total_out += co[nb];
+  return 0;
+}
+
+// dst_capacity must hold the worst-case output of every chunk
+static int check_capacity(mtsb_ctx* c, int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags,
+                          long long dst_capacity) {
+  long long need = 0;
+  for (int i = 0; i < n_chunks; i++) {
+    long long ns = chunk_rows[i + 1] - chunk_rows[i];
+    need += chunk_bound(c, ns * nc * itemsize, seg_size_for(c, ns, itemsize, flags));
+  }
+  if (dst_capacity < need) return fail(c, MTSB_E_CAPACITY, "dst_capacity %lld < bound %lld", dst_capacity, need);
+  return 0;
+}
+
 int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_chunks, const long long* chunk_rows,
                          int nc, int itemsize, int flags, void* dst, int dst_is_device, long long dst_capacity,
                          long long* out_offsets) {
@@ -902,13 +960,7 @@ int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_
   cudaSetDevice(c->device);
   c->reset_timing();
   const long long row_bytes = (long long)nc * itemsize;
-  // capacity check against the worst case
-  long long need = 0;
-  for (int i = 0; i < n_chunks; i++) {
-    long long ns = chunk_rows[i + 1] - chunk_rows[i];
-    need += chunk_bound(c, ns * row_bytes, seg_size_for(c, ns, itemsize, flags));
-  }
-  if (dst_capacity < need) return fail(c, MTSB_E_CAPACITY, "dst_capacity %lld < bound %lld", dst_capacity, need);
+  if (int r = check_capacity(c, n_chunks, chunk_rows, nc, itemsize, flags, dst_capacity)) return r;
 
   out_offsets[0] = 0;
   long long total_out = 0;
@@ -926,23 +978,7 @@ int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_
   for (int k = 0; k < n_sb; k++) {
     const int c0 = sb.first[k];
     EncodeBatch b;
-    plan_encode_tables(c, chunk_rows, nc, itemsize, flags, c0, sb.first[k + 1], b);
-    const int nb = b.nb, n_segs = (int)b.segs.size();
-    if (int r = b.tab.stage(c)) return r;
-    // scratch
-    NEED(c->d_T, sb_bytes(k) + 16384);
-    NEED(c->d_tok, sb_bytes(k) * 2 + 4096);
-    NEED(c->d_hist, (size_t)n_segs * HIST_STRIDE * 4);
-    NEED(c->d_codes, (size_t)n_segs * CODE_STRIDE * 4);
-    NEED(c->d_hdrs, (size_t)n_segs * HDR_WORDS * 4);
-    NEED(c->d_so, (size_t)n_segs * sizeof(DeflateSegOut));
-    NEED(c->d_seg_adler, (size_t)n_segs * 4);
-    NEED(c->d_chunk_adler, (size_t)nb * 4);
-    NEED(c->d_chunk_off, (size_t)(nb + 1) * 8);
-    NEED(c->d_subabs, (size_t)b.n_subs * 8 + 64);
-    NEED(c->d_subtok, (size_t)b.n_subs * 8 + 64);
-    NEED(c->h_small, (size_t)(nb + 1) * 8);
-
+    if (int r = plan_encode_sub_batch(c, chunk_rows, nc, itemsize, flags, c0, sb.first[k + 1], false, b)) return r;
     c->begin(0);
     if (int r = b.tab.upload(c)) return r;
     // only now queue the next sub-batch's upload: the copy engine serves transfers in submission order, so the small
@@ -953,18 +989,7 @@ int mtsb_compress_chunks(mtsb_ctx* c, const void* src, int src_is_device, int n_
     const void* raw = sb_src(k);
     if (int r = io.input(c, k, raw)) return r;
     c->end();
-    void* outp = (unsigned char*)dst + total_out;
-    if (int r = io.output(c, k, outp)) return r;
-    if (int r = launch_encode(c, b, raw, nc, itemsize, flags, (unsigned char*)outp)) return r;
-    ReadBack rb(c);
-    rb.add(c->d_chunk_off.p, (size_t)(nb + 1) * 8);
-    if (int r = rb.sync()) return r;
-    const long long* co = rb.get<long long>(0);
-    if (co[nb] > b.bound) return fail(c, MTSB_E_CAPACITY, "internal: sub-batch output %lld exceeds bound %lld", co[nb], b.bound);
-    for (int i = 0; i < nb; i++) out_offsets[c0 + i + 1] = total_out + co[i + 1];
-    // the kernels of this sub-batch are complete (synchronised above): drain it on the copy-out stream
-    if (int r = io.download(c, k, (char*)dst + total_out, (size_t)co[nb])) return r;
-    total_out += co[nb];
+    if (int r = encode_sub_batch(c, b, k, c0, raw, nc, itemsize, flags, nullptr, dst, total_out, out_offsets)) return r;
   }
   if (int r = io.finish(c)) return r;
   c->collect_timing();
@@ -1684,12 +1709,18 @@ static int redecode_misled(mtsb_ctx* c, const DecodeArgs& a, const std::vector<C
   return 0;
 }
 
-// The body both batch decode entry points share: plan, sub-batches through the copy pipeline, retry of misled chunks
-static int decode_call(mtsb_ctx* c, const char* name, const DecodeArgs& a, int* chunk_status) {
-  for (int i = 0; i < a.n_chunks; i++) {
-    long long l = a.comp_offsets[i + 1] - a.comp_offsets[i];
+// Every chunk's compressed length fits the kernels' 32-bit lengths and is not empty
+static int check_comp_lengths(mtsb_ctx* c, const char* name, const long long* comp_offsets, int n_chunks) {
+  for (int i = 0; i < n_chunks; i++) {
+    long long l = comp_offsets[i + 1] - comp_offsets[i];
     if (l < 1 || l > 0x7fffffffll) return fail(c, MTSB_E_ARG, "%s: bad compressed length of chunk %d", name, i);
   }
+  return 0;
+}
+
+// The body both batch decode entry points share: plan, sub-batches through the copy pipeline, retry of misled chunks
+static int decode_call(mtsb_ctx* c, const char* name, const DecodeArgs& a, int* chunk_status) {
+  if (int r = check_comp_lengths(c, name, a.comp_offsets, a.n_chunks)) return r;
   cudaSetDevice(c->device);
   c->reset_timing();
   c->par_survivors = c->par_candidates = c->par_chained = c->par_resumed = 0;
@@ -1764,20 +1795,12 @@ int mtsb_recompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, c
                            int dst_is_device, long long dst_capacity, long long* out_offsets, int* chunk_status) {
   if (!valid_common(c, n_chunks, chunk_rows, nc, itemsize) || !comp_ || !comp_offsets || !dst || !out_offsets || !chunk_status)
     return fail(c, MTSB_E_ARG, "recompress_chunks: bad arguments");
-  for (int i = 0; i < n_chunks; i++) {
-    long long l = comp_offsets[i + 1] - comp_offsets[i];
-    if (l < 1 || l > 0x7fffffffll) return fail(c, MTSB_E_ARG, "recompress_chunks: bad compressed length of chunk %d", i);
-  }
+  if (int r = check_comp_lengths(c, "recompress_chunks", comp_offsets, n_chunks)) return r;
   cudaSetDevice(c->device);
   c->reset_timing();
   c->par_survivors = c->par_candidates = c->par_chained = c->par_resumed = 0;
   const long long row_bytes = (long long)nc * itemsize;
-  long long need = 0;
-  for (int i = 0; i < n_chunks; i++) {
-    long long ns = chunk_rows[i + 1] - chunk_rows[i];
-    need += chunk_bound(c, ns * row_bytes, seg_size_for(c, ns, itemsize, flags));
-  }
-  if (dst_capacity < need) return fail(c, MTSB_E_CAPACITY, "dst_capacity %lld < bound %lld", dst_capacity, need);
+  if (int r = check_capacity(c, n_chunks, chunk_rows, nc, itemsize, flags, dst_capacity)) return r;
   const DecodeArgs a{(const unsigned char*)comp_, comp_is_device, comp_offsets, n_chunks, chunk_rows, nc, itemsize, flags,
                      nullptr, 0, row_bytes};
 
@@ -1840,42 +1863,12 @@ int mtsb_recompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, c
 
     // ---- encode half: deflate d_T as mtsb_compress_chunks does
     EncodeBatch e;
-    plan_encode_tables(c, chunk_rows, nc, itemsize, flags, c0, c1, e);
-    const int nb = e.nb, n_segs = (int)e.segs.size();
-    const size_t bbytes = (size_t)((chunk_rows[c1] - chunk_rows[c0]) * row_bytes);
-    if (int r = e.tab.stage(c)) return r;
-    NEED(c->d_tok, bbytes * 2 + 4096);
-    NEED(c->d_hist, (size_t)n_segs * HIST_STRIDE * 4);
-    NEED(c->d_codes, (size_t)n_segs * CODE_STRIDE * 4);
-    NEED(c->d_hdrs, (size_t)n_segs * HDR_WORDS * 4);
-    NEED(c->d_so, (size_t)n_segs * sizeof(DeflateSegOut));
-    NEED(c->d_seg_adler, (size_t)n_segs * 4);
-    NEED(c->d_chunk_adler, (size_t)nb * 4);
-    NEED(c->d_chunk_off, (size_t)(nb + 1) * 8);
-    NEED(c->d_subabs, (size_t)e.n_subs * 8 + 64);
-    NEED(c->d_subtok, (size_t)e.n_subs * 8 + 64);
-    NEED(c->h_small, (size_t)(nb + 1) * 8 + (size_t)nb * 4 + 64);
+    if (int r = plan_encode_sub_batch(c, chunk_rows, nc, itemsize, flags, c0, c1, true, e)) return r;
     c->begin(0);
     if (int r = e.tab.upload(c)) return r;
     c->end();
-    void* outp = (unsigned char*)dst + total_out;
-    if (int r = io.output(c, k, outp)) return r;
-    if (int r = launch_encode(c, e, nullptr, nc, itemsize, flags, (unsigned char*)outp)) return r;
-    ReadBack rb(c);
-    rb.add(c->d_chunk_off.p, (size_t)(nb + 1) * 8);
-    rb.add(c->d_chunk_adler.p, (size_t)nb * 4);
-    if (int r = rb.sync()) return r;
-    const long long* co = rb.get<long long>(0);
-    const uint32_t* enc_adler = rb.get<uint32_t>(1);
-    if (co[nb] > e.bound) return fail(c, MTSB_E_CAPACITY, "internal: sub-batch output %lld exceeds bound %lld", co[nb], e.bound);
-    // the match finder summed the bytes it read: they must be the bytes the decode stages produced and checked
-    for (int i = 0; i < nb; i++)
-      if (enc_adler[i] != adler[i])
-        return fail(c, MTSB_E_CUDA, "internal: chunk %d: the encoder read bytes with adler32 %08x, the inflated ones have %08x",
-                    c0 + i, enc_adler[i], adler[i]);
-    for (int i = 0; i < nb; i++) out_offsets[c0 + i + 1] = total_out + co[i + 1];
-    if (int r = io.download(c, k, (char*)dst + total_out, (size_t)co[nb])) return r;
-    total_out += co[nb];
+    if (int r = encode_sub_batch(c, e, k, c0, nullptr, nc, itemsize, flags, adler.data(), dst, total_out, out_offsets))
+      return r;
   }
   if (int r = io.finish(c)) return r;
   c->collect_timing();

@@ -75,29 +75,24 @@ def _barrier(group=None):
 
 
 def write_sharded(data_path, out, outmeta, rank, world, sample_rate=None, n_channels=None, dtype=None, group=None,
-                  hash_raw=True, codec=None, check_after_compress=False, before_check=None, **config):
+                  hash_raw=True, check_after_compress=False, before_check=None, **config):
     """ONE `.cbin` + `.ch` written by `world` ranks (one GPU each): every rank memory-maps the raw file, compresses its
     contiguous chunk range (shard_range) on its GPU, the per-chunk sizes are gathered on the host, and each rank writes
     its packed streams at its base offset with pwrite (reference mtscomp.py:453-486 builds the same offset table
     sequentially).  Rank 0 computes the two SHA-1 digests the format records — they are sequential passes over the raw
     and the compressed file — and writes the `.ch`.  Returns (chunk_offsets, seconds spent compressing on this rank).
-
-    `codec` is for tests (anything with compress_ptr-free `compress(data, rows, flags)`); by default the rank's
-    `_native.Codec` is used through the Writer's own batching.
+    The rank's range goes through the Writer's own batching, on the rank's `_native.Codec`.
 
     check_after_compress (off by default here): once the file is complete, each rank calls `before_check(writer)` and
     verifies its own chunk range of the written .cbin against its memory map on its GPU.  The verdicts are gathered, so
     that every rank raises the same error when any rank's check failed: the CRITICAL ERROR RuntimeError of
     Writer.write for a mismatch, IOError for a corrupt chunk (the first failure in chunk order decides)."""
     import time
-    from . import _native
-    from .core import Writer, _batch_ranges, _require_integer_dtype
+    from .core import Writer, _require_integer_dtype
     w = Writer(quiet=True, check_after_compress=check_after_compress, before_check=before_check, **config)
     w.open(data_path, sample_rate=sample_rate, n_channels=n_channels, dtype=dtype)
-    dt = _require_integer_dtype(w.dtype)
-    b, nc, isz = w.chunk_bounds, w.n_channels, dt.itemsize
+    nc, isz = w.n_channels, _require_integer_dtype(w.dtype).itemsize
     first, last = shard_range(w.n_chunks, rank, world)
-    flags = _native._fl(w._flags(), dt)
     raw_sha = None
     pool = ThreadPoolExecutor(1)
     if rank == 0 and hash_raw:
@@ -109,26 +104,14 @@ def write_sharded(data_path, out, outmeta, rank, world, sample_rate=None, n_chan
             return h.hexdigest()
         raw_sha = pool.submit(_hash_all)
     parts, sizes = [], []
+
+    def finish(raw, offs, comp):
+        sizes.extend(np.diff(offs).tolist())
+        return (lambda: parts.append(comp.copy()),)
+
     t0 = time.perf_counter()
     if last > first:
-        if codec is None:
-            codec = _native.default_codec(config.get('device', None))
-            with codec.stage_lock:
-                for lo, hi in _batch_ranges(b, nc * isz, first, last):
-                    n_raw = (b[hi] - b[lo]) * nc * isz
-                    cap = sum(codec.compress_bound(b[i + 1] - b[i], nc, isz, flags) for i in range(lo, hi))
-                    raw = codec.host_buffer('w_raw0', n_raw)
-                    comp = codec.host_buffer('w_comp0', cap)
-                    np.copyto(raw.array[:n_raw].view(dt).reshape(-1, nc), w.data[b[lo]:b[hi], :])
-                    rows = np.asarray(b[lo:hi + 1], dtype=np.int64) - b[lo]
-                    offs = codec.compress_ptr(raw.ptr, 0, rows, nc, isz, flags, comp.ptr, 0, cap)
-                    parts.append(comp.array[:int(offs[-1])].copy())
-                    sizes.extend(np.diff(offs).tolist())
-        else:
-            rows = np.asarray(b[first:last + 1], dtype=np.int64) - b[first]
-            comp, offs = codec.compress(w.data[b[first]:b[last]], rows, flags)
-            parts.append(np.asarray(comp))
-            sizes.extend(np.diff(offs).tolist())
+        w._compress_range(first, last, finish, 1)
     secs = time.perf_counter() - t0
     all_sizes = gather_sizes(sizes, group)
     offsets = assemble_offsets(all_sizes)

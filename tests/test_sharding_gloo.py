@@ -1,5 +1,5 @@
 """CPU, world_size 2 over gloo: the multi-GPU host logic — contiguous chunk ranges, size gather, offset assembly.
-The per-chunk codec is stood in for by the oracle here (this is a test; the product passes a `_native.Codec`)."""
+compress_sharded's per-chunk codec is stood in for by the oracle; write_sharded runs the host emulation of the kernels."""
 import os
 import socket
 
@@ -63,26 +63,31 @@ def test_two_ranks_reassemble_the_sequential_file(tmp_path):
     assert np.array_equal(np.concatenate(parts), want)
 
 
-def _file_worker(rank, world, port, tmp):
+def _file_worker(rank, world, port, tmp, emu_lib):
     import torch.distributed as dist
     os.environ['MASTER_ADDR'] = '127.0.0.1'
     os.environ['MASTER_PORT'] = str(port)
     dist.init_process_group('gloo', rank=rank, world_size=world)
     import mtscomp_b200 as M
+    from mtscomp_b200 import _native
     M.CONFIG_PATH = os.path.join(tmp, '.mtscomp')
+    _native._default[0] = _native.Codec(0, lib=_native.load_library(emu_lib))   # the emulated kernels as the rank's codec
     sharding.write_sharded(os.path.join(tmp, 'data.bin'), os.path.join(tmp, 'data.cbin'), os.path.join(tmp, 'data.ch'),
-                           rank, world, sample_rate=1000., n_channels=12, dtype=np.int16, codec=_OracleCodec())
+                           rank, world, sample_rate=1000., n_channels=12, dtype=np.int16)
     dist.destroy_process_group()
 
 
-def test_two_ranks_write_one_file(tmp_path):
-    """write_sharded at world size 2 (host logic only: offsets, pwrite at the rank bases, digests, .ch) gives the file
-    a sequential writer gives, and the reference's own Reader semantics hold for it (zlib per chunk, SHA-1s)."""
+def test_two_ranks_write_one_file_through_the_writer(tmp_path):
+    """write_sharded at world size 2 (offsets, pwrite at the rank bases, digests, .ch), each rank compressing through
+    the Writer's batches on the host emulation of the kernels, gives a file for which the reference's own Reader
+    semantics hold (zlib per chunk, SHA-1s)."""
     import hashlib
     import json
     import zlib
     import torch.multiprocessing as mp
+    from mtscomp_b200 import build
     from oracle import codec as ora
+    emu_lib = str(build.build_emulation())     # once here, not by both ranks at the same time
     rng = np.random.default_rng(3)
     data = np.cumsum(rng.integers(-9, 10, (7300, 12)), axis=0).astype(np.int16)
     data.tofile(tmp_path / 'data.bin')
@@ -90,7 +95,7 @@ def test_two_ranks_write_one_file(tmp_path):
     s.bind(('127.0.0.1', 0))
     port = s.getsockname()[1]
     s.close()
-    mp.spawn(_file_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
+    mp.spawn(_file_worker, args=(2, port, str(tmp_path), emu_lib), nprocs=2, join=True)
     meta = json.loads((tmp_path / 'data.ch').read_text())
     blob = (tmp_path / 'data.cbin').read_bytes()
     b, o = meta['chunk_bounds'], meta['chunk_offsets']
