@@ -146,6 +146,130 @@ __device__ unsigned long long g_lz_prof[16];
 #define LZ_PROF_ADD(i, v)
 #endif
 
+// Per-unit state of a step, from the lookup to the insert (M, mm and tokw: to the emit one step later)
+struct LzUnit {
+  unsigned M, mm, tokw;          // units on the token chain from here (stretch-local mask), matches of the stretch, token
+  unsigned hs, hl, cws, cwl;     // buckets and their words as of the end of the previous step
+  unsigned ub;                   // unit number (16 bits, biased)
+  bool vS, vL;                   // the unit goes into table S / L
+};
+
+// (A) lookup, (C) compare and stage 1 of the parse for this thread's unit of the step that starts at s0; u arrives
+// zeroed.  FULL: every unit of the step has at least 258 + 16 bytes of input from its position on -- all steps but the
+// last one or two of a segment -- so the body is compiled without the bounds tests (slen, lim), which only a step
+// near the segment's end needs.
+template <int STRIDE, int NT, bool FULL>
+__device__ __forceinline__ void lz_find(LzUnit& u, const unsigned char* ring, const unsigned* headL, const unsigned* headS,
+                                        unsigned* xs, unsigned s0, unsigned n, unsigned off0, unsigned tid,
+                                        unsigned& ad_a, unsigned& ad_c, unsigned long long& ad_b) {
+  typedef LzSmem<STRIDE, NT> L;
+  const unsigned SEG = L::SEG, RM = LZ_RING - 1, lane = tid & 31, wid = tid >> 5;
+  const unsigned* ringw = (const unsigned*)ring;
+  const unsigned slen = FULL ? SEG : min(SEG, n - s0);
+  // ---- (A) lookup + (C) compare
+  const unsigned li = tid * STRIDE;                   // local position in the step
+  const unsigned p = s0 + li;
+  u.ub = (p / STRIDE + LZ_BIAS) & 0xffffu;
+  unsigned mlen = 0, mdist = 0;
+  if (FULL || li < slen) {
+    const unsigned lim = FULL ? 258u : min(258u, n - p);
+    const unsigned pr = (p + off0) & RM;              // ring offset of this unit
+    unsigned w0, w1;
+    {
+      const unsigned* pw = ringw + (pr >> 2);
+      const unsigned sh = pr << 3;
+      const unsigned t0 = pw[0], t1 = pw[1], t2 = pw[2];
+      w0 = __funnelshift_r(t0, t1, sh); w1 = __funnelshift_r(t1, t2, sh);
+    }
+    u.tokw = STRIDE == 2 ? __byte_perm(w0, 0, 0x4140) : (w0 & 0xffu);   // literal token: the unit's bytes, one per element
+    // adler32 of the segment: a = sum of bytes, b = sum of (n - position) * byte
+    {
+      const unsigned b1 = STRIDE == 2 ? u.tokw >> 16 : 0u, sum = (u.tokw & 0xffu) + b1;
+      ad_a += sum; ad_c += b1;
+      ad_b += (unsigned long long)(n - p) * sum;
+    }
+    if (FULL || lim >= 4) {
+      u.hs = lz_hash4(w0, L::HS_BITS); u.vS = true; u.cws = headS[u.hs];
+      u.vL = FULL || lim >= 6;
+      u.hl = u.vL ? lz_hash6(w0, w1, L::HL_BITS) : 0u; u.cwl = headL[u.hl];
+      // Candidates: S newest, L newest, L second newest, evaluated without branches so that their loads are in
+      // flight together (an unusable candidate compares the unit with itself and is masked).  Fast path over
+      // the first 8 bytes: key = matched length class << 16 | ~distance, so that the largest key is the longest
+      // match and, among equals, the nearest.
+      unsigned bestk = 0;
+#pragma unroll
+      for (int k = 0; k < 3; k++) {
+        const unsigned cand = k == 0 ? u.cws >> 16 : k == 1 ? u.cwl >> 16 : u.cwl & 0xffffu;
+        const unsigned du = (u.ub - cand) & 0xffffu;          // any value: q below always lies inside the ring
+        // STEP RULE: a match must not read what its own step writes -- its source ends at or before the step's
+        // first byte, so cap = dist - li bytes are usable (candidates are units of earlier steps: dist > li; a
+        // stale table entry that points into this step is refused).  The decoder relies on it: all the tokens of
+        // a step can be resolved at once (seg_resolve_kernel).  A candidate with fewer than 8 usable bytes is not
+        // considered at all (so the 8-byte fast path needs no cap, and a long run finds the older candidate
+        // whose source is not cut short); the winner's extension is capped below.
+        const unsigned dist_k = du * STRIDE;
+        const bool ok = du - 1 < (unsigned)L::MAXD_UNITS && (k == 0 || u.vL) && dist_k >= li + 8;
+        const unsigned q = (pr - du * STRIDE) & RM;
+        const unsigned* qw = ringw + (q >> 2);
+        const unsigned sh = q << 3;
+        const unsigned t0 = qw[0], t1 = qw[1], t2 = qw[2];
+        const unsigned c0 = __funnelshift_r(t0, t1, sh), x1 = __funnelshift_r(t1, t2, sh) ^ w1;
+        // length class: 4..8 matched bytes (STRIDE 2: 4, 6, 8) from the trailing zeros of the second word's
+        // difference; 8 = the first 8 bytes match (extended below)
+        const unsigned tz = (unsigned)__clz((int)__brev(x1));   // 32 when x1 == 0
+        const unsigned lc = STRIDE == 2 ? 4u + 2u * (tz >> 4) : 4u + (tz >> 3);
+        const unsigned key = (lc << 16) | (0xffffu ^ du);
+        bestk = max(bestk, (ok && c0 == w0) ? key : 0u);
+      }
+      mlen = bestk >> 16;
+      if (mlen) {
+        mdist = (0xffffu ^ (bestk & 0xffffu)) * STRIDE;
+        const unsigned lim2 = min(lim, mdist - li);             // (step rule)
+        if (mlen == 8 && lim2 > 8) {
+          // the first 8 bytes match: check the next two bytes, which ends it for most; the few matches that go
+          // on are compared word by word (no wrap: the mirror covers pr + 258 + 8)
+          const unsigned q = (pr - mdist) & RM;
+          const bool more = STRIDE == 2 ? *(const unsigned short*)(ring + pr + 8) == *(const unsigned short*)(ring + q + 8)
+                                        : ring[pr + 8] == ring[q + 8];
+          if (more) {
+            unsigned x = 0;
+            while (mlen < lim2) {
+              x = ring_load4(ring, pr + mlen) ^ ring_load4(ring, q + mlen);
+              if (x) break;
+              mlen += 4;
+            }
+            if (x) mlen += (unsigned)(__ffs((int)x) - 1) >> 3;
+          }
+        }
+        mlen = min(mlen, lim2);
+        if (STRIDE == 2) mlen &= ~1u;                 // matches cover whole units
+        if (mlen < 4) mlen = 0;
+        else u.tokw = (0x8000u | mlen) | ((mdist - 1) << 16);
+      }
+    }
+  }
+  // ---- (D) greedy parse over units, hierarchical; thread = unit, warp = stretch of 32 units.
+  //      Stage 1 (registers, shuffles; here): pointer doubling gives every unit the exit of the token chain that
+  //      starts there (where it leaves the stretch) and the mask of the units it visits (= its tokens).
+  //      Stage 2 (chain warp): chains the stretches from the carried start (entry + element base per stretch).
+  //      Stage 3 (one step later): the warp picks the mask of its entry unit and emits those tokens.
+  //      A token is 2 elements (match: length, distance; STRIDE 2 literal: the unit's two bytes) or 1 (STRIDE 1 literal).
+  const unsigned nu = (slen + STRIDE - 1) / STRIDE;   // units in this step
+  const unsigned sb = wid * 32;
+  const unsigned sel = FULL ? 32u : min(sb + 32, nu) > sb ? min(sb + 32, nu) - sb : 0u;   // valid lanes of this stretch
+  u.mm = __ballot_sync(0xffffffffu, mlen != 0);
+  u.M = 1u << lane;
+  unsigned v = lane + (mlen ? mlen / STRIDE : 1u);   // next unit (stretch-local)
+#pragma unroll
+  for (unsigned r = 0; r < 5; r++) {
+    const unsigned tv = __shfl_sync(0xffffffffu, v, v & 31);
+    const unsigned tM = __shfl_sync(0xffffffffu, u.M, v & 31);
+    if (v < sel) { v = tv; u.M |= tM; }
+  }
+  const unsigned els = STRIDE == 2 ? 2 * __popc(u.M) : __popc(u.M) + __popc(u.M & u.mm);
+  xs[tid] = (sb + v) | (els << 16);
+}
+
 template <int STRIDE, int NT>
 __global__ void __launch_bounds__(NT + 32, NT <= 512 ? 2 : 1) lz77_kernel(const unsigned char* __restrict__ tbuf,
                                                                           const DeflateSeg* __restrict__ segs, int n_segs,
@@ -160,7 +284,6 @@ __global__ void __launch_bounds__(NT + 32, NT <= 512 ? 2 : 1) lz77_kernel(const 
   const int NALL = NT + 32;                                       // unit threads + the chain warp
   MTS_DYN_SMEM(sm);
   unsigned char* ring = sm + L::ring_off;
-  const unsigned* ringw = (const unsigned*)ring;
   unsigned* headL = (unsigned*)(sm + L::headl_off);
   unsigned* headS = (unsigned*)(sm + L::heads_off);
   unsigned* xe = (unsigned*)(sm + L::xe_off);                    // [step parity][unit]: exit of its stretch | token elements << 16
@@ -242,125 +365,23 @@ __global__ void __launch_bounds__(NT + 32, NT <= 512 ? 2 : 1) lz77_kernel(const 
     mbar_wait(mbar, phase & 1); phase++;
     unsigned pM = 0, pmm = 0, ptok = 0;                      // previous step's stage-1 results (emitted one step later)
     for (unsigned step = 0; step <= n_steps; step++) {
-      unsigned M = 0, mm = 0, tokw = 0, hs = 0, hl = 0, cwl = 0, cws = 0, ub = 0;
-      bool vS = false, vL = false;
+      LzUnit u = {};
       LZ_PROF_T(t_step);
       if (step < n_steps) {
         const unsigned s0 = step * SEG;                    // first position of this step
-        const unsigned slen = min(SEG, n - s0);
         // piece step + 1 (issued during the previous step) must have landed: this step reads up to s0 + SEG + 294
         if (step > 0 && (step + 1) * SEG < n_ring) { mbar_wait(mbar, phase & 1); phase++; }
-
-        // ---- (A) lookup + (C) compare
-        const unsigned li = tid * STRIDE;                   // local position in the step
-        const unsigned p = s0 + li;
-        ub = (p / STRIDE + LZ_BIAS) & 0xffffu;
-        unsigned mlen = 0, mdist = 0;
-        if (li < slen) {
-          const unsigned lim = min(258u, n - p);
-          const unsigned pr = (p + off0) & RM;              // ring offset of this unit
-          unsigned w0, w1;
-          {
-            const unsigned* pw = ringw + (pr >> 2);
-            const unsigned sh = pr << 3;
-            const unsigned t0 = pw[0], t1 = pw[1], t2 = pw[2];
-            w0 = __funnelshift_r(t0, t1, sh); w1 = __funnelshift_r(t1, t2, sh);
-          }
-          tokw = STRIDE == 2 ? __byte_perm(w0, 0, 0x4140) : (w0 & 0xffu);   // literal token: the unit's bytes, one per element
-          // adler32 of the segment: a = sum of bytes, b = sum of (n - position) * byte
-          {
-            const unsigned b1 = STRIDE == 2 ? tokw >> 16 : 0u, sum = (tokw & 0xffu) + b1;
-            ad_a += sum; ad_c += b1;
-            ad_b += (unsigned long long)(n - p) * sum;
-          }
-          if (lim >= 4) {
-            hs = lz_hash4(w0, L::HS_BITS); vS = true; cws = headS[hs];
-            vL = lim >= 6;
-            hl = vL ? lz_hash6(w0, w1, L::HL_BITS) : 0u; cwl = headL[hl];
-            // Candidates: S newest, L newest, L second newest, evaluated without branches so that their loads are in
-            // flight together (an unusable candidate compares the unit with itself and is masked).  Fast path over
-            // the first 8 bytes: key = matched length class << 16 | ~distance, so that the largest key is the longest
-            // match and, among equals, the nearest.
-            unsigned bestk = 0;
-#pragma unroll
-            for (int k = 0; k < 3; k++) {
-              const unsigned cand = k == 0 ? cws >> 16 : k == 1 ? cwl >> 16 : cwl & 0xffffu;
-              const unsigned du = (ub - cand) & 0xffffu;          // any value: q below always lies inside the ring
-              // STEP RULE: a match must not read what its own step writes -- its source ends at or before the step's
-              // first byte, so cap = dist - li bytes are usable (candidates are units of earlier steps: dist > li; a
-              // stale table entry that points into this step is refused).  The decoder relies on it: all the tokens of
-              // a step can be resolved at once (seg_resolve_kernel).  A candidate with fewer than 8 usable bytes is not
-              // considered at all (so the 8-byte fast path needs no cap, and a long run finds the older candidate
-              // whose source is not cut short); the winner's extension is capped below.
-              const unsigned dist_k = du * STRIDE;
-              const bool ok = du - 1 < (unsigned)L::MAXD_UNITS && (k == 0 || vL) && dist_k >= li + 8;
-              const unsigned q = (pr - du * STRIDE) & RM;
-              const unsigned* qw = ringw + (q >> 2);
-              const unsigned sh = q << 3;
-              const unsigned t0 = qw[0], t1 = qw[1], t2 = qw[2];
-              const unsigned c0 = __funnelshift_r(t0, t1, sh), x1 = __funnelshift_r(t1, t2, sh) ^ w1;
-              // length class: 4..8 matched bytes (STRIDE 2: 4, 6, 8) from the trailing zeros of the second word's
-              // difference; 8 = the first 8 bytes match (extended below)
-              const unsigned tz = (unsigned)__clz((int)__brev(x1));   // 32 when x1 == 0
-              const unsigned lc = STRIDE == 2 ? 4u + 2u * (tz >> 4) : 4u + (tz >> 3);
-              const unsigned key = (lc << 16) | (0xffffu ^ du);
-              bestk = max(bestk, (ok && c0 == w0) ? key : 0u);
-            }
-            mlen = bestk >> 16;
-            if (mlen) {
-              mdist = (0xffffu ^ (bestk & 0xffffu)) * STRIDE;
-              const unsigned lim2 = min(lim, mdist - li);             // (step rule)
-              if (mlen == 8 && lim2 > 8) {
-                // the first 8 bytes match: check the next two bytes, which ends it for most; the few matches that go
-                // on are compared word by word (no wrap: the mirror covers pr + 258 + 8)
-                const unsigned q = (pr - mdist) & RM;
-                const bool more = STRIDE == 2 ? *(const unsigned short*)(ring + pr + 8) == *(const unsigned short*)(ring + q + 8)
-                                              : ring[pr + 8] == ring[q + 8];
-                if (more) {
-                  unsigned x = 0;
-                  while (mlen < lim2) {
-                    x = ring_load4(ring, pr + mlen) ^ ring_load4(ring, q + mlen);
-                    if (x) break;
-                    mlen += 4;
-                  }
-                  if (x) mlen += (unsigned)(__ffs((int)x) - 1) >> 3;
-                }
-              }
-              mlen = min(mlen, lim2);
-              if (STRIDE == 2) mlen &= ~1u;                 // matches cover whole units
-              if (mlen < 4) mlen = 0;
-              else tokw = (0x8000u | mlen) | ((mdist - 1) << 16);
-            }
-          }
-        }
-        // ---- (D) greedy parse over units, hierarchical; thread = unit, warp = stretch of 32 units.
-        //      Stage 1 (registers, shuffles; here): pointer doubling gives every unit the exit of the token chain that
-        //      starts there (where it leaves the stretch) and the mask of the units it visits (= its tokens).
-        //      Stage 2 (chain warp): chains the stretches from the carried start (entry + element base per stretch).
-        //      Stage 3 (one step later): the warp picks the mask of its entry unit and emits those tokens.
-        //      A token is 2 elements (match: length, distance; STRIDE 2 literal: the unit's two bytes) or 1 (STRIDE 1 literal).
-        const unsigned nu = (slen + STRIDE - 1) / STRIDE;   // units in this step
-        const unsigned sb = wid * 32;
-        const unsigned sel = min(sb + 32, nu) > sb ? min(sb + 32, nu) - sb : 0;   // valid lanes of this stretch
-        mm = __ballot_sync(0xffffffffu, mlen != 0);
-        M = 1u << lane;
-        unsigned v = lane + (mlen ? mlen / STRIDE : 1u);   // next unit (stretch-local)
-#pragma unroll
-        for (unsigned r = 0; r < 5; r++) {
-          const unsigned tv = __shfl_sync(0xffffffffu, v, v & 31);
-          const unsigned tM = __shfl_sync(0xffffffffu, M, v & 31);
-          if (v < sel) { v = tv; M |= tM; }
-        }
-        const unsigned els = STRIDE == 2 ? 2 * __popc(M) : __popc(M) + __popc(M & mm);
-        xe[(step & 1) * NT + tid] = (sb + v) | (els << 16);
+        unsigned* xs = xe + (step & 1) * NT;
+        if (s0 + SEG + 258 + 16 <= n) lz_find<STRIDE, NT, true>(u, ring, headL, headS, xs, s0, n, off0, tid, ad_a, ad_c, ad_b);
+        else lz_find<STRIDE, NT, false>(u, ring, headL, headS, xs, s0, n, off0, tid, ad_a, ad_c, ad_b);
       }
       LZ_PROF_T(t_a);
       named_barrier(1, NALL);                             // #1: every lookup of this step is done; stage 2 of the previous step too
 
       // ---- (B) insert, first round: any unit of the step becomes the bucket's newest; the next piece of input
-      const unsigned myL = (ub << 16) | (cwl >> 16), myS = (ub << 16) | (cws >> 16);
-      if (vL) headL[hl] = myL;
-      if (vS) headS[hs] = myS;
+      const unsigned myL = (u.ub << 16) | (u.cwl >> 16), myS = (u.ub << 16) | (u.cws >> 16);
+      if (u.vL) headL[u.hl] = myL;
+      if (u.vS) headS[u.hs] = myS;
       if (tid == 0 && (step + 2) * SEG < n_ring) {
         const unsigned c0 = (step + 2) * SEG, o = c0 & RM;
         const unsigned len = min(SEG, (n_ring - c0 + 15) & ~15u), mir = o == 0 ? min((unsigned)LZ_MIRROR, len) : 0u;
@@ -410,13 +431,13 @@ __global__ void __launch_bounds__(NT + 32, NT <= 512 ? 2 : 1) lz77_kernel(const 
         run_tok += ms[64];
       }
       if (step == n_steps) break;
-      pM = M; pmm = mm; ptok = tokw;
+      pM = u.M; pmm = u.mm; ptok = u.tokw;
       LZ_PROF_T(t_b);
       named_barrier(2, NALL);                             // #2: first-round stores are visible (and xe[] to the chain warp)
 
       // ---- (B) insert, second round: a lower unit of this step in my bucket gives way
-      if (vL) { const unsigned d = (ub - (headL[hl] >> 16)) & 0xffffu; if (d - 1 < NT - 1) atomicMax(&headL[hl], myL); }
-      if (vS) { const unsigned d = (ub - (headS[hs] >> 16)) & 0xffffu; if (d - 1 < NT - 1) atomicMax(&headS[hs], myS); }
+      if (u.vL) { const unsigned d = (u.ub - (headL[u.hl] >> 16)) & 0xffffu; if (d - 1 < NT - 1) atomicMax(&headL[u.hl], myL); }
+      if (u.vS) { const unsigned d = (u.ub - (headS[u.hs] >> 16)) & 0xffffu; if (d - 1 < NT - 1) atomicMax(&headS[u.hs], myS); }
       LZ_PROF_T(t_c);
       named_barrier(3, NT);                               // #3: buckets settled
       LZ_PROF_ADD(0, 1); LZ_PROF_ADD(1, t_a - t_step); LZ_PROF_ADD(2, t_b - t_a); LZ_PROF_ADD(3, t_c - t_b); LZ_PROF_ADD(5, t_c - t_step);
