@@ -104,8 +104,9 @@ int mtsb_compress_chunks(mtsb_ctx* ctx, const void* src, int src_is_device, int 
  * step at once); any other valid zlib stream (e.g. written by the reference) by the block-parallel decoder, which
  * finds the deflate blocks itself; what neither takes is decoded serially by one warp, which also decides what is
  * corrupt.  A chunk whose trailing bytes look like an index but do not decode with it is decoded again as a plain
- * stream (zlib ignores what follows a stream, so such a chunk is valid).  chunk_status (n_chunks host ints, may be NULL) receives
- * MTSB_CHUNK_*; the call returns MTSB_E_CORRUPT if any is non-zero. */
+ * stream (zlib ignores what follows a stream, so such a chunk is valid), whether or not chunk_status is given.
+ * chunk_status (n_chunks host ints, may be NULL) receives MTSB_CHUNK_*; the call returns MTSB_E_CORRUPT if any chunk
+ * is corrupt. */
 int mtsb_decompress_chunks(mtsb_ctx* ctx, const void* comp, int comp_is_device, const long long* comp_offsets,
                            int n_chunks, const long long* chunk_rows, int nc, int itemsize, int flags, void* dst,
                            int dst_is_device, int* chunk_status);

@@ -165,7 +165,6 @@ struct mtsb_ctx {
   long long par_single_pass = 1;   // par_block_kernel keeps the tokens of its counting pass (see par_decode)
   Buf d_segv2, d_btab, d_subout;                                                          // indexed (second format) segments
   long long seg_v2 = 1;         // indexed segments of the second format go through seg_tokens / seg_resolve
-  bool ignore_index = false;    // (internal) decode every chunk as a plain zlib stream: the retry of chunks whose index misled
   Buf d_raw, d_raw2, d_out2, d_comp2, d_T, d_tok, d_hist, d_codes, d_hdrs, d_tab, d_so, d_seg_adler, d_chunk_adler, d_chunk_off, d_out,
       d_partial, d_comp, d_status, d_tadler, d_gather, d_subabs, d_subtok, d_invstate, d_invcells;
   Buf d_ref, d_ref2, d_vcount;     // verify: the reference rows of a host reference (a pair), the per-chunk counters
@@ -1073,7 +1072,7 @@ static int read_indexes(mtsb_ctx* c, const DecodeArgs& a, std::vector<ChunkIndex
   std::vector<unsigned char> tails;
   for (int i = 0; i < a.n_chunks; i++) {
     long long l = a.comp_offsets[i + 1] - a.comp_offsets[i];
-    if (l >= 2 + 6 + 4 + INDEX_TAIL && !c->ignore_index) { off.push_back(a.comp_offsets[i + 1] - INDEX_TAIL); len.push_back(INDEX_TAIL); who.push_back(i); }
+    if (l >= 2 + 6 + 4 + INDEX_TAIL) { off.push_back(a.comp_offsets[i + 1] - INDEX_TAIL); len.push_back(INDEX_TAIL); who.push_back(i); }
   }
   if (int r = fetch_ranges(c, a.comp, a.comp_is_device, off, len, tails, pos)) return r;
   std::vector<int> who2;
@@ -1548,11 +1547,9 @@ static int serial_inflate(mtsb_ctx* c, const unsigned char* dcomp, const std::ve
 
 // Each chunk's status: its first failing segment's, else INF_BAD_ADLER where the adler32 of its transformed bytes is not
 // the stored one (the index's, or the zlib trailer's the serial kernel read: ta).  st: the segments' statuses, ca: the
-// adler kernels' sums.  accepted (may be null): per chunk, the stored adler32 that a good chunk matched.  Returns
-// whether a chunk failed.
-static bool chunk_verdicts(const DecodeBatch& b, const std::vector<ChunkIndex>& ix, const int* st, const uint32_t* ta,
-                           const uint32_t* ca, int* status, uint32_t* accepted = nullptr) {
-  bool bad = false;
+// adler kernels' sums.  accepted (may be null): per chunk, the stored adler32 that a good chunk matched.
+static void chunk_verdicts(const DecodeBatch& b, const std::vector<ChunkIndex>& ix, const int* st, const uint32_t* ta,
+                           const uint32_t* ca, int* status, uint32_t* accepted) {
   for (int i = 0; i < b.nb; i++) {
     int s = 0;
     for (int j = b.first[i]; j < b.first[i + 1] && !s; j++) s = st[j];
@@ -1562,10 +1559,8 @@ static bool chunk_verdicts(const DecodeBatch& b, const std::vector<ChunkIndex>& 
       if (want != (b.have_adler[i] ? b.adler[i] : ca[i])) s = INF_BAD_ADLER;
       if (accepted) accepted[i] = want;
     }
-    if (s) bad = true;
     status[b.c0 + i] = s;
   }
-  return bad;
 }
 
 // The rows of sub-batch k in the caller's `ref` (verify)
@@ -1637,42 +1632,36 @@ static int inflate_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<Chu
   return inflate_stages(c, a, ix, dcomp, b);
 }
 
-// Sub-batch k: inflate_batch, inverse transform, verdicts.  Verify: the inverse writes to scratch (d_out), the compare
-// follows on the same stream and its counters come back with the verdicts.
-static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const Batches& sb, int k,
-                        int* status, bool& any_bad) {
-  CopyPipe& io = c->io;
-  DecodeBatch b;
-  const unsigned char* dcomp = nullptr;
-  const void* ref = nullptr;
-  if (int r = inflate_batch(c, a, ix, sb, k, b, dcomp, ref)) return r;
-  const int c0 = b.c0, nb = b.nb, n_segs = (int)b.segs.size();
-  const long long row0 = a.chunk_rows[c0], bbytes = (a.chunk_rows[sb.first[k + 1]] - row0) * a.row_bytes;
-  const size_t o_cd = b.o_cd;
-  void* outp = a.verify ? c->d_out.p : (char*)a.dst + row0 * a.row_bytes;
-  if (!a.verify) {
-    if (int r = io.output(c, k, outp)) return r;
-  }
+// The rows of b's chunks from d_T into outp (the sub-batch's first row; span_elems: the sub-batch's elements) and,
+// verify, their compare with the sub-batch's reference rows `ref`
+static int inverse_stages(mtsb_ctx* c, const DecodeArgs& a, const DecodeBatch& b, void* outp, const void* ref,
+                          size_t span_elems) {
+  const int nb = b.nb;
+  const ChunkDesc* d_cd = TableBlob::dev<ChunkDesc>(c, b.o_cd);
   c->begin(4);
-  if (int r = launch_inv(c, a.itemsize, c->d_T.p, outp, TableBlob::dev<ChunkDesc>(c, o_cd), nb, b.max_ns, a.nc, a.flags, (size_t)(bbytes / a.itemsize))) return r;
+  if (int r = launch_inv(c, a.itemsize, c->d_T.p, outp, d_cd, nb, b.max_ns, a.nc, a.flags, span_elems)) return r;
   c->end();
-  if (a.verify) {
-    NEED(c->d_vcount, (size_t)nb * 16);
-    NEED(c->h_small, (size_t)n_segs * 8 + (size_t)nb * 20 + 160);
-    c->begin(6);
-    if (int r = launch_verify(c, a.itemsize, a.flags, outp, ref, TableBlob::dev<ChunkDesc>(c, o_cd), nb, b.max_ns, a.nc, a.rtol, a.atol)) return r;
-    c->end();
-  }
+  if (!a.verify) return 0;
+  NEED(c->d_vcount, (size_t)nb * 16);
+  NEED(c->h_small, b.segs.size() * 8 + (size_t)nb * 20 + 160);
+  c->begin(6);
+  if (int r = launch_verify(c, a.itemsize, a.flags, outp, ref, d_cd, nb, b.max_ns, a.nc, a.rtol, a.atol)) return r;
+  c->end();
+  return 0;
+}
+
+// One synchronisation for what the stages of b left on the device, then b's statuses (chunk_verdicts, `accepted` as
+// there) and, verify, its compare counters
+static int batch_verdicts(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, const DecodeBatch& b,
+                          int* status, uint32_t* accepted = nullptr) {
+  const int c0 = b.c0, nb = b.nb, n_segs = (int)b.segs.size();
   ReadBack rb(c);
   rb.add(c->d_status.p, (size_t)n_segs * 4);
   rb.add(c->d_tadler.p, (size_t)n_segs * 4);
   rb.add(c->d_chunk_adler.p, (size_t)nb * 4);
   if (a.verify) rb.add(c->d_vcount.p, (size_t)nb * 16);
   if (int r = rb.sync()) return r;
-  if (!a.verify) {
-    if (int r = io.download(c, k, (char*)a.dst + row0 * a.row_bytes, (size_t)bbytes)) return r;
-  }
-  if (chunk_verdicts(b, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), status)) any_bad = true;
+  chunk_verdicts(b, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), status, accepted);
   if (a.verify) {
     const long long* cnt = rb.get<long long>(3);
     for (int i = 0; i < nb; i++) {
@@ -1685,57 +1674,78 @@ static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, const std::vector<Chun
 }
 
 // A chunk that carries something that looks like an index but does not decode with it (bytes after a foreign zlib
-// stream that happen to pass the index checks) is still a valid chunk for zlib, which ignores what follows the stream:
-// each such chunk is decoded again as a plain stream before it is called corrupt.  any_bad: whether a chunk stays bad.
-static int redecode_misled(mtsb_ctx* c, const DecodeArgs& a, const std::vector<ChunkIndex>& ix, int* status, bool& any_bad) {
-  any_bad = false;
-  for (int i = 0; i < a.n_chunks; i++) {
-    if (!status[i]) continue;
-    if (!ix[i].n_seg) { any_bad = true; continue; }
-    const long long one_off[2] = {0, a.comp_offsets[i + 1] - a.comp_offsets[i]}, one_rows[2] = {0, a.chunk_rows[i + 1] - a.chunk_rows[i]};
-    int st = 0;
-    c->ignore_index = true;
-    const int rc = a.verify
-        ? mtsb_verify_chunks(c, a.comp + a.comp_offsets[i], a.comp_is_device, one_off, 1, one_rows, a.nc, a.itemsize, a.flags,
-                             (const char*)a.ref + a.chunk_rows[i] * a.row_bytes, a.ref_is_device, a.rtol, a.atol,
-                             a.mismatches + i, a.first_mismatch + i, &st)
-        : mtsb_decompress_chunks(c, a.comp + a.comp_offsets[i], a.comp_is_device, one_off, 1, one_rows, a.nc, a.itemsize,
-                                 a.flags, (char*)a.dst + a.chunk_rows[i] * a.row_bytes, a.dst_is_device, &st);
-    c->ignore_index = false;
-    if (rc != 0 && rc != MTSB_E_CORRUPT) return rc;
-    status[i] = st;
-    if (st) any_bad = true;
+// stream that happen to pass the index checks) is still a valid chunk for zlib, which ignores what follows the stream.
+// Each such chunk of sub-batch b is inflated again alone as a plain stream into its own place in d_T (dcomp: the
+// sub-batch's compressed bytes), its rows go to their place at outp as inverse_stages puts them (outp null: recompress,
+// d_T only), and it gets a new verdict.  The sub-batch's buffers are still in their copy-pipeline slots: nothing of it
+// has been downloaded yet, and the next uploads go to the other slot.
+static int retry_misled(mtsb_ctx* c, const DecodeArgs& a, std::vector<ChunkIndex>& ix, const DecodeBatch& b,
+                        const unsigned char* dcomp, void* outp, const void* ref, size_t span_elems, int* status,
+                        uint32_t* accepted = nullptr) {
+  for (int i = b.c0; i < b.c0 + b.nb; i++) {
+    if (!status[i] || !ix[i].n_seg) continue;
+    ix[i] = ChunkIndex();
+    DecodeBatch one;
+    plan_segments(c, a, ix, i, i + 1, one, b.c0);
+    if (int r = inflate_stages(c, a, ix, dcomp, one)) return r;
+    if (outp) {
+      if (int r = inverse_stages(c, a, one, outp, ref, span_elems)) return r;
+    }
+    if (int r = batch_verdicts(c, a, ix, one, status, accepted ? accepted + (i - b.c0) : nullptr)) return r;
   }
   return 0;
 }
 
-// Every chunk's compressed length fits the kernels' 32-bit lengths and is not empty
-static int check_comp_lengths(mtsb_ctx* c, const char* name, const long long* comp_offsets, int n_chunks) {
-  for (int i = 0; i < n_chunks; i++) {
-    long long l = comp_offsets[i + 1] - comp_offsets[i];
+// Sub-batch k: inflate_batch, inverse transform, verdicts, retry of misled chunks, download.  Verify: the inverse
+// writes to scratch (d_out), the compare follows on the same stream and its counters come back with the verdicts.
+static int decode_batch(mtsb_ctx* c, const DecodeArgs& a, std::vector<ChunkIndex>& ix, const Batches& sb, int k,
+                        int* status) {
+  DecodeBatch b;
+  const unsigned char* dcomp = nullptr;
+  const void* ref = nullptr;
+  if (int r = inflate_batch(c, a, ix, sb, k, b, dcomp, ref)) return r;
+  const long long row0 = a.chunk_rows[b.c0], bbytes = (a.chunk_rows[sb.first[k + 1]] - row0) * a.row_bytes;
+  const size_t span_elems = (size_t)(bbytes / a.itemsize);
+  void* outp = a.verify ? c->d_out.p : (char*)a.dst + row0 * a.row_bytes;
+  if (!a.verify) {
+    if (int r = c->io.output(c, k, outp)) return r;
+  }
+  if (int r = inverse_stages(c, a, b, outp, ref, span_elems)) return r;
+  if (int r = batch_verdicts(c, a, ix, b, status)) return r;
+  if (int r = retry_misled(c, a, ix, b, dcomp, outp, ref, span_elems, status)) return r;
+  if (!a.verify) {
+    if (int r = c->io.download(c, k, (char*)a.dst + row0 * a.row_bytes, (size_t)bbytes)) return r;
+  }
+  return 0;
+}
+
+// The start of every call that decodes (decompress, verify, recompress): the compressed lengths fit the kernels'
+// 32-bit lengths and are not empty; timings and statistics restart; the segment index behind each chunk's zlib stream
+// is read (timed in slot 1) into ix, whose records point into ix_bytes; all n_chunks statuses are 0.
+static int start_decode_call(mtsb_ctx* c, const char* name, const DecodeArgs& a, int* status,
+                             std::vector<ChunkIndex>& ix, std::vector<unsigned char>& ix_bytes) {
+  for (int i = 0; i < a.n_chunks; i++) {
+    long long l = a.comp_offsets[i + 1] - a.comp_offsets[i];
     if (l < 1 || l > 0x7fffffffll) return fail(c, MTSB_E_ARG, "%s: bad compressed length of chunk %d", name, i);
   }
-  return 0;
-}
-
-// The body both batch decode entry points share: plan, sub-batches through the copy pipeline, retry of misled chunks
-static int decode_call(mtsb_ctx* c, const char* name, const DecodeArgs& a, int* chunk_status) {
-  if (int r = check_comp_lengths(c, name, a.comp_offsets, a.n_chunks)) return r;
   cudaSetDevice(c->device);
   c->reset_timing();
   c->par_survivors = c->par_candidates = c->par_chained = c->par_resumed = 0;
-
-  // ---- plan: look for the segment index after each chunk's zlib stream
   c->begin(1);
-  std::vector<ChunkIndex> ix;
-  std::vector<unsigned char> ix_bytes;
   if (int r = read_indexes(c, a, ix, ix_bytes)) return r;
   c->end();
+  for (int i = 0; i < a.n_chunks; i++) status[i] = 0;
+  return 0;
+}
 
+// The body both batch decode entry points share: plan, sub-batches through the copy pipeline
+static int decode_call(mtsb_ctx* c, const char* name, const DecodeArgs& a, int* chunk_status) {
   // every chunk's status, also when the caller does not ask for them
   std::vector<int> own_status(chunk_status ? 0 : a.n_chunks);
   int* status = chunk_status ? chunk_status : own_status.data();
-  for (int i = 0; i < a.n_chunks; i++) status[i] = 0;
+  std::vector<ChunkIndex> ix;
+  std::vector<unsigned char> ix_bytes;
+  if (int r = start_decode_call(c, name, a, status, ix, ix_bytes)) return r;
   const Batches sb = plan_decode_batches(c, a, ix);
   const int n_sb = sb.count();
   if (!a.comp_is_device) { NEED(c->d_comp, (size_t)sb.max_in + 256); if (n_sb > 1) NEED(c->d_comp2, (size_t)sb.max_in + 256); }
@@ -1750,15 +1760,12 @@ static int decode_call(mtsb_ctx* c, const char* name, const DecodeArgs& a, int* 
                                   &c->d_ref2, ref_rows(a, sb, 0), batch_bytes_of(a, sb, 0))
                     : c->io.start(c, in0, &c->d_comp2, host_rows ? &c->d_out : nullptr, &c->d_out2, comp0, comp_bytes0);
   if (r0) return r0;
-  bool any_bad = false;
   for (int k = 0; k < n_sb; k++)
-    if (int r = decode_batch(c, a, ix, sb, k, status, any_bad)) return r;
+    if (int r = decode_batch(c, a, ix, sb, k, status)) return r;
   if (int r = c->io.finish(c)) return r;
   c->collect_timing();
-  if (any_bad && chunk_status && !c->ignore_index) {
-    if (int r = redecode_misled(c, a, ix, status, any_bad)) return r;
-  }
-  if (any_bad) return fail(c, MTSB_E_CORRUPT, "at least one compressed chunk is corrupted");
+  for (int i = 0; i < a.n_chunks; i++)
+    if (status[i]) return fail(c, MTSB_E_CORRUPT, "at least one compressed chunk is corrupted");
   return 0;
 }
 
@@ -1795,21 +1802,13 @@ int mtsb_recompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, c
                            int dst_is_device, long long dst_capacity, long long* out_offsets, int* chunk_status) {
   if (!valid_common(c, n_chunks, chunk_rows, nc, itemsize) || !comp_ || !comp_offsets || !dst || !out_offsets || !chunk_status)
     return fail(c, MTSB_E_ARG, "recompress_chunks: bad arguments");
-  if (int r = check_comp_lengths(c, "recompress_chunks", comp_offsets, n_chunks)) return r;
-  cudaSetDevice(c->device);
-  c->reset_timing();
-  c->par_survivors = c->par_candidates = c->par_chained = c->par_resumed = 0;
   const long long row_bytes = (long long)nc * itemsize;
-  if (int r = check_capacity(c, n_chunks, chunk_rows, nc, itemsize, flags, dst_capacity)) return r;
   const DecodeArgs a{(const unsigned char*)comp_, comp_is_device, comp_offsets, n_chunks, chunk_rows, nc, itemsize, flags,
                      nullptr, 0, row_bytes};
-
-  c->begin(1);
   std::vector<ChunkIndex> ix;
   std::vector<unsigned char> ix_bytes;
-  if (int r = read_indexes(c, a, ix, ix_bytes)) return r;
-  c->end();
-  for (int i = 0; i < n_chunks; i++) chunk_status[i] = 0;
+  if (int r = start_decode_call(c, "recompress_chunks", a, chunk_status, ix, ix_bytes)) return r;
+  if (int r = check_capacity(c, n_chunks, chunk_rows, nc, itemsize, flags, dst_capacity)) return r;
 
   const bool host_io = !comp_is_device || !dst_is_device;
   const Batches sb = plan_encode_batches(c, n_chunks, chunk_rows, row_bytes, itemsize, flags,
@@ -1834,30 +1833,8 @@ int mtsb_recompress_chunks(mtsb_ctx* c, const void* comp_, int comp_is_device, c
     const void* unused_ref = nullptr;
     if (int r = inflate_batch(c, a, ix, sb, k, b, dcomp, unused_ref)) return r;
     std::vector<uint32_t> adler(b.nb, 0);     // the adler32 each good chunk's stored checksum confirmed
-    {
-      const int n_segs = (int)b.segs.size();
-      ReadBack rb(c);
-      rb.add(c->d_status.p, (size_t)n_segs * 4);
-      rb.add(c->d_tadler.p, (size_t)n_segs * 4);
-      rb.add(c->d_chunk_adler.p, (size_t)b.nb * 4);
-      if (int r = rb.sync()) return r;
-      chunk_verdicts(b, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), chunk_status, adler.data());
-    }
-    // a chunk whose index misled the decoder (see redecode_misled) is inflated again as a plain stream, alone, into its
-    // own place in d_T, before anything of the sub-batch is encoded
-    for (int i = c0; i < c1; i++) {
-      if (!chunk_status[i] || !ix[i].n_seg) continue;
-      ix[i] = ChunkIndex();
-      DecodeBatch one;
-      plan_segments(c, a, ix, i, i + 1, one, c0);
-      if (int r = inflate_stages(c, a, ix, dcomp, one)) return r;
-      ReadBack rb(c);
-      rb.add(c->d_status.p, 4);
-      rb.add(c->d_tadler.p, 4);
-      rb.add(c->d_chunk_adler.p, 4);
-      if (int r = rb.sync()) return r;
-      chunk_verdicts(one, ix, rb.get<int>(0), rb.get<uint32_t>(1), rb.get<uint32_t>(2), chunk_status, &adler[i - c0]);
-    }
+    if (int r = batch_verdicts(c, a, ix, b, chunk_status, adler.data())) return r;
+    if (int r = retry_misled(c, a, ix, b, dcomp, nullptr, nullptr, 0, chunk_status, adler.data())) return r;
     for (int i = c0; i < c1; i++) if (chunk_status[i]) any_bad = true;
     if (any_bad) continue;          // the output is undefined: only the statuses of the remaining chunks are wanted
 

@@ -1,4 +1,5 @@
-"""Shared helpers of the recompress suites (tests/test_emu_recompress.py, tests/test_gpu_recompress.py)."""
+"""Shared helpers of the recompress suites (tests/test_emu_recompress.py, tests/test_gpu_recompress.py), also used by the
+misled-index cases (tests/misled_cases.py, tests/test_emu_verify.py)."""
 import json
 import struct
 import zlib

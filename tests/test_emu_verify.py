@@ -3,7 +3,6 @@ kernels.  Every verdict is compared with NumPy's on the rows mtsb_decompress_chu
 ~np.isclose(decoded, ref, rtol, atol) for floats."""
 import ctypes as C
 import json
-import struct
 import zlib
 
 import numpy as np
@@ -14,6 +13,7 @@ import mtscomp_b200 as M
 from mtscomp_b200 import _native
 from mtscomp_b200.config import CHECK_ATOL
 from mtscomp_b200.core import CHECK_RTOL
+from recompress_cases import misleading_chunk
 
 DTYPES = (np.uint8, np.int16, np.int32, np.int64, np.float32, np.float64)
 ROWS = np.array([0, 301, 302, 1033, 1500, 2211, 2212, 2900], np.int64)   # ragged, with one-row chunks
@@ -185,40 +185,27 @@ def test_verify_corrupt_chunk(emu):
     assert m[good].tolist() == [0, 0, 0, 0, 1, 0] and f[5] == 2
 
 
-def _misleading(emu, data, flags):
-    """One chunk: a zlib stream of the chunk's bytes written by CPython's zlib, followed by a segment index written for
-    the GPU's own stream of the same rows, its last length adjusted so that the index passes every check of the
-    decoder (its lengths tile the foreign stream's body), yet does not describe that stream."""
-    from oracle import codec as ora
-    rows = np.array([0, data.shape[0]], np.int64)
-    gpu, offs = emu.compress(data, rows, flags)
-    gpu = gpu.tobytes()
-    d = zlib.decompressobj()
-    d.decompress(gpu)
-    index = d.unused_data
-    foreign = zlib.compress(ora.transform_chunk(data), 1)
-    sb, k, magic, total = struct.unpack('<4I', index[-16:])
-    v2 = len(index) > 4 * k + 16
-    lens_end = len(index) - 16 - (8 if v2 else 0)
-    lens = list(struct.unpack('<%dI' % k, index[lens_end - 4 * k:lens_end]))
-    body = len(foreign) - 6
-    lens[-1] += body - sum(lens)
-    assert lens[-1] > 0
-    index = (index[:lens_end - 4 * k] + struct.pack('<%dI' % k, *lens) + index[lens_end:-4] + struct.pack('<I', body))
-    return foreign + index
-
-
 def test_verify_misleading_index_is_retried(emu):
     nc, flags = 19, _native.flags_of(True, False, 'F')
     data = _data(np.int16, nc, 8)[:2000]
-    chunk = _misleading(emu, data, flags)
-    offs, rows = [0, len(chunk)], [0, data.shape[0]]
-    dec, st = emu.decompress(chunk, offs, rows, nc, np.int16, flags)
-    assert not st.any() and np.array_equal(dec, data)
-    assert _verify(emu, np.frombuffer(chunk, np.uint8), offs, rows, data, flags) == (np.zeros(1, np.int32), [0], [-1])
+    chunk = misleading_chunk(emu, data, flags)
+    d = zlib.decompressobj()
+    d.decompress(chunk)
+    plain = chunk[:len(chunk) - len(d.unused_data)]          # the same stream without the bytes after it
+    rows = [0, data.shape[0]]
+    launches = {}
+    for blob in (plain, chunk):
+        offs = [0, len(blob)]
+        dec, st = emu.decompress(blob, offs, rows, nc, np.int16, flags)
+        assert not st.any() and np.array_equal(dec, data)
+        n = emu.launches()
+        assert _verify(emu, np.frombuffer(blob, np.uint8), offs, rows, data, flags) == (np.zeros(1, np.int32), [0], [-1])
+        launches[blob] = (n, emu.launches())
+    # the call decoded the misled chunk through its index, then again as a plain stream
+    assert all(m > p for m, p in zip(launches[chunk], launches[plain])), launches.values()
     ref = data.copy()
     ref[1999, 18] += 3
-    st, m, f = _verify(emu, np.frombuffer(chunk, np.uint8), offs, rows, ref, flags)
+    st, m, f = _verify(emu, np.frombuffer(chunk, np.uint8), [0, len(chunk)], rows, ref, flags)
     assert not st.any() and m == [1] and f == [1999 * nc + 18]
 
 
